@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the similar-face-filtering hot path: face pairs compared per second.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg3] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic embeddings that are already resident in HBM:
 K1 (row L2-normalise + fp16 cast of the references; of the candidates too unless K2 does it in-kernel) -> K2 (tcgen05
@@ -68,6 +68,7 @@ THR = 0.5
 BLOCK = 62_500            # rows per synthetic block; data of a global row never depends on the GPU count
 L2_BYTES = 126 * 1024 * 1024
 VERIFY_ROWS = 10_240
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much
 METRIC_NAME = "face pairs compared/sec (ref x cand cosine+filter)"
 
 
@@ -356,6 +357,27 @@ def verify_sample(w, ref, cand, keep, idx, val, seed, threads):
             "oracle_seconds": round(secs, 2), "ok": mism == 0}
 
 
+def dump_outputs(out_dir, outputs, max_bytes=DUMP_BYTES, seed=0):
+    """--dump-outputs: each array of ``outputs`` -> ``out_dir/<name>.npy``, float64 for indices (float32 is exact only up
+    to 2**24), float32 otherwise, so that two builds can be compared output for output.  When the arrays would exceed
+    ``max_bytes`` in all, each is cut to the same seeded sample of rows and ``<name>_rows.npy`` (float64) says which."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {}
+    for name, t in outputs.items():
+        a = t.cpu().numpy()
+        host[name] = a.astype(np.float64 if a.dtype.kind in "iu" and a.dtype.itemsize > 2 else np.float32)
+    budget = max_bytes - 256 * 2 * len(host)                   # room for the .npy headers
+    sample = sum(a.nbytes for a in host.values()) > budget
+    frac = budget / sum(a.nbytes + 8 * len(a) for a in host.values())
+    for name, a in host.items():
+        if sample:
+            rows = np.sort(np.random.default_rng(seed).choice(len(a), int(len(a) * frac), replace=False))
+            np.save(os.path.join(out_dir, f"{name}_rows.npy"), rows.astype(np.float64))
+            a = a[rows]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def result_hash(keep, idx):
     import torch
     wgt = (torch.arange(idx.numel(), device=idx.device, dtype=torch.int64) % 1_000_003) + 1
@@ -363,10 +385,11 @@ def result_hash(keep, idx):
 
 
 # ------------------------------------------------------------------------------------------------ one workload on the GPU(s)
-def run_workload(key, steps, warmup, ctx, first_row=None, n_cand=None, do_verify=True, use_gather=True, sampler=None):
+def run_workload(key, steps, warmup, ctx, first_row=None, n_cand=None, do_verify=True, use_gather=True, sampler=None,
+                 keep_outputs=False):
     """Data generation, warm-up, the timed region (CUDA events on the launch stream, barrier + synchronize on both sides),
     per-launch K2 events, statistics, verification.  Returns a dict of raw measurements (this rank's; reduced by the
-    caller)."""
+    caller); with ``keep_outputs``, ``outputs`` holds copies of the arrays the last timed step handed back."""
     import torch
     import torch.distributed as dist
     ops, lib, dev = ctx["ops"], ctx["lib"], ctx["dev"]
@@ -429,6 +452,8 @@ def run_workload(key, steps, warmup, ctx, first_row=None, n_cand=None, do_verify
     lib.ffr_debug_set_k2_events(None, None)
     barrier()
     t_host1 = time.perf_counter()
+    # copied before the eager K2 timing and the stats call below write the same buffers again
+    outputs = {"keep": keep_all.clone(), "best_idx": idx_all.clone(), "best_val": val.clone()} if keep_outputs else None
     launches = ops.launch_count() - l0
     if graphs is not None:
         launches = steps * graphs[0].launches
@@ -447,7 +472,7 @@ def run_workload(key, steps, warmup, ctx, first_row=None, n_cand=None, do_verify
     last = (steps - 1) % n_buf
     res = {"key": key, "w": w, "n_cand": n_cand, "ms_total": ms_total, "k2_ms": k2_ms, "launches": launches, "steps": steps,
            "tensor_path": tensor_path, "n_buf": n_buf, "in_bytes": in_bytes, "clocks": clocks, "graph": graphs is not None,
-           "keep_frac": float(keep.float().mean())}
+           "keep_frac": float(keep.float().mean()), "outputs": outputs}
     if gather is not None:
         hashes = torch.stack([result_hash(keep_all[r * n_cand:(r + 1) * n_cand], idx_all[r * n_cand:(r + 1) * n_cand])
                               for r in range(world)])
@@ -531,7 +556,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the short cfg1 / hbm256 / cfg4 / dup8 / near8 / n1 runs of the default line")
     ap.add_argument("--no-strong", action="store_true", help="skip the one-GPU run of the whole N-GPU job")
     ap.add_argument("--no-verify", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (keep, best_idx, best_val) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     rank, world, local_rank = env_rank()
     # the contract is ONE JSON line on stdout: anything libraries print while we run (NCCL's version banner, warnings)
     # is sent to stderr by pointing fd 1 at fd 2 until the result line is written
@@ -571,10 +602,15 @@ def main():
     sampler = ClockSampler("GPU-" + str(torch.cuda.get_device_properties(local_rank).uuid)) if rank == 0 else None
     if sampler:
         sampler.start()
-    r = run_workload(args.workload, args.steps, args.warmup, ctx, do_verify=not args.no_verify, sampler=sampler)
+    r = run_workload(args.workload, args.steps, args.warmup, ctx, do_verify=not args.no_verify, sampler=sampler,
+                     keep_outputs=bool(args.dump_outputs) and rank == 0)
     if sampler:
         sampler.stop()
     ref, cands, keep, idx, val = r.pop("_data")
+    outputs = r.pop("outputs")
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs)
+        del outputs
     ms_total, k2_ms, launches = r["ms_total"], r["k2_ms"], r["launches"]
 
     # ---- end to end through the host-buffer C-ABI call (pinned host memory, H2D + D2H inside the timed region)

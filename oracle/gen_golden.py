@@ -97,7 +97,24 @@ def _facenetlike_factory():
     return lambda path: Adapter()
 
 
-def run_reference_main(reference_root, factory, out_path, tag):
+def sample_candidates(out, n_rows, seed=0):
+    """Cuts every class's candidate embeddings in ``out`` to ``n_rows`` rows: the quarter nearest to the threshold (where a
+    last-bit difference flips a decision) plus a seeded draw of the others.  ``c<i>_cand_rows`` lists the rows kept;
+    the decisions, names and summary line of all candidates stay.  Keeps a 512-d fixture under 1 MB."""
+    rng = np.random.default_rng(seed)
+    for c in range(int(out["n_classes"])):
+        cand = out[f"c{c}_cand"]
+        if cand.shape[0] <= n_rows:
+            continue
+        d = np.linalg.norm(cand.astype(np.float64) - out[f"c{c}_mu"].astype(np.float64), axis=1)
+        order = np.argsort(np.abs(d - float(out[f"c{c}_thres"])), kind="stable")
+        near, rest = order[:n_rows // 4], order[n_rows // 4:]
+        rows = np.sort(np.concatenate([near, rng.choice(rest, n_rows - len(near), replace=False)]))
+        out[f"c{c}_cand"] = cand[rows]
+        out[f"c{c}_cand_rows"] = rows.astype(np.int32)
+
+
+def run_reference_main(reference_root, factory, out_path, tag, max_cand=None):
     sff = os.path.join(reference_root, "similar_face_filtering")
     calls = []                        # ("predict", ndarray) | ("stats", path, mu, thres) | ("glob", pattern, list)
 
@@ -190,6 +207,8 @@ def run_reference_main(reference_root, factory, out_path, tag):
         else:
             i += 1
     out["n_classes"] = np.int32(cls_i)
+    if max_cand is not None:
+        sample_candidates(out, max_cand)
     np.savez_compressed(out_path, **out)
     print(f"[{tag}] {cls_i} classes ->", out_path, {k: (v.shape if hasattr(v, 'shape') else v) for k, v in out.items()
                                                      if k.endswith(('_cand', '_thres'))})
@@ -275,7 +294,7 @@ def main():
     run_reference_main(args.reference, _facenetlike_factory(), os.path.join(args.out, "ref_main_facenetlike.npz"),
                        "facenetlike")
     run_reference_main(args.reference, _mobilefacenet_factory(args.reference),
-                       os.path.join(args.out, "ref_main_mobilefacenet.npz"), "mobilefacenet")
+                       os.path.join(args.out, "ref_main_mobilefacenet.npz"), "mobilefacenet", max_cand=64)
 
 
 if __name__ == "__main__":

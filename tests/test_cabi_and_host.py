@@ -139,17 +139,46 @@ def test_class_mismatch_raises(tmp_path):
         main(["--ud", str(tmp_path / "u"), "--rd", str(tmp_path / "r"), "--td", str(tmp_path / "t")], model=object())
 
 
-REFERENCE_MFN = "/root/reference/face_detection_and_extraction/modules/mobile_facenet"
+# Stands in for the reference's face_detection_and_extraction/modules/mobile_facenet/mobile_facenet.py, which is not part
+# of this repository: same module name, same MobileFaceNet(embedding_size) constructor, [b, 3, 112, 112] in, and the
+# output goes through the reference's l2_norm (:30-33, :154).
+MOBILE_FACENET_PY = '''
+import torch
 
 
-@pytest.mark.skipif(not os.path.isdir(REFERENCE_MFN), reason="reference checkout not mounted (authoring container only)")
+def l2_norm(input, axis=1):
+    norm = torch.norm(input, 2, axis, True)
+    return torch.div(input, norm)
+
+
+class MobileFaceNet(torch.nn.Module):
+    def __init__(self, embedding_size):
+        super().__init__()
+        self.conv = torch.nn.Conv2d(3, 16, 3, stride=2, padding=1, bias=False)
+        self.bn = torch.nn.BatchNorm2d(16)
+        self.pool = torch.nn.AdaptiveAvgPool2d(7)
+        self.linear = torch.nn.Linear(16 * 7 * 7, embedding_size)
+
+    def forward(self, x):
+        x = self.pool(torch.relu(self.bn(self.conv(x))))
+        return l2_norm(self.linear(x.flatten(1)))
+'''
+
+
 def test_mobilefacenet_adapter_wraps_the_reference_model(tmp_path):
     """north_star: embedding extraction stays in the reference's own PyTorch MobileFaceNet.  The adapter imports that
-    class (never a copy), honours the predict() contract of filter_faces_using_reference.py:84,184 and returns exactly
-    what the reference network computes."""
+    class from the given directory (never a copy), honours the predict() contract of filter_faces_using_reference.py:84,184
+    and returns exactly what the wrapped network computes."""
     import sys
     import torch
     from face_detection_and_recognition_b200.filter_faces_using_reference import MobileFaceNetModel
+    REFERENCE_MFN = str(tmp_path / "mobile_facenet")
+    os.makedirs(REFERENCE_MFN)
+    with open(os.path.join(REFERENCE_MFN, "mobile_facenet.py"), "w") as f:
+        f.write(MOBILE_FACENET_PY)
+    sys.modules.pop("mobile_facenet", None)
+    with pytest.raises(FileNotFoundError):
+        MobileFaceNetModel(str(tmp_path / "missing.pth"), str(tmp_path), device="cpu", allow_random_init=True)
     with pytest.raises(FileNotFoundError):
         MobileFaceNetModel(str(tmp_path / "missing.pth"), REFERENCE_MFN, device="cpu")
     torch.manual_seed(0)

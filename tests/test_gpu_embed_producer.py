@@ -1,7 +1,7 @@
 """SURVEY §8f row 3 / §8a row a3 on the GPU: the device-side embedding producer (batched nvJPEG decode, GPU resize +
 standardisation, embeddings handed to the filter without leaving the device) behind the drop-in entry point, driven by a
 small torch module with the ``embed`` contract of ``MobileFaceNetModel`` (the reference's own MobileFaceNet class is not
-available on the GPU box, its adapter is covered in tests/test_cabi_and_host.py where /root/reference is mounted).
+part of this repository; its adapter is covered in tests/test_cabi_and_host.py).
 
 Replaces, for models that accept CUDA tensors, the reference's per-image host pipeline
 (similar_face_filtering/filter_faces_using_reference.py:60-68), its batch-1 reference embedding (:77-84) and the
