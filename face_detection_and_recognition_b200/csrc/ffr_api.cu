@@ -118,10 +118,18 @@ inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct WsLayout {
     size_t hdr, ref16, cand16, recs, full_rows, full_keys, full_ctr, dedup, total;
+    size_t e_bias, e_bias_c, e_nsq, e_scal, e_cscale;     // Euclid on the tensor cores (see EuclidWs)
     bool mma;
 };
 
+// The tcgen05 Euclid kernel exists for cta_group::2 only (an SM count that pairs up, FFR_CTA_GROUP=2): elsewhere Euclid keeps the
+// exact CUDA-core kernel K2s, like every other shape the tensor-core path does not take.
+bool euclid_mma_available() { return knobs().cta_group == 2 && (num_sms() & 1) == 0; }
+
 bool mma_eligible(int64_t n_ref, int32_t dim, int metric, int flags) {
+    if (metric == FFR_METRIC_EUCLID)   // K3 always re-checks Euclid: without it (FFR_FLAG_NO_RECHECK) the exact K2s path runs
+        return !(flags & FFR_FLAG_FORCE_FP32) && dim <= 512 && n_ref > 8 && !(flags & FFR_FLAG_NO_RECHECK) &&
+               euclid_mma_available();
     if (metric != FFR_METRIC_COSINE) return false;
     if (flags & FFR_FLAG_FORCE_FP32) return false;
     if (dim > 512) return false;
@@ -131,7 +139,10 @@ bool mma_eligible(int64_t n_ref, int32_t dim, int metric, int flags) {
 
 // need_c16: the fp16 copy of the candidates lives in the workspace (false for fp16 input and for stage32, whose fp16 A
 // tiles only ever exist in shared memory: 320 MB less at BASELINE configs[4]'s shard)
-WsLayout ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup) {
+// euclid: the tcgen05 Euclid path's extra buffers -- the reference bias (and its deduplicated copy), the references' squared
+// norms, two scalars, and the candidates' 1 / |c| (n_ref == 0: the caller prepared the references)
+WsLayout ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup,
+                   bool euclid = false) {
     WsLayout L{};
     L.mma = mma;
     size_t off = 0;
@@ -145,6 +156,14 @@ WsLayout ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool m
         L.full_keys = off; off += align_up(static_cast<size_t>(n_cand) * sizeof(unsigned long long), 256);
         L.full_ctr = off;  off += align_up((static_cast<size_t>(n_cand) / kFullGroup + 1) * sizeof(int32_t), 256);
         L.dedup = off;     if (dedup && dtype == FFR_DTYPE_F32) off += align_up(dedup_workspace_bytes(n_ref, static_cast<int32_t>(ld)), 256);
+        if (euclid) {
+            const size_t nb = n_ref > 0 ? static_cast<size_t>(euclid_bias_len(n_ref)) * 4 : 0;
+            L.e_bias = off;    off += align_up(nb, 256);
+            L.e_bias_c = off;  if (dedup) off += align_up(nb, 256);
+            L.e_nsq = off;     off += align_up(static_cast<size_t>(n_ref) * 4, 256);
+            L.e_scal = off;    off += 256;
+            L.e_cscale = off;  off += align_up(static_cast<size_t>(n_cand) * 4, 256);
+        }
     }
     L.total = off;
     return L;
@@ -167,23 +186,31 @@ int check_common(const void* ref, int64_t n_ref, const void* cand, int64_t n_can
 // core: ref16_pre != nullptr -> references already normalised/converted (ctx pipeline caches them)
 // ref16_pre != nullptr: the caller already holds the prepared references (fp16, normalised; when map_pre / nuniq_pre are given:
 // exact duplicates folded, see ffr_dedup.cu)
+// ref16_pre with metric Euclid: fp16(r * 2^-f) rows, and euclid_pre = {bias, bias_max} (launch_euclid_refs)
 int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre, const int32_t* nuniq_pre, int64_t n_ref,
                 const void* cand, int64_t n_cand, int32_t dim,
                 int dtype, int metric, float thr, int64_t ref_index_base, uint8_t* keep, int32_t* best_idx,
                 float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, int flags,
-                void* workspace, size_t ws_bytes, cudaStream_t s) {
+                void* workspace, size_t ws_bytes, cudaStream_t s, const float* const* euclid_pre = nullptr) {
     const bool mma = mma_eligible(n_ref, dim, metric, flags);
     if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
-        set_error("FFR_FLAG_FORCE_MMA: tcgen05 path needs metric cosine and dim <= 512 (dim=%d metric=%d)", dim, metric);
+        set_error("FFR_FLAG_FORCE_MMA: tcgen05 path needs dim <= 512, metric cosine, or metric euclid with n_ref > 8, the re-check "
+                  "and cta_group::2 (dim=%d metric=%d n_ref=%lld)", dim, metric, (long long)n_ref);
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    if (euclid && dtype != FFR_DTYPE_F32) {
+        set_error("metric euclid needs fp32 rows (FFR_DTYPE_F16 rows are normalised: their distances are not the embeddings')");
         return FFR_ERR_UNSUPPORTED;
     }
     const int32_t ld = ffr_padded_dim(dim);
-    // K2 normalises the candidates itself (K1 fused) when the shape pays for it; in its stage32 form no fp16 copy exists
-    const bool fuse = mma && dtype == FFR_DTYPE_F32 && n_cand > 0 &&
+    // K2 normalises the candidates itself (K1 fused) when the shape pays for it; in its stage32 form no fp16 copy exists.
+    // (Euclid always takes the K1 schedule: K1 also writes the candidates' 1 / |c|.)
+    const bool fuse = mma && !euclid && dtype == FFR_DTYPE_F32 && n_cand > 0 &&
                       filter_mma_can_fuse(static_cast<const float*>(cand), n_ref, n_cand, dim, ld);
     const bool need_c16 = !(fuse && filter_mma_skips_cand16(n_ref, n_cand, dim));
     const bool dedup = mma && dtype == FFR_DTYPE_F32 && ref16_pre == nullptr && dedup_wanted(n_ref, n_cand);
-    const WsLayout L = ws_layout(ref16_pre ? 0 : n_ref, n_cand, dim, dtype, mma, need_c16, dedup);
+    const WsLayout L = ws_layout(ref16_pre ? 0 : n_ref, n_cand, dim, dtype, mma, need_c16, dedup, mma && euclid);
     if (workspace == nullptr || ws_bytes < L.total) {
         set_error("workspace too small: need %zu bytes, got %zu%s", L.total, workspace ? ws_bytes : (size_t)0,
                   (mma && dtype == FFR_DTYPE_F32 && need_c16 && (reinterpret_cast<uintptr_t>(cand) & 15) != 0)
@@ -202,7 +229,7 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
 
     if (!mma) {
         if (dtype != FFR_DTYPE_F32) {
-            set_error("fp16 inputs are only accepted by the tcgen05 cosine path (n_ref > 8, dim <= 512)");
+            set_error("fp16 inputs are only accepted by the tcgen05 cosine path (n_ref > 8, dim <= 512; not with metric euclid)");
             return FFR_ERR_UNSUPPORTED;
         }
         g_last.launches = 1;
@@ -216,6 +243,25 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
     const float* fuse_cand = nullptr;        // non-null: K2 normalises the candidates itself (K1 fused)
     int launches = 0;
     int rc;
+    // Euclid: the reference bias, its maximum and the candidates' 1 / |c| (K2's score is acc + bias * scale)
+    const float* e_bias = nullptr;
+    const float* e_bmax = nullptr;
+    float* e_cscale = nullptr;
+    if (mma && euclid) {
+        e_cscale = reinterpret_cast<float*>(ws + L.e_cscale);
+        if (ref16_pre != nullptr) {
+            e_bias = euclid_pre[0]; e_bmax = euclid_pre[1];
+        } else {
+            __half* r16 = reinterpret_cast<__half*>(ws + L.ref16);
+            float* bias = reinterpret_cast<float*>(ws + L.e_bias);
+            float* scal = reinterpret_cast<float*>(ws + L.e_scal);
+            rc = launch_euclid_refs(static_cast<const float*>(ref), n_ref, dim, ld, r16, bias, reinterpret_cast<float*>(ws + L.e_nsq),
+                                    reinterpret_cast<uint32_t*>(scal), scal + 1, s);
+            if (rc != FFR_OK) return rc;
+            launches += 2;
+            ref16 = r16; e_bias = bias; e_bmax = scal + 1;
+        }
+    }
     if (dtype == FFR_DTYPE_F32) {
         // K1: references (unless the caller cached them) and candidates in ONE launch, which also zeroes the header
         static_assert(sizeof(WsHeader) % 4 == 0 && sizeof(WsHeader) / 4 <= 256, "header is zeroed by one CTA");
@@ -223,10 +269,10 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
         fuse_cand = fuse ? static_cast<const float*>(cand) : nullptr;
         __half* c16 = need_c16 ? reinterpret_cast<__half*>(ws + L.cand16) : nullptr;
         const bool k1_cand = fuse_cand == nullptr;          // otherwise K2's normaliser warps produce the fp16 rows themselves
-        const float* r32 = r16 ? static_cast<const float*>(ref) : nullptr;
-        const int64_t r_rows = r16 ? n_ref : 0;
+        const float* r32 = r16 && !euclid ? static_cast<const float*>(ref) : nullptr;   // (Euclid: prepared above)
+        const int64_t r_rows = r32 ? n_ref : 0;
         if (k1_cand) rc = launch_l2norm_pair(static_cast<const float*>(cand), n_cand, c16, r32, r_rows, r16, dim, ld, hdr,
-                                             static_cast<int32_t>(sizeof(WsHeader) / 4), s);
+                                             static_cast<int32_t>(sizeof(WsHeader) / 4), s, e_cscale);
         else         rc = launch_l2norm_pair(r32, r_rows, r16, nullptr, 0, nullptr, dim, ld, hdr,
                                              static_cast<int32_t>(sizeof(WsHeader) / 4), s);
         if (rc != FFR_OK) return rc;
@@ -236,17 +282,20 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
         if (dedup) {                       // fold bit-identical reference rows: K2 scans the unique ones and maps its columns back
             __half* r16c = nullptr;
             int32_t *map = nullptr, *nuniq = nullptr;
-            rc = launch_dedup_refs(static_cast<const float*>(ref), r16, n_ref, dim, ld, ws + L.dedup, &r16c, &map, &nuniq, s);
+            float* bias_c = euclid ? reinterpret_cast<float*>(ws + L.e_bias_c) : nullptr;
+            rc = launch_dedup_refs(static_cast<const float*>(ref), ref16, n_ref, dim, ld, ws + L.dedup, &r16c, &map, &nuniq, s,
+                                   euclid ? e_bias : nullptr, bias_c);
             if (rc != FFR_OK) return rc;
             launches += 4;
             ref16 = r16c; map_pre = map; nuniq_pre = nuniq;
+            if (euclid) e_bias = bias_c;
         }
     } else {
         if (ref16 == nullptr) ref16 = static_cast<const __half*>(ref);
         cand16 = const_cast<__half*>(static_cast<const __half*>(cand));      // fp16 input: only read
     }
     const bool recheck = (dtype == FFR_DTYPE_F32) && !(flags & FFR_FLAG_NO_RECHECK);
-    g_last.launches = launches + 1 + (recheck ? 1 : 0);
+    g_last.launches = launches + 1 + (recheck ? 1 : 0) + (euclid ? 1 : 0);
     RecheckLists lists;
     lists.hdr = hdr;
     lists.recs = reinterpret_cast<RecheckRec*>(ws + L.recs);
@@ -259,17 +308,23 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
     float thr_band = delta;
     if (band_count != nullptr && band_tol + delta > thr_band) thr_band = band_tol + delta;
     if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
-    rc = launch_filter_mma(ref16, n_ref, cand16, fuse_cand, dim, n_cand, ld, thr, delta, thr_band, ref_index_base, keep, best_idx,
-                           best_val, lists, recheck ? 0 : 1, band_tol, band_count, band_rows, band_cap,
-                           /*after_k1=*/dtype == FFR_DTYPE_F32 && !dedup, map_pre, nuniq_pre, s);
+    // Euclid: K2 and K3 only choose the index -- a threshold that never flags a row, no band -- and the value pass decides
+    rc = launch_filter_mma(ref16, n_ref, cand16, fuse_cand, dim, n_cand, ld, euclid ? -INFINITY : thr, delta, euclid ? 0.f : thr_band,
+                           ref_index_base, keep, best_idx, best_val, lists, recheck ? 0 : 1, band_tol, band_count, band_rows,
+                           band_cap, /*after_k1=*/dtype == FFR_DTYPE_F32 && !dedup, map_pre, nuniq_pre, s,
+                           e_bias, e_cscale, e_bmax);
     if (rc != FFR_OK) return rc;
     if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
+    const int emode = euclid ? k2s_dist_mode_gallery(static_cast<const float*>(ref), static_cast<const float*>(cand), dim) : -1;
     if (recheck) {
         rc = launch_recheck(static_cast<const float*>(ref), n_ref, static_cast<const float*>(cand), n_cand, dim, nullptr,
                             nullptr, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol,
-                            band_count, band_rows, band_cap, map_pre, nuniq_pre, s);
+                            euclid ? nullptr : band_count, band_rows, band_cap, map_pre, nuniq_pre, s, emode);
         if (rc != FFR_OK) return rc;
     }
+    if (euclid)
+        return launch_euclid_values(static_cast<const float*>(ref), static_cast<const float*>(cand), n_cand, dim, thr,
+                                    ref_index_base, keep, best_idx, best_val, band_tol, band_count, band_rows, band_cap, emode, s);
     return FFR_OK;
 }
 
@@ -323,6 +378,10 @@ int ffr_l2norm_rows_f32(const float* x, int64_t rows, int32_t dim, void* y_f16, 
 size_t ffr_filter_workspace_bytes(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, int metric) {
     if (n_ref <= 0 || n_cand < 0 || dim <= 0) return 0;
     // sized for the tcgen05 path whenever it could be chosen (including FFR_FLAG_FORCE_MMA)
+    if (metric == FFR_METRIC_EUCLID) {      // the tcgen05 Euclid path (K1 schedule: the fp16 candidates live in the workspace)
+        const bool mma = dim <= 512 && n_ref > 8 && dtype == FFR_DTYPE_F32;
+        return ws_layout(n_ref, n_cand, dim, dtype, mma, true, mma && dedup_wanted(n_ref, n_cand), mma).total;
+    }
     const bool mma = metric == FFR_METRIC_COSINE && dim <= 512;
     const bool need_c16 = !(mma && dtype == FFR_DTYPE_F32 && filter_mma_skips_cand16(n_ref, n_cand, dim));
     return ws_layout(n_ref, n_cand, dim, dtype, mma, need_c16, mma && dedup_wanted(n_ref, n_cand)).total;
@@ -430,6 +489,10 @@ struct ffr_ctx {
     float* d_ref;
     __half* d_ref16;
     void* d_dedup;             // scratch of the duplicate-reference fold (per call, not per chunk)
+    float* d_ebias;            // Euclid: reference bias [pad(max_ref)], its deduplicated copy, squared norms, two scalars
+    float* d_ebias_c;
+    float* d_ensq;
+    float* d_escal;
     float* d_cand[2];
     uint8_t* d_keep[2];
     int32_t* d_idx[2];
@@ -447,6 +510,7 @@ void ffr_ctx_destroy(ffr_ctx* c) {
     if (c->s_comp) cudaStreamSynchronize(c->s_comp);
     if (c->s_copy) cudaStreamSynchronize(c->s_copy);
     cudaFree(c->d_ref); cudaFree(c->d_ref16); cudaFree(c->d_dedup);
+    cudaFree(c->d_ebias); cudaFree(c->d_ebias_c); cudaFree(c->d_ensq); cudaFree(c->d_escal);
     for (int i = 0; i < 2; ++i) {
         cudaFree(c->d_cand[i]); cudaFree(c->d_keep[i]); cudaFree(c->d_idx[i]); cudaFree(c->d_val[i]); cudaFree(c->ws[i]);
         if (c->ev_h2d[i]) cudaEventDestroy(c->ev_h2d[i]);
@@ -473,7 +537,12 @@ int ffr_ctx_create(int device, int64_t max_ref, int64_t chunk_cand, int32_t max_
     FFR_CTX_TRY(cudaMalloc(&c->d_ref, static_cast<size_t>(max_ref) * max_dim * sizeof(float)));
     FFR_CTX_TRY(cudaMalloc(&c->d_ref16, static_cast<size_t>(max_ref) * ld * 2));
     FFR_CTX_TRY(cudaMalloc(&c->d_dedup, dedup_workspace_bytes(max_ref, static_cast<int32_t>(ld))));
-    c->ws_bytes = ws_layout(1, chunk_cand, max_dim <= 512 ? max_dim : 512, FFR_DTYPE_F32, true, true, false).total;   // any dim <= max_dim
+    FFR_CTX_TRY(cudaMalloc(&c->d_ebias, static_cast<size_t>(euclid_bias_len(max_ref)) * sizeof(float)));
+    FFR_CTX_TRY(cudaMalloc(&c->d_ebias_c, static_cast<size_t>(euclid_bias_len(max_ref)) * sizeof(float)));
+    FFR_CTX_TRY(cudaMalloc(&c->d_ensq, static_cast<size_t>(max_ref) * sizeof(float)));
+    FFR_CTX_TRY(cudaMalloc(&c->d_escal, 256));
+    // any dim <= max_dim, either metric
+    c->ws_bytes = ws_layout(1, chunk_cand, max_dim <= 512 ? max_dim : 512, FFR_DTYPE_F32, true, true, false, true).total;
     if (c->ws_bytes < 4096) c->ws_bytes = 4096;
     for (int i = 0; i < 2; ++i) {
         FFR_CTX_TRY(cudaEventCreateWithFlags(&c->ev_h2d[i], cudaEventDisableTiming));
@@ -502,16 +571,24 @@ int ffr_ctx_filter_host(ffr_ctx* c, const float* ref, int64_t n_ref, const float
     FFR_CUDA_TRY(cudaMemcpyAsync(c->d_ref, ref, static_cast<size_t>(n_ref) * dim * sizeof(float), cudaMemcpyHostToDevice, c->s_comp));
     const __half* ref16 = nullptr;
     const int32_t *ref_map = nullptr, *n_unique = nullptr;
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    const float* euclid_pre[2] = {c->d_ebias, c->d_escal + 1};
     if (mma) {      // references are normalised / converted (and exact duplicates folded) once, not per chunk
-        rc = launch_l2norm(c->d_ref, n_ref, dim, c->d_ref16, ffr_padded_dim(dim), nullptr, nullptr, c->s_comp);
+        if (euclid)
+            rc = launch_euclid_refs(c->d_ref, n_ref, dim, ffr_padded_dim(dim), c->d_ref16, c->d_ebias, c->d_ensq,
+                                    reinterpret_cast<uint32_t*>(c->d_escal), c->d_escal + 1, c->s_comp);
+        else
+            rc = launch_l2norm(c->d_ref, n_ref, dim, c->d_ref16, ffr_padded_dim(dim), nullptr, nullptr, c->s_comp);
         if (rc != FFR_OK) return rc;
         ref16 = c->d_ref16;
         if (dedup_wanted(n_ref, n_cand)) {
             __half* r16c = nullptr;
             int32_t *map = nullptr, *nuniq = nullptr;
-            rc = launch_dedup_refs(c->d_ref, c->d_ref16, n_ref, dim, ffr_padded_dim(dim), c->d_dedup, &r16c, &map, &nuniq, c->s_comp);
+            rc = launch_dedup_refs(c->d_ref, c->d_ref16, n_ref, dim, ffr_padded_dim(dim), c->d_dedup, &r16c, &map, &nuniq, c->s_comp,
+                                   euclid ? c->d_ebias : nullptr, c->d_ebias_c);
             if (rc != FFR_OK) return rc;
             ref16 = r16c; ref_map = map; n_unique = nuniq;
+            if (euclid) euclid_pre[0] = c->d_ebias_c;
         }
     }
     int64_t i = 0;
@@ -525,7 +602,7 @@ int ffr_ctx_filter_host(ffr_ctx* c, const float* ref, int64_t n_ref, const float
         FFR_CUDA_TRY(cudaStreamWaitEvent(c->s_comp, c->ev_h2d[b], 0));
         rc = filter_core(c->d_ref, ref16, ref_map, n_unique, n_ref, c->d_cand[b], m, dim, FFR_DTYPE_F32, metric, thr, ref_index_base,
                          c->d_keep[b], c->d_idx[b], c->d_val[b], 0.f, nullptr, nullptr, 0, flags, c->ws[b], c->ws_bytes,
-                         c->s_comp);
+                         c->s_comp, euclid_pre);
         if (rc != FFR_OK) return rc;
         FFR_CUDA_TRY(cudaMemcpyAsync(keep + off, c->d_keep[b], static_cast<size_t>(m), cudaMemcpyDeviceToHost, c->s_comp));
         FFR_CUDA_TRY(cudaMemcpyAsync(best_idx + off, c->d_idx[b], static_cast<size_t>(m) * sizeof(int32_t), cudaMemcpyDeviceToHost, c->s_comp));

@@ -322,25 +322,38 @@ int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64
                        float thr, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                        float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s);
 int launch_l2norm_pair(const float* x_a, int64_t rows_a, __half* y16_a, const float* x_b, int64_t rows_b, __half* y16_b,
-                       int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s);
+                       int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s,
+                       float* scale_a = nullptr);
+// Euclid on the tensor cores (ffr_l2norm.cu): fp16(r * 2^-f) rows, f from the largest reference norm (device side), and the
+// per-reference bias beta_i = -|r_i|^2 * 2^-f / 2 (zero padded to a multiple of 256); bmax[0] = max_i |beta_i|.
+// nsq: n_ref floats of scratch, max_bits: one zeroed-here word.
+int launch_euclid_refs(const float* ref, int64_t n_ref, int32_t dim, int32_t ld16, __half* ref16, float* beta, float* nsq,
+                       uint32_t* max_bits, float* bmax, cudaStream_t s);
+inline int64_t euclid_bias_len(int64_t n_ref) { return (n_ref + 255) / 256 * 256; }
 bool filter_mma_can_fuse(const float* cand32, int64_t n_ref, int64_t n_cand, int32_t dim, int32_t dim_pad);
 int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const float* cand32, int32_t dim,
                       int64_t n_cand, int32_t dim_pad,
                       float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                       RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
-                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s);
+                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
+                      const float* euclid_bias = nullptr, const float* cand_scale = nullptr, const float* bias_max = nullptr);
 // exact-duplicate reference rows folded before K2 (ffr_dedup.cu)
 bool dedup_wanted(int64_t n_ref, int64_t n_cand);
 size_t dedup_workspace_bytes(int64_t n_ref, int32_t ld);
 int launch_dedup_refs(const float* ref32, const __half* ref16_full, int64_t n_ref, int32_t dim, int32_t ld, void* ws,
-                      __half** out_ref16, int32_t** out_map, int32_t** out_n_unique_dev, cudaStream_t s);
+                      __half** out_ref16, int32_t** out_map, int32_t** out_n_unique_dev, cudaStream_t s,
+                      const float* bias = nullptr, float* bias_c = nullptr);   // Euclid: the bias is compacted with the rows
 bool filter_mma_skips_cand16(int64_t n_ref, int64_t n_cand, int32_t dim);
 void get_last_k2_config(int out[8]);
 int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim,
                    const float* ref_norm, const float* cand_norm, float thr, int64_t ref_index_base,
                    uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s);
+                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode = -1);
+// Euclid after the tensor-core pass: keep / best_val / band from the K2s distance to the chosen reference (ffr_filter_fp32.cu)
+int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
+                         uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
+                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s);
 int launch_ref_stats_batched(const float* ref_feat, const int32_t* offsets, int32_t n_classes, int32_t dim, float* mean,
                              float* thres, cudaStream_t s);
 int launch_first_match_stream(float* g_feat, float* g_bbox, int32_t* g_count, int32_t cap, const float* queries,
@@ -349,6 +362,7 @@ int launch_first_match_stream(float* g_feat, float* g_bbox, int32_t* g_count, in
 void set_mma_prof_buffer(unsigned long long* dev_ptr);   // diagnostics: [grid][16] stall-cycle counters of K2
 int launch_ref_stats(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres, cudaStream_t s);
 int k2s_dist_mode(const float* rows, int32_t dim);       // which K2s form scores (n_ref = 1, Euclid) rows of this width / alignment
+int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim);   // ... and which form K2s uses for n_ref > 2
 int launch_pack_results(const uint8_t* keep, const int32_t* idx, int64_t m, int64_t m_pad, uint8_t* packed,
                         cudaStream_t s);
 int launch_unpack_results(const uint8_t* packed, int64_t m, int64_t m_pad, int nranks, uint8_t* keep, int32_t* idx,

@@ -13,7 +13,8 @@
 //   D2 mark_dups_kernel     one warp per row: the representative of its hash; bit-for-bit comparison of the two rows
 //                           (a hash collision between different rows keeps both: dedup is an optimisation, never a guess)
 //   D3 scan_unique_kernel   exclusive prefix sum of the "unique" flags (one CTA), number of unique rows
-//   D4 compact_rows_kernel  unique fp16 rows (K1's output) -> consecutive rows; map[new] = old
+//   D4 compact_rows_kernel  unique fp16 rows (K1's output) -> consecutive rows; map[new] = old; with the Euclid filter the
+//                           per-reference bias moves with its row
 #include "ffr_common.cuh"
 
 namespace ffr {
@@ -124,7 +125,8 @@ scan_unique_kernel(int32_t* __restrict__ unique, int64_t rows, int32_t* __restri
 
 __global__ void __launch_bounds__(kThreads)
 compact_rows_kernel(const __half* __restrict__ src, int64_t rows, int32_t ld, const int32_t* __restrict__ pos,
-                    __half* __restrict__ dst, int32_t* __restrict__ map) {
+                    __half* __restrict__ dst, int32_t* __restrict__ map, const float* __restrict__ bias,
+                    float* __restrict__ bias_c) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
@@ -136,6 +138,7 @@ compact_rows_kernel(const __half* __restrict__ src, int64_t rows, int32_t ld, co
         uint4* d = reinterpret_cast<uint4*>(dst + static_cast<int64_t>(q) * ld);
         for (int k = lane; k < n16; k += 32) d[k] = __ldg(s + k);
         if (lane == 0) map[q] = static_cast<int32_t>(r);
+        if (lane == 0 && bias != nullptr) bias_c[q] = bias[r];
     }
 }
 
@@ -164,7 +167,8 @@ size_t dedup_workspace_bytes(int64_t n_ref, int32_t ld) {
 // ref32: the original rows; ref16_full: K1's normalised fp16 rows of ALL references (leading dimension ld).  On return (stream
 // order) *out_ref16 holds the unique rows, *out_map the compact -> original index map, *out_n_unique (device) their count.
 int launch_dedup_refs(const float* ref32, const __half* ref16_full, int64_t n_ref, int32_t dim, int32_t ld, void* ws,
-                      __half** out_ref16, int32_t** out_map, int32_t** out_n_unique_dev, cudaStream_t s) {
+                      __half** out_ref16, int32_t** out_map, int32_t** out_n_unique_dev, cudaStream_t s,
+                      const float* bias, float* bias_c) {
     uint8_t* w = static_cast<uint8_t*>(ws);
     const size_t n = static_cast<size_t>(n_ref);
     const uint32_t t = table_size(n_ref);
@@ -186,7 +190,7 @@ int launch_dedup_refs(const float* ref32, const __half* ref16_full, int64_t n_re
     FFR_LAUNCH_CHECK("dedup_mark_dups");
     scan_unique_kernel<<<1, 1024, 0, s>>>(pos, n_ref, pos + n_ref);
     FFR_LAUNCH_CHECK("dedup_scan_unique");
-    compact_rows_kernel<<<g, kThreads, 0, s>>>(ref16_full, n_ref, ld, pos, ref16c, map);
+    compact_rows_kernel<<<g, kThreads, 0, s>>>(ref16_full, n_ref, ld, pos, ref16c, map, bias, bias_c);
     FFR_LAUNCH_CHECK("dedup_compact_rows");
     *out_ref16 = ref16c;
     *out_map = map;

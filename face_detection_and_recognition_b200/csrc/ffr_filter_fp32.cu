@@ -322,6 +322,32 @@ ref_stats_kernel(const float* __restrict__ x, int32_t n, int32_t dim, float* __r
     }
 }
 
+// Value pass of the tcgen05 Euclid filter: K2 + K3 chose best_idx; the distance to that reference is recomputed here with
+// exactly the arithmetic K2s uses for the same (row, reference) pair (k2s_euclid_dist in K2s's mode for n_ref > 2), so keep and
+// best_val are bit-identical to the FFR_FLAG_FORCE_FP32 result wherever the index agrees.  One warp per row; HBM-bound (one
+// read of the candidate matrix, the winners' rows mostly from L2).
+template <int kMode>
+__global__ void __launch_bounds__(kThreads)
+euclid_value_kernel(const float* __restrict__ ref, const float* __restrict__ cand, int64_t n_cand, int32_t dim, float thr,
+                    int64_t ref_index_base, uint8_t* __restrict__ keep, const int32_t* __restrict__ best_idx,
+                    float* __restrict__ best_val, BandOut band) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
+    const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
+    for (int64_t row = warp; row < n_cand; row += nwarps) {
+        const int64_t ri = static_cast<int64_t>(__ldg(best_idx + row)) - ref_index_base;
+        const float d = k2s_euclid_dist(cand + row * dim, ref + ri * dim, dim, lane, kMode);
+        if (lane == 0) {
+            keep[row] = d <= thr ? 1 : 0;
+            if (best_val != nullptr) best_val[row] = d;
+            if (band.count != nullptr && fabsf(d - thr) <= band.tol) {
+                const int32_t slot = atomicAdd(band.count, 1);
+                if (band.rows != nullptr && slot < band.cap) band.rows[slot] = row;
+            }
+        }
+    }
+}
+
 template <int NV, bool kCosine>
 int launch_vec(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, float thr,
                int64_t base, uint8_t* keep, int32_t* idx, float* val, BandOut band, dim3 g, cudaStream_t s) {
@@ -394,6 +420,35 @@ int k2s_dist_mode(const float* rows, int32_t dim) {
     if ((dim == 128 || dim == 256) && knobs().k2s_subwarp != 0) return dim == 128 ? 16 : 32;
     const int nv = (dim + 127) / 128;
     return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
+}
+
+// mirrors launch_filter_fp32's choice of kernel for n_ref > 2 (metric Euclid): the warp-per-row kernel with NV float4 per lane,
+// or the scalar catch-all
+int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim) {
+    const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
+    if (!vec_ok) return 0;
+    const int nv = (dim + 127) / 128;
+    return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
+}
+
+int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
+                         uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
+                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s) {
+    if (n_cand == 0) return FFR_OK;
+    int64_t grid = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
+    if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
+    const dim3 g(static_cast<unsigned>(grid));
+    const BandOut band{band_tol, band_count, band_rows, band_cap};
+    switch (mode) {
+        case 1: euclid_value_kernel<1><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        case 2: euclid_value_kernel<2><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        case 4: euclid_value_kernel<4><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        case 8: euclid_value_kernel<8><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        default: euclid_value_kernel<0><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+    }
+    FFR_LAUNCH_CHECK("euclid_values");
+    return FFR_OK;
 }
 
 int launch_ref_stats(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres, cudaStream_t s) {

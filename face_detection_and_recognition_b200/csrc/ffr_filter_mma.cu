@@ -470,6 +470,10 @@ struct KParams {
     uint32_t b_tx_bytes;           // bytes one CTA's B-stage TMA load delivers (diagnostics can halve the box: FFR_DIAG_HALF_B)
     int epi_mode;                  // diagnostics: 1 = epilogue only loads TMEM (no max tree), results invalid
     unsigned long long* prof;      // optional [gridDim.x][32] stall-cycle counters (diagnostics)
+    // kEuclid: score = acc + ref_bias[col] * cand_scale[row] (DESIGN.md section 4, "Euclid on the tensor cores")
+    const float* ref_bias;         // -|r|^2 * 2^-f / 2 per (compact) reference column, zero padded to a multiple of kTileN
+    const float* cand_scale;       // 1 / |c| per candidate row (K1)
+    const float* bias_max;         // max |ref_bias| (device scalar): sizes the per-row window
 };
 
 // End of a candidate tile, once per row (the two column halves merged): classify_row writes keep / index / score and decides
@@ -484,16 +488,21 @@ struct RowOut {
     RecheckRec rec;
 };
 
-__device__ __forceinline__ RowOut classify_row(const KParams& p, const Top3& t, const HiddenM& hid, int64_t row) {
+// kEuclid: the row's window is delta_e (not p.delta), and force_full sends the row to the full rescan whatever its scores
+template <bool kEuclid = false>
+__device__ __forceinline__ RowOut classify_row(const KParams& p, const Top3& t, const HiddenM& hid, int64_t row,
+                                               float delta_e = 0.f, bool force_full = false) {
     RowOut o;
+    const auto delta = [&]() { return kEuclid ? delta_e : p.delta; };
     const bool valid = row < p.n_cand;
-    const bool near_tie = (t.i2 >= 0) && (t.b1 - t.b2 <= p.delta);
+    const bool near_tie = (t.i2 >= 0) && (t.b1 - t.b2 <= delta());
     const bool near_thr = fabsf(t.b1 - p.thr) <= p.thr_band;
     // un-inserted columns may be inside the window: of ONE part (K3 rescans its 128 references), or of more
-    const bool hid2 = hid.amb2 > -INFINITY && hid.amb2 >= t.b1 - p.delta;
-    const bool hid1 = hid.amb > -INFINITY && hid.amb >= t.b1 - p.delta;
-    const bool flagged = valid && !p.no_recheck && (near_tie || near_thr || hid1 || hid2);
-    const bool full = flagged && (hid2 || t.b1 - t.b4 <= p.delta);     // four or more inside the window, or hidden ones anywhere
+    const bool hid2 = hid.amb2 > -INFINITY && hid.amb2 >= t.b1 - delta();
+    const bool hid1 = hid.amb > -INFINITY && hid.amb >= t.b1 - delta();
+    const bool forced = kEuclid && force_full;
+    const bool flagged = valid && !p.no_recheck && (forced || near_tie || near_thr || hid1 || hid2);
+    const bool full = flagged && (forced || hid2 || t.b1 - t.b4 <= delta());   // four or more inside the window, or hidden ones anywhere
     const bool part = flagged && !full && hid1;                        // hidden columns in one known part
     const int32_t* map = p.ref_map;                                     // duplicate references folded: compact -> original index
     const auto orig = [&](int32_t i) { return (map != nullptr && i >= 0) ? map[i] : i; };
@@ -516,7 +525,7 @@ __device__ __forceinline__ RowOut classify_row(const KParams& p, const Top3& t, 
         // makes it a full rescan.  (Layout: ffr_recheck.cu, K3p.)
         const int32_t span = (hid.xm >> 16) != 0u ? kTileN : kTileN / 2;     // one part, or two adjacent ones
         const auto outside = [&](float b, int32_t i) {
-            return i >= 0 && b >= t.b1 - p.delta && (i < hid.base || i >= hid.base + span);
+            return i >= 0 && b >= t.b1 - delta() && (i < hid.base || i >= hid.base + span);
         };
         int32_t e = -1;
         int ne = 0;
@@ -530,7 +539,7 @@ __device__ __forceinline__ RowOut classify_row(const KParams& p, const Top3& t, 
     } else if (o.cls == 1) {
         o.rec.idx1 = orig(t.i1);
         o.rec.idx2 = near_tie ? orig(t.i2) : -1;
-        o.rec.idx3 = (near_tie && t.i3 >= 0 && t.b1 - t.b3 <= p.delta) ? orig(t.i3) : -1;
+        o.rec.idx3 = (near_tie && t.i3 >= 0 && t.b1 - t.b3 <= delta()) ? orig(t.i3) : -1;
     }
     return o;
 }
@@ -586,7 +595,9 @@ __device__ __forceinline__ void append_rows(const KParams& p, const RowOut (&o)[
 // kExact / kAlways: the two epilogue policies as COMPILE-TIME constants (0 | 1; 2 = read the run-time flag, used by the
 // instrumented build and cta_group::1).  kExact = 0 removes the ~1100-instruction exact fall-back (update_part) from the
 // hot loop's body altogether; kAlways picks the unconditional or the gated update path.
-template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr>
+// kEuclid: the Euclid decision rule (K1 schedule, cta_group::2, production policies only): every score gets the per-reference
+// bias scaled by the row's 1 / |c| before the max trees, and the row's window widens with that bias (DESIGN.md section 4).
+template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr, bool kEuclid = false>
 __global__ void __launch_bounds__(64 + 32 * 8 + (kNormMode ? 64 : 0), 1)   // 10 warps are allocated as 12: <= 168 registers
 filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_constant__ CUtensorMap tmap_ref,
                   const __grid_constant__ CUtensorMap tmap_cand32, const KParams p) {
@@ -1128,6 +1139,17 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             hid.base = 0;
             hid.mask = 0;
             const int64_t row = tile * (kTileM * kCG) + cta_rank * kTileM + r_in_tile;
+            float delta_row = 0.f, s_row = 0.f;
+            if constexpr (kEuclid) {
+                static_assert(kNormMode == 0 && !kInstr, "Euclid runs on the K1 schedule, production build only");
+                // K1 writes the scales; it precedes this kernel as its programmatic dependency
+                if (first_tile) pdl_wait();
+                s_row = row < p.n_cand ? __ldg(p.cand_scale + row) : 0.f;
+                // |score error| <= fp16 operand error (delta, as for cosine) + a few fp32 roundings of the bias term (beta and
+                // 1/|c| each carry one, the FFMA another): 8 ulp of max |beta| / |c| covers them.  (A zero-norm or non-finite row
+                // -- s_row not finite -- gets a NaN window here and goes to the full fp32 rescan in the tail.)
+                delta_row = fmaf(__ldg(p.bias_max) * s_row, 4.76837158e-7f, p.delta);
+            }
             // One reference tile.  The loop over FULL tiles and the one partial last tile are separate copies of this body: the
             // masking of columns >= n_ref is 260 instructions that the hot loop would otherwise carry (and jump over) on every
             // tile -- the body is what has to stream through the instruction cache.
@@ -1160,6 +1182,19 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                         if (kCG == 2 && !leader) mbar_arrive_leader_relaxed(&t_empty[acc]);
                         else                     mbar_arrive(&t_empty[acc]);
                     }
+                    if constexpr (kEuclid) {                       // score = acc + beta_col / |c|, two columns per FFMA2
+                        const float4* bp = reinterpret_cast<const float4*>(p.ref_bias + base0);
+                        const float2 s2 = make_float2(s_row, s_row);
+#pragma unroll
+                        for (int cc = 0; cc < kChunksPerPart; ++cc)
+#pragma unroll
+                            for (int j4 = 0; j4 < 8; ++j4) {
+                                const float4 b = __ldg(bp + cc * 8 + j4);
+                                const float2 lo = __ffma2_rn(make_float2(b.x, b.y), s2, make_float2(v[cc][4 * j4], v[cc][4 * j4 + 1]));
+                                const float2 hi = __ffma2_rn(make_float2(b.z, b.w), s2, make_float2(v[cc][4 * j4 + 2], v[cc][4 * j4 + 3]));
+                                v[cc][4 * j4] = lo.x; v[cc][4 * j4 + 1] = lo.y; v[cc][4 * j4 + 2] = hi.x; v[cc][4 * j4 + 3] = hi.y;
+                            }
+                    }
                     if constexpr (kPartial) {                      // partial last reference tile: columns >= n_ref -> -inf
                         const int n_left = static_cast<int>(ncols64) - h * (kChunksPerPart * 32);
 #pragma unroll
@@ -1178,7 +1213,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     // short reference sets: some lane of the warp sets a record on nearly every tile, so the update runs
                     // unconditionally and branch-free; long ones: behind one branch on the part maximum.  (Round-1c's
                     // per-chunk update paths are gone from this loop: dead code in it costs wall clock.)
-                    if (grid_updates || m >= gate) update_grid<kChunksPerPart>(v, sx, cm, m, base0, p.delta, grid_exact, t, gate, hid);
+                    if (grid_updates || m >= gate) update_grid<kChunksPerPart>(v, sx, cm, m, base0, kEuclid ? delta_row : p.delta, grid_exact, t, gate, hid);
                     if (pr) c_hot += static_cast<unsigned long long>(clock64() - tp0);
                 } else {
                     // ---- general loop, one chunk at a time: diagnostics only (score dump, epilogue modes)
@@ -1308,7 +1343,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 }
 
                 RowOut ro[1];
-                ro[0] = classify_row(p, t, hm, row);
+                ro[0] = classify_row<kEuclid>(p, t, hm, row, delta_row, !(fabsf(s_row) <= 3.4e38f));
                 append_rows<1>(p, ro, lane);
             }
             }   // !st32
@@ -1438,7 +1473,8 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                            int64_t n_cand, int32_t dim_pad,
                            float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                            RecheckLists lists, int no_recheck, BandArgs band, float* dbg_scores, bool after_k1,
-                           const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s) {
+                           const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
+                           const float* euclid_bias, const float* cand_scale, const float* bias_max) {
     if (dim_pad % kBlockK != 0 || dim_pad < kBlockK || dim_pad > 512) {
         set_error("filter_mma: padded dim %d not in {64..512 step 64}", dim_pad);
         return FFR_ERR_UNSUPPORTED;
@@ -1454,6 +1490,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     int cg = kn.cta_group;
     if (cg != 2 || (sms & 1)) cg = 1;
     const bool fuse = cand32 != nullptr;
+    const bool euclid = euclid_bias != nullptr;
+    if (euclid && (cg != 2 || fuse || no_recheck || dbg_scores != nullptr)) {
+        set_error("filter_mma: the Euclid kernel exists for cta_group::2, the K1 schedule and the re-checked build only");
+        return FFR_ERR_UNSUPPORTED;
+    }
     const int kb = dim_pad / kBlockK;
     constexpr int acc_n = kTileN;
     const uint32_t a_stage = kb * kABlockBytes;
@@ -1505,6 +1546,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     p.thr = thr; p.delta = delta; p.thr_band = thr_band; p.ref_index_base = ref_index_base;
     p.keep = keep; p.best_idx = idx; p.best_val = val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof; p.epi_mode = kn.epi_mode;
     p.band_tol = band.tol; p.band_count = no_recheck ? band.count : nullptr; p.band_rows = band.rows; p.band_cap = band.cap;
+    p.ref_bias = euclid_bias; p.cand_scale = cand_scale; p.bias_max = bias_max;
     p.acc_stages = kn.acc_stages == 1 ? 1 : 2;
     p.cand32 = cand32; p.cand16 = cand16; p.dim = dim;
     p.b_tx_bytes = b_stage / half_b;
@@ -1523,6 +1565,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     // callers always get the exact per-column masks (FFR_GRID_EXACT=1 forces them everywhere).
     p.grid_exact = kn.grid_exact >= 0 ? kn.grid_exact : 0;
     if (no_recheck || dbg_scores != nullptr) p.grid_exact = 1;
+    if (euclid) p.grid_exact = 0;                          // (K3 always runs behind the Euclid kernel)
     p.norm_ahead = kn.norm_ahead < 1 ? 1 : kn.norm_ahead;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const KParams);
@@ -1539,9 +1582,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     static const KernelFn instr1[4] = {FFR_K(1, 0, 2, 2, true), FFR_K(1, 1, 2, 2, true), FFR_K(1, 2, 2, 2, true), FFR_K(1, 3, 2, 2, true)};
 #undef FFR_K_POLICY
 #undef FFR_K
+    static const KernelFn euclid2[2] = {filter_mma_kernel<2, 0, 0, 0, false, true>, filter_mma_kernel<2, 0, 0, 1, false, true>};
     KernelFn fn;
-    if (cg == 2) fn = instr ? instr2[nm] : prod2[nm][(p.grid_exact ? 2 : 0) + (p.grid_updates ? 1 : 0)];
-    else         fn = instr ? instr1[nm] : prod1[nm];
+    if (euclid)       fn = euclid2[p.grid_updates ? 1 : 0];
+    else if (cg == 2) fn = instr ? instr2[nm] : prod2[nm][(p.grid_exact ? 2 : 0) + (p.grid_updates ? 1 : 0)];
+    else              fn = instr ? instr1[nm] : prod1[nm];
     // the opt-in to > 48 KB of dynamic shared memory is a per-DEVICE function attribute: set once per device this process uses
     {
         static std::mutex mu;
@@ -1556,6 +1601,8 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                 FFR_CUDA_TRY(cudaFuncSetAttribute(prod1[m], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
                 FFR_CUDA_TRY(cudaFuncSetAttribute(instr1[m], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
             }
+            for (int v = 0; v < 2; ++v)
+                FFR_CUDA_TRY(cudaFuncSetAttribute(euclid2[v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
             attr_set[slot] = true;
         }
     }
@@ -1609,10 +1656,11 @@ int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const 
                       int64_t n_cand, int32_t dim_pad,
                       float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                       RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
-                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s) {
+                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
+                      const float* euclid_bias, const float* cand_scale, const float* bias_max) {
     return launch_filter_mma_impl(ref16, n_ref, cand16, cand32, dim, n_cand, dim_pad, thr, delta, thr_band, ref_index_base,
                                   keep, idx, val, lists, no_recheck, BandArgs{band_tol, band_count, band_rows, band_cap}, nullptr,
-                                  after_k1, ref_map, n_ref_dev, s);
+                                  after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale, bias_max);
 }
 
 // true when the fused schedule needs NO fp16 copy of the candidates in the workspace (stage32: the fp16 A tiles only ever
@@ -1634,7 +1682,8 @@ int launch_filter_mma_debug(const __half* ref16, int64_t n_ref, const __half* ca
                             float thr, float delta, uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
                             float* scores, cudaStream_t s) {
     return launch_filter_mma_impl(ref16, n_ref, const_cast<__half*>(cand16), nullptr, dim_pad, n_cand, dim_pad, thr, delta, delta, 0, keep, idx,
-                                  val, lists, 0, BandArgs{0.f, nullptr, nullptr, 0}, scores, false, nullptr, nullptr, s);
+                                  val, lists, 0, BandArgs{0.f, nullptr, nullptr, 0}, scores, false, nullptr, nullptr, s,
+                                  nullptr, nullptr, nullptr);
 }
 
 }  // namespace ffr

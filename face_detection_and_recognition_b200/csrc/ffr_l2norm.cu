@@ -31,6 +31,7 @@ struct L2Second {
     __half* y16;
     uint32_t* zero_ptr;
     int32_t zero_words;
+    float* scale_a;           // optional: 1 / |x| of matrix a's rows (the Euclid filter's candidate scales)
 };
 
 template <int NV, int kRows>             // NV float4 per lane per row (dim == 128 * NV), kRows rows in flight per warp
@@ -71,6 +72,7 @@ l2norm_rows_vec_kernel(const float* __restrict__ x_a, int64_t rows_a, int32_t di
             ss = warp_sum(ss);
             const float nrm = sqrtf(ss);
             if (norms != nullptr && lane == 0) norms[r] = nrm;
+            if (sec.scale_a != nullptr && lane == 0 && r < rows_a) sec.scale_a[r] = __fdiv_rn(1.0f, nrm);
             __half* y16 = y16_a;
             int64_t ro = r;                                         // row inside its own matrix
             if (r >= rows_a) { y16 = sec.y16; ro = r - rows_a; }
@@ -142,6 +144,7 @@ l2norm_rows_sub_kernel(const float* __restrict__ x_a, int64_t rows_a, int32_t di
 #pragma unroll
             for (int o = L / 2; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
             const float inv = __fdiv_rn(1.0f, sqrtf(ss));
+            if (sec.scale_a != nullptr && sub == 0 && r < rows_a) sec.scale_a[r] = inv;
             if (r < rows) {
                 __half* y = (r < rows_a) ? y16_a + r * ld16 : sec.y16 + (r - rows_a) * ld16;
 #pragma unroll
@@ -179,6 +182,7 @@ l2norm_rows_generic_kernel(const float* __restrict__ x_a, int64_t rows_a, int32_
         ss = warp_sum(ss);
         const float nrm = sqrtf(ss);
         if (norms != nullptr && lane == 0) norms[r] = nrm;
+        if (sec.scale_a != nullptr && lane == 0 && !second) sec.scale_a[r] = __fdiv_rn(1.0f, nrm);
         for (int c = lane; c < ld16 || c < dim; c += 32) {
             const float o = c < dim ? __fdiv_rn(__ldg(p + c), nrm) : 0.f;
             if (y32 != nullptr && c < dim) y32[r * dim + c] = o;
@@ -236,15 +240,79 @@ static int launch_l2norm_impl(const float* x, int64_t rows, int32_t dim, __half*
 
 int launch_l2norm(const float* x, int64_t rows, int32_t dim, __half* y16, int32_t ld16, float* y32, float* norms,
                   cudaStream_t s) {
-    return launch_l2norm_impl(x, rows, dim, y16, ld16, y32, norms, L2Second{nullptr, 0, nullptr, nullptr, 0}, s);
+    return launch_l2norm_impl(x, rows, dim, y16, ld16, y32, norms, L2Second{nullptr, 0, nullptr, nullptr, 0, nullptr}, s);
 }
 
 // fp16 normalised copies of two matrices of the same width in one launch (either may be empty), plus zero_words 32-bit
 // zeros at zero_ptr (<= 256 words)
 int launch_l2norm_pair(const float* x_a, int64_t rows_a, __half* y16_a, const float* x_b, int64_t rows_b, __half* y16_b,
-                       int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s) {
+                       int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s, float* scale_a) {
     return launch_l2norm_impl(x_a, rows_a, dim, y16_a, ld16, nullptr, nullptr,
-                              L2Second{x_b, rows_b, y16_b, static_cast<uint32_t*>(zero_ptr), zero_words}, s);
+                              L2Second{x_b, rows_b, y16_b, static_cast<uint32_t*>(zero_ptr), zero_words, scale_a}, s);
+}
+
+// ---- Euclid references for the tensor-core filter (DESIGN.md section 4, "Euclid on the tensor cores") ----
+// argmin_i |c - r_i| = argmax_i (r_i.c - |r_i|^2 / 2).  K2 multiplies fp16(r * 2^-f) by the candidate's normalised fp16 row
+// and adds beta_i / |c|, beta_i = -|r_i|^2 * 2^-f / 2.  One power of two f per call, from the largest reference norm, keeps
+// |r * 2^-f| <= 1, so the fp16 operand error is bounded like the cosine score's.  The squares are summed in fp64 and rounded
+// once: beta then carries a single fp32 rounding, which is what K2's per-row window accounts for.
+// E1: one warp per row, |r_i|^2 and the running maximum (the bits of non-negative floats order like the floats).
+__global__ void __launch_bounds__(kThreads)
+euclid_ref_norms_kernel(const float* __restrict__ ref, int64_t n_ref, int32_t dim, float* __restrict__ nsq,
+                        uint32_t* __restrict__ max_bits) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
+    const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
+    for (int64_t r = warp; r < n_ref; r += nwarps) {
+        const float* p = ref + r * dim;
+        double ss = 0.0;
+        for (int c = lane; c < dim; c += 32) { const double t = __ldg(p + c); ss = fma(t, t, ss); }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
+        if (lane == 0) {
+            const float v = static_cast<float>(ss);
+            nsq[r] = v;
+            atomicMax(max_bits, __float_as_uint(v));
+        }
+    }
+}
+
+// E2: f = the smallest integer with 2^(2f) > max |r|^2; fp16(r * 2^-f) rows (zero K padding), beta (zero padded to a multiple
+// of 256 so that K2's reads of a partial reference tile stay inside the tensor), bmax = max |beta|.
+__global__ void __launch_bounds__(kThreads)
+euclid_ref_scale_kernel(const float* __restrict__ ref, int64_t n_ref, int32_t dim, int32_t ld16, __half* __restrict__ ref16,
+                        const float* __restrict__ nsq, const uint32_t* __restrict__ max_bits, float* __restrict__ beta,
+                        int64_t n_pad, float* __restrict__ bmax) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
+    const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
+    const float mx = __uint_as_float(*max_bits);
+    int e = 0;
+    if (mx > 0.f && mx <= 3.4e38f) frexpf(mx, &e);                     // mx < 2^e
+    const int f = (e + 1) >> 1;                                         // |r| < 2^(e/2) <= 2^f
+    const float sc = ldexpf(1.0f, -f);
+    if (blockIdx.x == 0 && threadIdx.x == 0) *bmax = 0.5f * (mx * sc);
+    for (int64_t r = warp; r < n_pad; r += nwarps) {
+        if (r >= n_ref) { if (lane == 0) beta[r] = 0.f; continue; }
+        const float* p = ref + r * dim;
+        __half* y = ref16 + r * ld16;
+        for (int c = lane; c < ld16; c += 32) y[c] = __float2half_rn(c < dim ? __ldg(p + c) * sc : 0.f);
+        if (lane == 0) beta[r] = -0.5f * (nsq[r] * sc);
+    }
+}
+
+int launch_euclid_refs(const float* ref, int64_t n_ref, int32_t dim, int32_t ld16, __half* ref16, float* beta, float* nsq,
+                       uint32_t* max_bits, float* bmax, cudaStream_t s) {
+    const int64_t n_pad = euclid_bias_len(n_ref);
+    int64_t grid = (n_pad + (kThreads / 32) - 1) / (kThreads / 32);
+    if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
+    FFR_CUDA_TRY(cudaMemsetAsync(max_bits, 0, sizeof(uint32_t), s));
+    euclid_ref_norms_kernel<<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, dim, nsq, max_bits);
+    FFR_LAUNCH_CHECK("euclid_ref_norms");
+    euclid_ref_scale_kernel<<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, dim, ld16, ref16, nsq, max_bits, beta,
+                                                                             n_pad, bmax);
+    FFR_LAUNCH_CHECK("euclid_ref_scale");
+    return FFR_OK;
 }
 
 }  // namespace ffr

@@ -8,6 +8,12 @@
 // on the ORIGINAL fp32 embeddings: only the two leading references when the third-best score was clearly
 // lower, the whole reference set otherwise (first-occurrence argmax, strict '>' in ascending order).
 // One warp per flagged row; the candidate row is parked in shared memory.
+//
+// Euclid form (kEuclid, the tcgen05 Euclid filter): the same lists, ranked by fp32 distance computed with direct differences
+// (c - r, never |c|^2 + |r|^2 - 2 c.r), smallest first, ties to the first index.  Only best_idx is written: keep, best_val and
+// the band come from the value pass that follows (ffr_filter_fp32.cu), which recomputes the winner's distance with K2s's
+// arithmetic.  The pairs, parts and few-row phases use k2s_euclid_dist in K2s's mode (`emode`); the tiled walk has its own
+// difference-and-square loop.
 #include <mutex>
 
 #include "ffr_common.cuh"
@@ -114,11 +120,30 @@ __device__ __forceinline__ void
 recheck_pairs_phase(float* s_rows, const float* __restrict__ ref, const float* __restrict__ cand, int32_t dim, float thr,
                     int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                     float* __restrict__ best_val, const RecheckLists& lists, float band_tol, int32_t* band_count,
-                    int64_t* band_rows, int64_t band_cap, bool vec) {
+                    int64_t* band_rows, int64_t band_cap, bool vec, int emode) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     float* c_smem = s_rows + static_cast<size_t>(w) * dim;
     const int64_t warp = static_cast<int64_t>(blockIdx.x) * kWarps + w;
     const int64_t nwarps = static_cast<int64_t>(gridDim.x) * kWarps;
+    if (emode >= 0) {                                           // Euclid: the one to three leading references by fp32 distance
+        int64_t count = lists.hdr->recheck_count;
+        if (count > lists.rec_cap) count = lists.rec_cap;
+        for (int64_t k = warp; k < count; k += nwarps) {
+            const RecheckRec rec = lists.recs[k];
+            const float* c = cand + static_cast<int64_t>(rec.row) * dim;
+            float best = k2s_euclid_dist(c, ref + static_cast<int64_t>(rec.idx1) * dim, dim, lane, emode);
+            int32_t bi = rec.idx1;
+            const int32_t more[2] = {rec.idx2, rec.idx2 >= 0 ? rec.idx3 : -1};
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                if (more[e] < 0) continue;
+                const float d = k2s_euclid_dist(c, ref + static_cast<int64_t>(more[e]) * dim, dim, lane, emode);
+                if (d < best || (d == best && more[e] < bi)) { best = d; bi = more[e]; }
+            }
+            if (lane == 0) best_idx[rec.row] = static_cast<int32_t>(bi + ref_index_base);
+        }
+        return;
+    }
     // the warp's first record is requested TOGETHER with the list length, not after it (it is only used when it exists):
     // with a short list the phase is one chain of dependent memory latencies, and this takes one L2 round trip out of it
     RecheckRec rec0{};
@@ -263,7 +288,7 @@ recheck_parts_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref,
                     float thr, int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                     float* __restrict__ best_val, const RecheckLists& lists, float band_tol, int32_t* band_count,
                     int64_t* band_rows, int64_t band_cap, bool vec, const int32_t* __restrict__ ref_map,
-                    const int32_t* __restrict__ n_unique_dev) {
+                    const int32_t* __restrict__ n_unique_dev, int emode) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     float* c_smem = s_rows + static_cast<size_t>(w) * dim;
     // records are dealt from the LAST warp of the grid downwards: with a short pairs list (dealt from warp 0 upwards) the two
@@ -283,6 +308,26 @@ recheck_parts_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref,
         const int ny = __popc(ym);
         const int n_in = __popc(xm) * ny;                         // candidate columns inside the part(s) (<= 256)
         const int n_all = n_in + (rec.idx2 >= 0 ? 1 : 0);         // + the tracked candidate outside it
+        if (emode >= 0) {                                         // Euclid: one reference at a time, the whole warp on it
+            const float* c = cand + static_cast<int64_t>(rec.row) * dim;
+            float best = INFINITY;
+            int32_t bi = 0x7FFFFFFF;
+            for (int e = 0; e < n_all; ++e) {
+                int64_t ri = -1;
+                if (e < n_in) {
+                    const int a = __fns(xm, 0, e / ny + 1), b = __fns(ym, 0, e % ny + 1);
+                    const int64_t col = col0 + 8 * a + b;
+                    if (col < n_cols) ri = ref_map != nullptr ? static_cast<int64_t>(__ldg(ref_map + col)) : col;
+                } else {
+                    ri = rec.idx2;
+                }
+                if (ri < 0) continue;
+                const float d = k2s_euclid_dist(c, ref + ri * dim, dim, lane, emode);
+                if (d < best || (d == best && ri < bi)) { best = d; bi = static_cast<int32_t>(ri); }
+            }
+            if (lane == 0 && bi != 0x7FFFFFFF) best_idx[rec.row] = static_cast<int32_t>(bi + ref_index_base);
+            continue;
+        }
         unsigned long long key = 0ull;
         // L lanes per reference (the embedding split between them): with the typical 2-8 references of a record most lanes
         // would idle and every lane would walk a whole row -- four times the dependent L2 round trips
@@ -390,7 +435,7 @@ __device__ __forceinline__ void
 rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim,
                    float thr, int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                    float* __restrict__ best_val, const RecheckLists& lists, int64_t count, float band_tol,
-                   int32_t* band_count, int64_t* band_rows, int64_t band_cap, bool vec) {
+                   int32_t* band_count, int64_t* band_rows, int64_t band_cap, bool vec, int emode) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     float* c_smem = s_rows + static_cast<size_t>(w) * dim;
     const int64_t nb = (n_ref + kSmallRefs - 1) / kSmallRefs;
@@ -423,10 +468,26 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
             int32_t bidx;
             unpack_key(key, v, bidx);
             if (key == 0ull) { v = -INFINITY; bidx = 0; }
-            emit_result(lists.full_rows[sl], v, bidx, thr, ref_index_base, keep, best_idx, best_val, band_tol,
-                        band_count, band_rows, band_cap);
+            if (emode >= 0) best_idx[lists.full_rows[sl]] = static_cast<int32_t>(bidx + ref_index_base);
+            else emit_result(lists.full_rows[sl], v, bidx, thr, ref_index_base, keep, best_idx, best_val, band_tol,
+                             band_count, band_rows, band_cap);
         }
     };
+    if (emode >= 0) {           // Euclid: score = -distance, so the key's "largest, then smallest index" is the first argmin
+        for (int64_t item = i0; item < i1; ++item) {
+            const int64_t slot = item / nb, blk = item - slot * nb;
+            if (slot != cur) { flush(); cur = slot; pending = 0; best = -INFINITY; bi = 0x7FFFFFFF; }
+            const float* c = cand + static_cast<int64_t>(lists.full_rows[slot]) * dim;
+            const int64_t lo = blk * kSmallRefs, hi = (lo + kSmallRefs < n_ref) ? lo + kSmallRefs : n_ref;
+            for (int64_t i = lo; i < hi; ++i) {
+                const float sc = -k2s_euclid_dist(c, ref + i * dim, dim, lane, emode);
+                if (sc > best) { best = sc; bi = static_cast<int32_t>(i); }
+            }
+            ++pending;
+        }
+        flush();
+        return;
+    }
     const int nvec = dim >> 2;
     if (vec && nvec <= 32) {
         // rows of <= 128 floats: one float4 per lane and row, all in registers, and the item's reference rows (which need no
@@ -509,13 +570,14 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
 
 // One launch re-checks everything K2 flagged: phase A = K3a (pairs list), phase B = K3b (full-rescan list; small or
 // tiled walk, chosen from the device-side count, uniform over the grid).  The phases touch disjoint rows.
-template <bool kVec>
+template <bool kVec, bool kEuclid>
 __global__ void __launch_bounds__(kThreads, 2)      // two CTAs per SM (<= 128 registers): the fixed grid of 2 x SMs is ONE wave
 recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim, float thr,
                int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                float* __restrict__ best_val, RecheckLists lists, float band_tol, int32_t* band_count,
                int64_t* band_rows, int64_t band_cap, const int32_t* __restrict__ ref_map,
-               const int32_t* __restrict__ n_unique_dev, int skip) {
+               const int32_t* __restrict__ n_unique_dev, int skip, int emode_arg) {
+    const int emode = kEuclid ? emode_arg : -1;           // K2s distance mode (Euclid), -1 = cosine
     extern __shared__ __align__(16) float s_c[];               // kFullGroup x dim candidate rows | staged reference tile
     __shared__ float s_ccs[kFullGroup];
     __shared__ unsigned long long s_key[kWarps][kFullGroup];
@@ -524,17 +586,17 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
     pdl_wait();                 // launched as K2's programmatic dependent: everything below reads K2's lists and outputs
     if (!(skip & 1))
         recheck_pairs_phase(s_c, ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
-                            band_rows, band_cap, kVec);
+                            band_rows, band_cap, kVec, emode);
     if (!(skip & 2))
         recheck_parts_phase(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
-                            band_rows, band_cap, kVec, ref_map, n_unique_dev);
+                            band_rows, band_cap, kVec, ref_map, n_unique_dev, emode);
     if (skip & 4) return;
     int64_t count = lists.hdr->full_count;
     if (count > lists.full_cap) count = lists.full_cap;
     if (count == 0) return;
     if (static_cast<long long>(count) * n_ref * dim <= kSmallElems) {
         rescan_small_phase(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, count, band_tol,
-                           band_count, band_rows, band_cap, kVec);
+                           band_count, band_rows, band_cap, kVec, emode);
         return;
     }
     __syncthreads();                                            // phase A's per-warp rows are dead: the tiled walk reuses s_c
@@ -647,8 +709,10 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                         for (int r = 0; r < kRefsPerThread; ++r) {
                             const float4 t = *reinterpret_cast<const float4*>(s_r + (threadIdx.x + r * kThreads) * kKCPad + j4 * 4);
                             rv[r][0] = t.x; rv[r][1] = t.y; rv[r][2] = t.z; rv[r][3] = t.w;
-                            rr[r] = fmaf(t.x, t.x, rr[r]); rr[r] = fmaf(t.y, t.y, rr[r]);
-                            rr[r] = fmaf(t.z, t.z, rr[r]); rr[r] = fmaf(t.w, t.w, rr[r]);
+                            if (!kEuclid) {
+                                rr[r] = fmaf(t.x, t.x, rr[r]); rr[r] = fmaf(t.y, t.y, rr[r]);
+                                rr[r] = fmaf(t.z, t.z, rr[r]); rr[r] = fmaf(t.w, t.w, rr[r]);
+                            }
                         }
 #pragma unroll
                         for (int kk = 0; kk < 4; ++kk) {
@@ -662,8 +726,17 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
 #pragma unroll
                             for (int r = 0; r < kRefsPerThread; ++r) {
                                 const float2 r2 = make_float2(rv[r][kk], rv[r][kk]);
+                                if (kEuclid) {                  // d = c - r (one rounding, as a subtraction), then d * d
+                                    const float2 m1 = make_float2(-1.0f, -1.0f);
 #pragma unroll
-                                for (int pj = 0; pj < kFullGroup / 2; ++pj) acc[r][pj] = __ffma2_rn(cp[pj], r2, acc[r][pj]);
+                                    for (int pj = 0; pj < kFullGroup / 2; ++pj) {
+                                        const float2 d = __ffma2_rn(r2, m1, cp[pj]);
+                                        acc[r][pj] = __ffma2_rn(d, d, acc[r][pj]);
+                                    }
+                                } else {
+#pragma unroll
+                                    for (int pj = 0; pj < kFullGroup / 2; ++pj) acc[r][pj] = __ffma2_rn(cp[pj], r2, acc[r][pj]);
+                                }
                             }
                         }
                     }
@@ -677,7 +750,7 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
 #pragma unroll
                             for (int j = 0; j < kFullGroup; ++j) {
                                 const float dot = (j & 1) ? acc[r][j >> 1].y : acc[r][j >> 1].x;
-                                const float sc = __fdiv_rn(dot, __fmul_rn(rs, s_ccs[j]));
+                                const float sc = kEuclid ? -__fsqrt_rn(dot) : __fdiv_rn(dot, __fmul_rn(rs, s_ccs[j]));
                                 if (sc > best[j]) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
                             }
                         }
@@ -697,12 +770,15 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                     const float rv = __ldg(r + k);
                     rr = fmaf(rv, rv, rr);
 #pragma unroll
-                    for (int j = 0; j < kFullGroup; ++j) acc[j] = fmaf(s_c[j * dim + k], rv, acc[j]);
+                    for (int j = 0; j < kFullGroup; ++j) {
+                        if (kEuclid) { const float d = s_c[j * dim + k] - rv; acc[j] = fmaf(d, d, acc[j]); }
+                        else acc[j] = fmaf(s_c[j * dim + k], rv, acc[j]);
+                    }
                 }
                 const float rs = __fsqrt_rn(rr);
 #pragma unroll
                 for (int j = 0; j < kFullGroup; ++j) {
-                    const float sc = __fdiv_rn(acc[j], __fmul_rn(rs, s_ccs[j]));
+                    const float sc = kEuclid ? -__fsqrt_rn(acc[j]) : __fdiv_rn(acc[j], __fmul_rn(rs, s_ccs[j]));
                     if (sc > best[j]) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
                 }
             }
@@ -740,8 +816,9 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                 unpack_key(key, v, bi);
                 if (key == 0ull) { v = -INFINITY; bi = 0; }
                 else if (ref_map != nullptr) bi = __ldg(ref_map + bi);          // compact column -> original reference
-                emit_result(lists.full_rows[slot], v, bi, thr, ref_index_base, keep, best_idx, best_val, band_tol,
-                            band_count, band_rows, band_cap);
+                if (kEuclid) best_idx[lists.full_rows[slot]] = static_cast<int32_t>(bi + ref_index_base);
+                else emit_result(lists.full_rows[slot], v, bi, thr, ref_index_base, keep, best_idx, best_val, band_tol,
+                                 band_count, band_rows, band_cap);
             }
         }
     }
@@ -777,8 +854,9 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
                    const float* /*ref_norm*/, const float* /*cand_norm*/, float thr, int64_t ref_index_base,
                    uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s) {
+                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode) {
     if (n_cand == 0) return FFR_OK;
+    const bool euclid = euclid_mode >= 0;
     static_assert(kFullGroup % kWarps == 0, "every warp parks kFullGroup / kWarps candidate rows of a full-rescan group");
     const int sms = num_sms();
     // kFullGroup parked candidate rows (the per-warp phases use the first kWarps of them)
@@ -795,8 +873,10 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
         const int slot = current_device_slot();
         std::lock_guard<std::mutex> lock(mu);
         if (!attr_set[slot]) {
-            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
-            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
             attr_set[slot] = true;
         }
     }
@@ -811,10 +891,10 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
     cfg.attrs = attr;
     cfg.numAttrs = (knobs().pdl & 2) != 0 ? 1 : 0;        // FFR_PDL bit 1 (bit 0: K1 -> K2)
     const int skip = knobs().k3_skip;                     // timing experiments only (FFR_K3_SKIP: phases left out, WRONG results)
-    if (vec) FFR_CUDA_TRY(cudaLaunchKernelEx(&cfg, recheck_kernel<true>, ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val,
-                                             lists, band_tol, band_count, band_rows, band_cap, ref_map, n_unique_dev, skip));
-    else     FFR_CUDA_TRY(cudaLaunchKernelEx(&cfg, recheck_kernel<false>, ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val,
-                                             lists, band_tol, band_count, band_rows, band_cap, ref_map, n_unique_dev, skip));
+    auto* fn = euclid ? (vec ? recheck_kernel<true, true> : recheck_kernel<false, true>)
+                      : (vec ? recheck_kernel<true, false> : recheck_kernel<false, false>);
+    FFR_CUDA_TRY(cudaLaunchKernelEx(&cfg, fn, ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val, lists, band_tol,
+                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, skip, euclid_mode));
     FFR_LAUNCH_CHECK("recheck");
     return FFR_OK;
 }

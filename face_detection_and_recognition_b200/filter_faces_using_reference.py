@@ -10,6 +10,7 @@ per-class summary line (reference :198-199).  What changes is where the arithmet
   np.mean / max_i np.linalg.norm(mu - ref_i)          :85-99         ffr_ref_mean_and_thres        (K5)
   np.linalg.norm(out - mu) <= thres per row           :186-189       ffr_filter metric=euclid N=1  (K2s, fp32)
   (new) gallery mode: all reference embeddings, cosine + threshold   ffr_filter metric=cosine      (K1+K2+K3, tcgen05)
+  (new) gallery mode, --metric euclid: smallest distance <= threshold ffr_filter metric=euclid     (K1+K2+K3, tcgen05)
 
 Embedding extraction stays in the reference's own PyTorch ``MobileFaceNet`` (imported from the reference
 checkout, never copied): ``-m`` is reinterpreted as the path of its state dict.  Any object with
@@ -222,9 +223,12 @@ def get_parsed_args(argv=None):
                         help='Number of reference images to consider per class: %(default)s)')
     # optional additions (defaults reproduce the reference's behaviour)
     parser.add_argument('--gallery', action='store_true',
-                        help='match every candidate against ALL reference embeddings (cosine, tensor cores) instead of '
+                        help='match every candidate against ALL reference embeddings (tensor cores) instead of '
                              'the class mean vector')
-    parser.add_argument('--threshold', type=float, default=0.5, help='cosine threshold of --gallery mode')
+    parser.add_argument('--metric', choices=['cosine', 'euclid'], default='cosine',
+                        help='decision rule of --gallery mode: best cosine >= threshold, or smallest Euclid distance <= threshold')
+    parser.add_argument('--threshold', type=float, default=0.5,
+                        help='threshold of --gallery mode: a cosine similarity, or a distance with --metric euclid')
     parser.add_argument('--mobilefacenet_dir', type=str,
                         default=os.environ.get("FFR_MOBILEFACENET_DIR",
                                                "../face_detection_and_extraction/modules/mobile_facenet"))
@@ -238,9 +242,10 @@ def get_parsed_args(argv=None):
 
 def filter_class(model, ref_class_path: str, unfiltered_class_path: str, clean_dir: str, unclean_dir: str,
                  batch_size: int = 32, ref_img_per_class: int = 32, gallery: bool = False, threshold: float = 0.5,
-                 device: str = "cuda:0", ref_stats=None):
+                 device: str = "cuda:0", ref_stats=None, metric: str = "cosine"):
     """One iteration of the reference's per-class loop (:161-199).  Returns (similar_cnt, total, keep mask).
-    ``ref_stats`` = (mean [1, D] CUDA, thres float) when the caller computed all classes' statistics up front."""
+    ``ref_stats`` = (mean [1, D] CUDA, thres float) when the caller computed all classes' statistics up front; ``metric`` is the
+    decision rule of gallery mode."""
     dev = torch.device(device)
     cls = unfiltered_class_path.split('/')[-1]
     filtered_class_clean_dir = os.path.join(clean_dir, cls)
@@ -252,7 +257,7 @@ def filter_class(model, ref_class_path: str, unfiltered_class_path: str, clean_d
     if gallery:
         ref_imgs = sorted(glob.glob(ref_class_path + "/*.jpg"))[:ref_img_per_class]
         ref = _embed_paths_device(model, ref_imgs, batch_size, dev)
-        thr, metric = threshold, "cosine"
+        thr = threshold
     elif ref_stats is not None:
         ref, thr, metric = ref_stats[0].reshape(1, -1), float(ref_stats[1]), "euclid"
     else:
@@ -335,7 +340,7 @@ def main(argv=None, model=None, model_factory=None):
         for k, i in enumerate(indices):
             similar_cnt, total, _ = filter_class(mdl, ref_class_paths[i], unfiltered_class_paths[i], clean_dir, unclean_dir,
                                                  batch_size=args.batch_size, ref_img_per_class=args.ref_img_per_class,
-                                                 gallery=args.gallery, threshold=args.threshold, device=device,
+                                                 gallery=args.gallery, threshold=args.threshold, device=device, metric=args.metric,
                                                  ref_stats=None if stats is None else stats[k])
             # the reference divides unconditionally (ZeroDivisionError on an empty class, :199); keep that behaviour
             lines[i] = f"Similar images percentage={similar_cnt/total:2.2f}%, positive={similar_cnt}, total={total}"

@@ -104,7 +104,11 @@ def face_filter(ref: torch.Tensor, cand: torch.Tensor, thr: float, metric="cosin
     cosine: best = max_i cos(r_i, c), keep = best >= thr;  euclid: best = min_i |c - r_i|, keep = best <= thr.
     ``ref`` [N, D], ``cand`` [M, D]: float32 CUDA tensors (raw embeddings; normalisation is internal), or both
     float16 rows produced by ``l2norm_rows(want_f16=True)`` (cosine only).  ``band_tol`` additionally returns
-    the rows whose best lies within that tolerance of ``thr``."""
+    the rows whose best lies within that tolerance of ``thr``.
+
+    Both metrics use the tensor cores from 9 references up (dim <= 512).  Euclid then returns the index of the exact fp32
+    kernel (``FLAG_FORCE_FP32``) except on fp32 ties (two smallest distances within 1e-6 relative), and the same keep and
+    distance bit for bit wherever the index agrees; with ``FLAG_NO_RECHECK`` Euclid runs the exact kernel."""
     lib = _lib.load()
     m = _METRICS[metric]
     if ref.dtype == torch.float16:

@@ -52,7 +52,7 @@ extern "C" {
 
 /* flags for ffr_filter_ex */
 #define FFR_FLAG_FORCE_FP32   1  /* use the exact fp32 CUDA-core kernel whatever the shape */
-#define FFR_FLAG_FORCE_MMA    2  /* use the tcgen05 kernel (cosine, dim <= 512) whatever n_ref */
+#define FFR_FLAG_FORCE_MMA    2  /* use the tcgen05 kernel (dim <= 512) whatever n_ref (euclid: n_ref > 8 still required) */
 #define FFR_FLAG_NO_RECHECK   4  /* skip the fp32 re-check of near-tie / near-threshold rows (benchmarking only): decisions as for FFR_DTYPE_F16 */
 
 typedef void* ffr_stream_t;      /* cudaStream_t */
@@ -92,7 +92,13 @@ int ffr_l2norm_rows_f32(const float* x, int64_t rows, int32_t dim,
  * (unordered) to band_rows[0..band_cap) and counted in *band_count (device int32; count may exceed cap); `best` is the
  * fp32 re-checked score, or the fp16-operand score where no re-check runs (FFR_DTYPE_F16, FFR_FLAG_NO_RECHECK).
  * Bit-identical reference rows are folded internally (a later copy can never be the first arg-best); best_idx always
- * refers to the caller's row numbering. */
+ * refers to the caller's row numbering.
+ * Euclid on the tensor cores: with n_ref > 8, dim <= 512, FFR_DTYPE_F32, the re-check on (no FFR_FLAG_NO_RECHECK, no
+ * FFR_FLAG_FORCE_FP32) and a GPU whose SMs pair up (cta_group::2), euclid runs K1 + K2 (fp16 dot products plus a per-reference
+ * bias) + K3 (fp32 distances of the near ties) + a value pass; otherwise the exact fp32 kernel K2s.  Contract: best_idx equals
+ * the FFR_FLAG_FORCE_FP32 result except on rows whose two smallest distances differ by < 1e-6 relative (fp32 ties); keep and
+ * best_val are bit-identical to it wherever best_idx agrees; the band list is exact.  FFR_DTYPE_F16 rows are refused for
+ * euclid (FFR_ERR_UNSUPPORTED). */
 size_t ffr_filter_workspace_bytes(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, int metric);
 
 int ffr_filter(const void* ref, int64_t n_ref, const void* cand, int64_t n_cand, int32_t dim, int dtype,
