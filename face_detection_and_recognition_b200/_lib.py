@@ -17,6 +17,8 @@ ERR_NAMES = {-1: "FFR_ERR_INVALID", -2: "FFR_ERR_CUDA", -3: "FFR_ERR_WORKSPACE",
 METRIC_COSINE, METRIC_EUCLID = 0, 1
 DTYPE_F32, DTYPE_F16 = 0, 1
 FLAG_FORCE_FP32, FLAG_FORCE_MMA, FLAG_NO_RECHECK = 1, 2, 4
+SELF_OTHERS, SELF_EARLIER = 0, 1
+ERR_INVALID, ERR_UNSUPPORTED = -1, -4
 
 
 class FfrError(RuntimeError):
@@ -40,6 +42,9 @@ SIGNATURES = {
                              _vp, _sz, _vp]),
     "ffr_filter_ex": (C.c_int, [_vp, _i64, _vp, _i64, _i32, C.c_int, _vp, _vp, C.c_int, _f32, _i64, _vp, _vp, _vp,
                                 _f32, _vp, _vp, _i64, C.c_int, _vp, _sz, _vp]),
+    "ffr_filter_self_workspace_bytes": (_sz, [_i64, _i64, _i32, C.c_int]),
+    "ffr_filter_self": (C.c_int, [_vp, _i64, _i64, _i64, _i32, C.c_int, C.c_int, _f32, _vp, _vp, _vp,
+                                  _f32, _vp, _vp, _i64, C.c_int, _vp, _sz, _vp]),
     "ffr_filter_stats": (C.c_int, [_vp, C.POINTER(_i64), _vp]),
     "ffr_ref_mean_and_thres": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "ffr_ref_mean_and_thres_batched": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp]),

@@ -328,6 +328,101 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
     return FFR_OK;
 }
 
+// Self mode (ffr_filter_self): x is both matrices.  K1 normalises x ONCE and, for cosine, the A operand is the candidates' slice
+// of that same fp16 copy (kNormMode 0: stage32 or the fused scratch would only read or write those rows a second time).  Euclid
+// keeps its operands: E1/E2 turn all n rows into the B operand and its bias, K1 over the slice writes the normalised A rows and
+// 1 / |c|.  No duplicate fold: bit-identical rows are what the caller looks for.
+bool self_mma_eligible(int64_t n, int32_t dim, int flags) {
+    return !(flags & FFR_FLAG_FORCE_FP32) && dim <= 512 && n > 8 && euclid_mma_available();
+}
+
+WsLayout self_ws_layout(int64_t n, int64_t n_rows, int32_t dim, int metric, bool mma) {
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    return ws_layout(n, n_rows, dim, FFR_DTYPE_F32, mma, /*need_c16=*/euclid, /*dedup=*/false, mma && euclid);
+}
+
+int self_core(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, int mode, float thr,
+              uint8_t* keep, int32_t* best_idx, float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows,
+              int64_t band_cap, int flags, void* workspace, size_t ws_bytes, cudaStream_t s) {
+    const bool mma = self_mma_eligible(n, dim, flags);
+    if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
+        set_error("FFR_FLAG_FORCE_MMA: the self-mode tcgen05 path needs n > 8, dim <= 512 and cta_group::2 (n=%lld dim=%d)",
+                  (long long)n, dim);
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    const WsLayout L = self_ws_layout(n, n_rows, dim, metric, mma);
+    if (workspace == nullptr || ws_bytes < L.total) {
+        set_error("workspace too small: need %zu bytes, got %zu", L.total, workspace ? ws_bytes : (size_t)0);
+        return FFR_ERR_WORKSPACE;
+    }
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) { set_error("workspace must be 256-byte aligned"); return FFR_ERR_INVALID; }
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    WsHeader* hdr = reinterpret_cast<WsHeader*>(ws + L.hdr);
+    g_last = {workspace, mma ? 1 : 0, 0};
+    if (band_count != nullptr) FFR_CUDA_TRY(cudaMemsetAsync(band_count, 0, sizeof(int32_t), s));
+    if (!(mma && n_rows > 0)) FFR_CUDA_TRY(cudaMemsetAsync(hdr, 0, sizeof(WsHeader), s));     // (otherwise K1 zeroes it)
+    if (n_rows == 0) return FFR_OK;
+    const SelfArgs self{row_begin, mode};
+    if (!mma) {
+        g_last.launches = 1;
+        return launch_filter_fp32_self(x, n, n_rows, dim, metric, self, thr, keep, best_idx, best_val, band_tol, band_count,
+                                       band_rows, band_cap, s);
+    }
+    const int32_t ld = ffr_padded_dim(dim);
+    const float* cand = x + row_begin * dim;
+    __half* x16 = reinterpret_cast<__half*>(ws + L.ref16);
+    __half* c16 = nullptr;
+    const float *e_bias = nullptr, *e_bmax = nullptr;
+    float* e_cscale = nullptr;
+    int rc, launches = 0;
+    const int32_t hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
+    if (euclid) {
+        float* bias = reinterpret_cast<float*>(ws + L.e_bias);
+        float* scal = reinterpret_cast<float*>(ws + L.e_scal);
+        rc = launch_euclid_refs(x, n, dim, ld, x16, bias, reinterpret_cast<float*>(ws + L.e_nsq), reinterpret_cast<uint32_t*>(scal),
+                                scal + 1, s);
+        if (rc != FFR_OK) return rc;
+        c16 = reinterpret_cast<__half*>(ws + L.cand16);
+        e_cscale = reinterpret_cast<float*>(ws + L.e_cscale);
+        rc = launch_l2norm_pair(cand, n_rows, c16, nullptr, 0, nullptr, dim, ld, hdr, hdr_words, s, e_cscale);
+        if (rc != FFR_OK) return rc;
+        launches += 3;
+        e_bias = bias; e_bmax = scal + 1;
+    } else {
+        rc = launch_l2norm_pair(x, n, x16, nullptr, 0, nullptr, dim, ld, hdr, hdr_words, s);
+        if (rc != FFR_OK) return rc;
+        ++launches;
+        c16 = x16 + row_begin * ld;
+    }
+    g_last.launches = launches + 2 + (euclid ? 1 : 0);
+    RecheckLists lists;
+    lists.hdr = hdr;
+    lists.recs = reinterpret_cast<RecheckRec*>(ws + L.recs);
+    lists.rec_cap = n_rows;
+    lists.full_rows = reinterpret_cast<int32_t*>(ws + L.full_rows);
+    lists.full_keys = reinterpret_cast<unsigned long long*>(ws + L.full_keys);
+    lists.full_ctr = reinterpret_cast<int32_t*>(ws + L.full_ctr);
+    lists.full_cap = n_rows;
+    const float delta = recheck_delta();
+    float thr_band = delta;
+    if (band_count != nullptr && band_tol + delta > thr_band) thr_band = band_tol + delta;
+    if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
+    rc = launch_filter_mma(x16, n, c16, nullptr, dim, n_rows, ld, euclid ? -INFINITY : thr, delta, euclid ? 0.f : thr_band, 0,
+                           keep, best_idx, best_val, lists, 0, band_tol, nullptr, band_rows, band_cap, /*after_k1=*/true,
+                           nullptr, nullptr, s, e_bias, e_cscale, e_bmax, self);
+    if (rc != FFR_OK) return rc;
+    if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
+    const int emode = euclid ? k2s_dist_mode_gallery(x, cand, dim) : -1;
+    rc = launch_recheck(x, n, cand, n_rows, dim, nullptr, nullptr, thr, 0, keep, best_idx, best_val, lists, band_tol,
+                        euclid ? nullptr : band_count, band_rows, band_cap, nullptr, nullptr, s, emode, self);
+    if (rc != FFR_OK) return rc;
+    if (euclid)
+        return launch_euclid_values(x, cand, n_rows, dim, thr, 0, keep, best_idx, best_val, band_tol, band_count, band_rows,
+                                    band_cap, emode, s, /*self=*/true);
+    return FFR_OK;
+}
+
 }  // namespace
 }  // namespace ffr
 
@@ -407,6 +502,33 @@ int ffr_filter(const void* ref, int64_t n_ref, const void* cand, int64_t n_cand,
                ffr_stream_t stream) {
     return ffr_filter_ex(ref, n_ref, cand, n_cand, dim, dtype, ref_norm, cand_norm, metric, thr, ref_index_base, keep,
                          best_idx, best_val, 0.f, nullptr, nullptr, 0, 0, workspace, ws_bytes, stream);
+}
+
+size_t ffr_filter_self_workspace_bytes(int64_t n, int64_t n_rows, int32_t dim, int metric) {
+    if (n <= 0 || n_rows < 0 || dim <= 0) return 0;
+    return self_ws_layout(n, n_rows, dim, metric, dim <= 512 && n > 8).total;     // sized for the tcgen05 path whenever it could run
+}
+
+int ffr_filter_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, int mode,
+                    float thr, uint8_t* keep, int32_t* best_idx, float* best_val,
+                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
+                    int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream) {
+    if (n <= 0) { set_error("n must be > 0 (got %lld)", (long long)n); return FFR_ERR_INVALID; }
+    if (dim <= 0) { set_error("dim must be > 0 (got %d)", dim); return FFR_ERR_INVALID; }
+    if (row_begin < 0 || n_rows < 0 || row_begin > n - n_rows) {
+        set_error("row range [%lld, %lld) is not inside [0, %lld)", (long long)row_begin, (long long)(row_begin + n_rows), (long long)n);
+        return FFR_ERR_INVALID;
+    }
+    if (x == nullptr || (n_rows > 0 && (keep == nullptr || best_idx == nullptr))) { set_error("null pointer argument"); return FFR_ERR_INVALID; }
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) { set_error("unknown metric %d", metric); return FFR_ERR_INVALID; }
+    if (mode != FFR_SELF_OTHERS && mode != FFR_SELF_EARLIER) { set_error("unknown self mode %d", mode); return FFR_ERR_INVALID; }
+    if (flags & FFR_FLAG_NO_RECHECK) {
+        set_error("FFR_FLAG_NO_RECHECK is not supported in self mode (the fp32 re-check decides the masked rows)");
+        return FFR_ERR_UNSUPPORTED;
+    }
+    if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
+    return self_core(x, n, row_begin, n_rows, dim, metric, mode, thr, keep, best_idx, best_val, band_tol, band_count, band_rows,
+                     band_cap, flags, workspace, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 int ffr_filter_stats(const void* workspace, int64_t out[8], ffr_stream_t stream) {

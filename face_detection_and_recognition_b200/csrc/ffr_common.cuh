@@ -79,8 +79,20 @@ struct WsHeader {
     int32_t pad[58];
 };
 
+// Self mode (ffr_filter_self): the candidates are rows [row0, row0 + n_cand) of the reference matrix itself, and candidate row g
+// (global index) may not match reference i == g (FFR_SELF_OTHERS) or any i >= g (FFR_SELF_EARLIER).  mode < 0: gallery call.
+struct SelfArgs {
+    int64_t row0;
+    int mode;
+};
+constexpr SelfArgs kNoSelf = {0, -1};
+
 // ---- device helpers -------------------------------------------------------------------------------
 #ifdef __CUDACC__
+
+__device__ __forceinline__ bool self_eligible(int64_t i, int64_t g, int mode) {
+    return i >= 0 && (mode == FFR_SELF_EARLIER ? i < g : i != g);
+}
 
 // ---- programmatic dependent launch (K1 -> K2 -> K3 without launch gaps) ----
 // pdl_launch_dependents: the NEXT kernel of the stream (if it was launched with the programmatic-serialisation attribute)
@@ -321,6 +333,10 @@ int launch_l2norm(const float* x, int64_t rows, int32_t dim, __half* y16, int32_
 int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric,
                        float thr, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                        float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s);
+// K2s self form: candidates x[self.row0 .. self.row0 + n_cand) against all n rows of x, excluded references skipped
+int launch_filter_fp32_self(const float* x, int64_t n, int64_t n_cand, int32_t dim, int metric, SelfArgs self, float thr,
+                            uint8_t* keep, int32_t* idx, float* val, float band_tol, int32_t* band_count, int64_t* band_rows,
+                            int64_t band_cap, cudaStream_t s);
 int launch_l2norm_pair(const float* x_a, int64_t rows_a, __half* y16_a, const float* x_b, int64_t rows_b, __half* y16_b,
                        int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s,
                        float* scale_a = nullptr);
@@ -336,7 +352,8 @@ int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const 
                       float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                       RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
                       int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
-                      const float* euclid_bias = nullptr, const float* cand_scale = nullptr, const float* bias_max = nullptr);
+                      const float* euclid_bias = nullptr, const float* cand_scale = nullptr, const float* bias_max = nullptr,
+                      SelfArgs self = kNoSelf);
 // exact-duplicate reference rows folded before K2 (ffr_dedup.cu)
 bool dedup_wanted(int64_t n_ref, int64_t n_cand);
 size_t dedup_workspace_bytes(int64_t n_ref, int32_t ld);
@@ -349,11 +366,12 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
                    const float* ref_norm, const float* cand_norm, float thr, int64_t ref_index_base,
                    uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode = -1);
+                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode = -1,
+                   SelfArgs self = kNoSelf);
 // Euclid after the tensor-core pass: keep / best_val / band from the K2s distance to the chosen reference (ffr_filter_fp32.cu)
 int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
                          uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
-                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s);
+                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s, bool self = false);
 int launch_ref_stats_batched(const float* ref_feat, const int32_t* offsets, int32_t n_classes, int32_t dim, float* mean,
                              float* thres, cudaStream_t s);
 int launch_first_match_stream(float* g_feat, float* g_bbox, int32_t* g_count, int32_t cap, const float* queries,

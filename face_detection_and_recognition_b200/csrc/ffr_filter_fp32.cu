@@ -73,13 +73,15 @@ __device__ __forceinline__ void load_row(const float* __restrict__ base, int32_t
     }
 }
 
-// rows: optional indirection (row_list[k] = candidate row to process), used by the recheck fallback
-template <int NV, bool kCosine, int kRegRefs>
+// kSelf (ffr_filter_self, kRegRefs 0): cand = rows [self.row0, ...) of ref; candidate row g skips reference g
+// (FFR_SELF_OTHERS) or every reference >= g (FFR_SELF_EARLIER); a row with none left gets index -1 and -inf / +inf
+template <int NV, bool kCosine, int kRegRefs, bool kSelf = false>
 __global__ void __launch_bounds__(kThreads)
 filter_fp32_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int64_t n_cand,
                    int32_t dim, float thr, int64_t ref_index_base,
                    uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
-                   BandOut band) {
+                   BandOut band, SelfArgs self) {
+    static_assert(!kSelf || kRegRefs == 0, "self form: references from global memory");
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
@@ -115,7 +117,7 @@ filter_fp32_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __
             cc_sqrt = __fsqrt_rn(warp_sum(cc));
         }
         float best = kCosine ? -INFINITY : INFINITY;
-        int32_t bi = 0;
+        int32_t bi = kSelf ? -1 : 0;
         if (kRegRefs > 0) {
 #pragma unroll
             for (int i = 0; i < kRegRefs; ++i) {
@@ -127,17 +129,20 @@ filter_fp32_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __
                 }
             }
         } else {
-            for (int64_t i = 0; i < n_ref; ++i) {
+            const int64_t g = self.row0 + row;
+            const int64_t i_end = kSelf && self.mode == FFR_SELF_EARLIER ? g : n_ref;
+            for (int64_t i = 0; i < i_end; ++i) {
+                if (kSelf && i == g) continue;
                 float4 r[NV];
                 load_row<NV>(ref + i * dim, dim, lane, r, false);
                 float s;
                 score_row<NV, kCosine>(c, r, cc_sqrt, s);
                 const bool better = kCosine ? (s > best) : (s < best);
-                if (better || i == 0) { best = s; bi = static_cast<int32_t>(i); }
+                if (better || (kSelf ? bi < 0 : i == 0)) { best = s; bi = static_cast<int32_t>(i); }
             }
         }
         if (lane == 0) {
-            const bool k = kCosine ? (best >= thr) : (best <= thr);
+            const bool k = (kCosine ? (best >= thr) : (best <= thr)) && (!kSelf || bi >= 0);
             keep[row] = k ? 1 : 0;
             best_idx[row] = static_cast<int32_t>(bi + ref_index_base);
             if (best_val != nullptr) best_val[row] = best;
@@ -246,13 +251,13 @@ filter_fp32_sub_kernel(const float* __restrict__ ref, int32_t n_ref, const float
     }
 }
 
-// catch-all: any dim / alignment; one warp per candidate, scalar loads
-template <bool kCosine>
+// catch-all: any dim / alignment; one warp per candidate, scalar loads (kSelf: as filter_fp32_kernel)
+template <bool kCosine, bool kSelf = false>
 __global__ void __launch_bounds__(kThreads)
 filter_fp32_generic_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand,
                            int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
                            uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
-                           BandOut band) {
+                           BandOut band, SelfArgs self) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
@@ -265,8 +270,11 @@ filter_fp32_generic_kernel(const float* __restrict__ ref, int64_t n_ref, const f
             cc_sqrt = __fsqrt_rn(warp_sum(cc));
         }
         float best = kCosine ? -INFINITY : INFINITY;
-        int32_t bi = 0;
-        for (int64_t i = 0; i < n_ref; ++i) {
+        int32_t bi = kSelf ? -1 : 0;
+        const int64_t g = self.row0 + row;
+        const int64_t i_end = kSelf && self.mode == FFR_SELF_EARLIER ? g : n_ref;
+        for (int64_t i = 0; i < i_end; ++i) {
+            if (kSelf && i == g) continue;
             const float* r = ref + i * dim;
             float a = 0.f, b = 0.f;
             for (int k = lane; k < dim; k += 32) {
@@ -279,10 +287,10 @@ filter_fp32_generic_kernel(const float* __restrict__ ref, int64_t n_ref, const f
             if (kCosine) { b = warp_sum(b); s = __fdiv_rn(a, __fmul_rn(__fsqrt_rn(b), cc_sqrt)); }
             else s = __fsqrt_rn(a);
             const bool better = kCosine ? (s > best) : (s < best);
-            if (better || i == 0) { best = s; bi = static_cast<int32_t>(i); }
+            if (better || (kSelf ? bi < 0 : i == 0)) { best = s; bi = static_cast<int32_t>(i); }
         }
         if (lane == 0) {
-            const bool k = kCosine ? (best >= thr) : (best <= thr);
+            const bool k = (kCosine ? (best >= thr) : (best <= thr)) && (!kSelf || bi >= 0);
             keep[row] = k ? 1 : 0;
             best_idx[row] = static_cast<int32_t>(bi + ref_index_base);
             if (best_val != nullptr) best_val[row] = best;
@@ -326,7 +334,8 @@ ref_stats_kernel(const float* __restrict__ x, int32_t n, int32_t dim, float* __r
 // exactly the arithmetic K2s uses for the same (row, reference) pair (k2s_euclid_dist in K2s's mode for n_ref > 2), so keep and
 // best_val are bit-identical to the FFR_FLAG_FORCE_FP32 result wherever the index agrees.  One warp per row; HBM-bound (one
 // read of the candidate matrix, the winners' rows mostly from L2).
-template <int kMode>
+// kSelf: a row without an eligible reference (best_idx -1) gets keep 0 and +inf, and never enters the band
+template <int kMode, bool kSelf = false>
 __global__ void __launch_bounds__(kThreads)
 euclid_value_kernel(const float* __restrict__ ref, const float* __restrict__ cand, int64_t n_cand, int32_t dim, float thr,
                     int64_t ref_index_base, uint8_t* __restrict__ keep, const int32_t* __restrict__ best_idx,
@@ -336,6 +345,12 @@ euclid_value_kernel(const float* __restrict__ ref, const float* __restrict__ can
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
     for (int64_t row = warp; row < n_cand; row += nwarps) {
         const int64_t ri = static_cast<int64_t>(__ldg(best_idx + row)) - ref_index_base;
+        if constexpr (kSelf) {
+            if (ri < 0) {
+                if (lane == 0) { keep[row] = 0; if (best_val != nullptr) best_val[row] = INFINITY; }
+                continue;
+            }
+        }
         const float d = k2s_euclid_dist(cand + row * dim, ref + ri * dim, dim, lane, kMode);
         if (lane == 0) {
             keep[row] = d <= thr ? 1 : 0;
@@ -354,12 +369,12 @@ int launch_vec(const float* ref, int64_t n_ref, const float* cand, int64_t n_can
     const dim3 b(kThreads);
     const int64_t ref_vecs = n_ref * NV;
     if (ref_vecs <= 8) {
-        if (n_ref == 1)      filter_fp32_kernel<NV, kCosine, 1><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band);
-        else if (n_ref == 2) filter_fp32_kernel<NV, kCosine, 2><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band);
-        else if (n_ref <= 4) filter_fp32_kernel<NV, kCosine, (NV <= 2 ? 4 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band);
-        else                 filter_fp32_kernel<NV, kCosine, (NV == 1 ? 8 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band);
+        if (n_ref == 1)      filter_fp32_kernel<NV, kCosine, 1><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
+        else if (n_ref == 2) filter_fp32_kernel<NV, kCosine, 2><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
+        else if (n_ref <= 4) filter_fp32_kernel<NV, kCosine, (NV <= 2 ? 4 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
+        else                 filter_fp32_kernel<NV, kCosine, (NV == 1 ? 8 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
     } else {
-        filter_fp32_kernel<NV, kCosine, 0><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band);
+        filter_fp32_kernel<NV, kCosine, 0><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
     }
     FFR_LAUNCH_CHECK("filter_fp32");
     return FFR_OK;
@@ -380,8 +395,8 @@ int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64
     const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
                         ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
     if (!vec_ok) {
-        if (cosine) filter_fp32_generic_kernel<true><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
-        else        filter_fp32_generic_kernel<false><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
+        if (cosine) filter_fp32_generic_kernel<true><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, kNoSelf);
+        else        filter_fp32_generic_kernel<false><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, kNoSelf);
         FFR_LAUNCH_CHECK("filter_fp32_generic");
         return FFR_OK;
     }
@@ -434,12 +449,23 @@ int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim) {
 
 int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
                          uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
-                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s) {
+                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s, bool self) {
     if (n_cand == 0) return FFR_OK;
     int64_t grid = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
     if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
     const dim3 g(static_cast<unsigned>(grid));
     const BandOut band{band_tol, band_count, band_rows, band_cap};
+    if (self) {
+        switch (mode) {
+            case 1: euclid_value_kernel<1, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+            case 2: euclid_value_kernel<2, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+            case 4: euclid_value_kernel<4, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+            case 8: euclid_value_kernel<8, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+            default: euclid_value_kernel<0, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        }
+        FFR_LAUNCH_CHECK("euclid_values");
+        return FFR_OK;
+    }
     switch (mode) {
         case 1: euclid_value_kernel<1><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
         case 2: euclid_value_kernel<2><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
@@ -448,6 +474,35 @@ int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, in
         default: euclid_value_kernel<0><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
     }
     FFR_LAUNCH_CHECK("euclid_values");
+    return FFR_OK;
+}
+
+int launch_filter_fp32_self(const float* x, int64_t n, int64_t n_cand, int32_t dim, int metric, SelfArgs self, float thr,
+                            uint8_t* keep, int32_t* idx, float* val, float band_tol, int32_t* band_count, int64_t* band_rows,
+                            int64_t band_cap, cudaStream_t s) {
+    if (n_cand == 0) return FFR_OK;
+    const float* cand = x + self.row0 * dim;
+    const int sms = num_sms();
+    const int64_t blocks_needed = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
+    const dim3 g(static_cast<unsigned>(blocks_needed < static_cast<int64_t>(sms) * 8 ? blocks_needed : static_cast<int64_t>(sms) * 8));
+    const BandOut band{band_tol, band_count, band_rows, band_cap};
+    const bool cosine = metric == FFR_METRIC_COSINE;
+    // the form K2s's gallery kernel takes for n_ref > 2 (k2s_dist_mode_gallery): what the tcgen05 Euclid value pass reproduces
+    const int mode = k2s_dist_mode_gallery(x, cand, dim);
+#define FFR_SELF_LAUNCH(NV)                                                                                                   \
+    if (cosine) filter_fp32_kernel<NV, true, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);  \
+    else        filter_fp32_kernel<NV, false, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self)
+    switch (mode) {
+        case 1: FFR_SELF_LAUNCH(1); break;
+        case 2: FFR_SELF_LAUNCH(2); break;
+        case 4: FFR_SELF_LAUNCH(4); break;
+        case 8: FFR_SELF_LAUNCH(8); break;
+        default:
+            if (cosine) filter_fp32_generic_kernel<true, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);
+            else        filter_fp32_generic_kernel<false, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);
+    }
+#undef FFR_SELF_LAUNCH
+    FFR_LAUNCH_CHECK("filter_fp32_self");
     return FFR_OK;
 }
 

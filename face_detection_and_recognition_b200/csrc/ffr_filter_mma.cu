@@ -474,6 +474,9 @@ struct KParams {
     const float* ref_bias;         // -|r|^2 * 2^-f / 2 per (compact) reference column, zero padded to a multiple of kTileN
     const float* cand_scale;       // 1 / |c| per candidate row (K1)
     const float* bias_max;         // max |ref_bias| (device scalar): sizes the per-row window
+    // kSelf: the candidates are rows [self_row0, self_row0 + n_cand) of the reference matrix (DESIGN.md section 4, "Self mode")
+    int64_t self_row0;
+    int self_mode;                 // FFR_SELF_OTHERS | FFR_SELF_EARLIER
 };
 
 // End of a candidate tile, once per row (the two column halves merged): classify_row writes keep / index / score and decides
@@ -488,11 +491,25 @@ struct RowOut {
     RecheckRec rec;
 };
 
-// kEuclid: the row's window is delta_e (not p.delta), and force_full sends the row to the full rescan whatever its scores
-template <bool kEuclid = false>
+// kEuclid: the row's window is delta_e (not p.delta), and force_full sends the row to the full rescan whatever its scores.
+// kSelf: `none` = the row has no eligible reference (row 0 in FFR_SELF_EARLIER): index -1, score -inf, no re-check, no band.
+template <bool kEuclid = false, bool kSelf = false>
 __device__ __forceinline__ RowOut classify_row(const KParams& p, const Top3& t, const HiddenM& hid, int64_t row,
-                                               float delta_e = 0.f, bool force_full = false) {
+                                               float delta_e = 0.f, bool force_full = false, bool none = false) {
     RowOut o;
+    if constexpr (kSelf) {
+        if (none) {
+            if (row < p.n_cand) {
+                p.keep[row] = 0;
+                p.best_idx[row] = -1;
+                if (p.best_val != nullptr) p.best_val[row] = -INFINITY;
+            }
+            o.cls = 0;
+            o.rec.row = static_cast<int32_t>(row);
+            o.rec.idx1 = o.rec.idx2 = o.rec.idx3 = -1;
+            return o;
+        }
+    }
     const auto delta = [&]() { return kEuclid ? delta_e : p.delta; };
     const bool valid = row < p.n_cand;
     const bool near_tie = (t.i2 >= 0) && (t.b1 - t.b2 <= delta());
@@ -586,6 +603,17 @@ __device__ __forceinline__ void append_rows(const KParams& p, const RowOut (&o)[
     }
 }
 
+// Self mode, FFR_SELF_EARLIER: candidate tile t only needs the reference tiles up to the last one with a column below its last
+// row.  The TMA producer, the MMA thread and the epilogue derive the same range from the tile index.  (Candidate tiles stay
+// dealt round-robin: with per-tile work growing linearly, a reversed order gives the busiest CTA pair the same sum -- the
+// last-wave imbalance is the wave quantisation the gallery call has too; tools/bench_self.py prints it.)
+__device__ __forceinline__ int32_t self_rt_end(const KParams& p, int64_t ct, int32_t n_rt) {
+    if (p.self_mode != FFR_SELF_EARLIER) return n_rt;
+    constexpr int64_t kPair = 2 * kTileM;                              // (self mode runs cta_group::2)
+    const int64_t last = ct * kPair + (kPair - 1) < p.n_cand ? ct * kPair + (kPair - 1) : p.n_cand - 1;
+    return static_cast<int32_t>((p.self_row0 + last + kTileN - 1) / kTileN);
+}
+
 // kCG: tcgen05 cta_group (1|2).  Eight epilogue warps = 4 TMEM lane quadrants x 2 column halves.
 // kNormMode != 0 (kNorm): K1 for the candidates runs INSIDE this kernel.  Two extra "normaliser" warps (the hardware allocates warps in
 // fours, so 10 warps cost 12 anyway) read the fp32 rows of the CTA's NEXT candidate tile, L2-normalise them exactly like K1
@@ -597,7 +625,11 @@ __device__ __forceinline__ void append_rows(const KParams& p, const RowOut (&o)[
 // hot loop's body altogether; kAlways picks the unconditional or the gated update path.
 // kEuclid: the Euclid decision rule (K1 schedule, cta_group::2, production policies only): every score gets the per-reference
 // bias scaled by the row's 1 / |c| before the max trees, and the row's window widens with that bias (DESIGN.md section 4).
-template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr, bool kEuclid = false>
+// kSelf: self mode (ffr_filter_self; K1 schedule, cta_group::2, production policies only).  A reference tile that holds a
+// column the row may not match -- its own (FFR_SELF_OTHERS) or any at or after it (FFR_SELF_EARLIER) -- runs the masked copy of
+// the epilogue body; FFR_SELF_EARLIER stops every role at the last reference tile with a column below the candidate tile's last
+// row.
+template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr, bool kEuclid = false, bool kSelf = false>
 __global__ void __launch_bounds__(64 + 32 * 8 + (kNormMode ? 64 : 0), 1)   // 10 warps are allocated as 12: <= 168 registers
 filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_constant__ CUtensorMap tmap_ref,
                   const __grid_constant__ CUtensorMap tmap_cand32, const KParams p) {
@@ -605,6 +637,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
     // (Separate instantiations: with stage32 as a run-time branch its mere presence cost the dim-512 kernel 1.5 % of wall clock.)
     // kInstr: the instrumented build (in-kernel cycle counters, score dump, epilogue diagnostics).  The production
     // instantiation contains none of it: the counters alone were half a dozen spilled 64-bit values per role.
+    static_assert(!kSelf || (kCG == 2 && kNormMode == 0 && !kInstr), "self mode runs on the K1 schedule, cta_group::2, production build");
     constexpr bool kNorm = kNormMode != 0;
     constexpr bool st32 = kNormMode >= 2;
     // stage32 comes in two forms: kNormMode 2 hands the end-of-tile work (merge of the column halves, classification, K3's
@@ -757,7 +790,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 try_issue_a();
                 if (!p.decouple_a && !st32) { while (need_a) try_issue_a(); }      // (A/B knob: the old blocking order)
                 if (!k1_done) { pdl_wait(); k1_done = true; }
-                for (int rt = 0; rt < n_rt; ++rt) {
+                for (int rt = 0; rt < (kSelf ? self_rt_end(p, tile, n_rt) : n_rt); ++rt) {
                     int32_t rrow0 = rt * kAccN + static_cast<int32_t>(cta_rank * kBRows);
                     // A box that lies ENTIRELY past the last reference (the peer CTA's half of a last tile with <= 128 live
                     // references) is not loaded as such: measured, a tile with such a box costs 4-5 x a normal one (the MMA
@@ -820,7 +853,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 }
                 tc_fence_after();
                 const uint32_t a_lo0 = ((smem_u32(smem_a + as * a_stage_bytes) & 0x3FFFFu) >> 4) | (1u << 16);
-                for (int rt = 0; rt < n_rt; ++rt) {
+                for (int rt = 0; rt < (kSelf ? self_rt_end(p, tile, n_rt) : n_rt); ++rt) {
                     mbar_wait_timed(&t_empty[acc], tph ^ 1, pr, w_tempty);
                     tc_fence_after();
                     uint32_t idesc = idesc_full;
@@ -1139,6 +1172,10 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             hid.base = 0;
             hid.mask = 0;
             const int64_t row = tile * (kTileM * kCG) + cta_rank * kTileM + r_in_tile;
+            // kSelf: this row's global index g; the masked body sets columns >= self_lim (past the last reference, or from g on
+            // in FFR_SELF_EARLIER) and column g to -inf
+            const int32_t self_g = kSelf ? static_cast<int32_t>(p.self_row0 + row) : 0;
+            const int32_t self_lim = kSelf ? (p.self_mode == FFR_SELF_EARLIER ? self_g : static_cast<int32_t>(n_ref)) : 0;
             float delta_row = 0.f, s_row = 0.f;
             if constexpr (kEuclid) {
                 static_assert(kNormMode == 0 && !kInstr, "Euclid runs on the K1 schedule, production build only");
@@ -1195,7 +1232,17 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                                 v[cc][4 * j4] = lo.x; v[cc][4 * j4 + 1] = lo.y; v[cc][4 * j4 + 2] = hi.x; v[cc][4 * j4 + 3] = hi.y;
                             }
                     }
-                    if constexpr (kPartial) {                      // partial last reference tile: columns >= n_ref -> -inf
+                    if constexpr (kSelf) {
+                        if constexpr (kPartial) {                  // masked body of self mode (after the Euclid bias)
+#pragma unroll
+                            for (int cc = 0; cc < kChunksPerPart; ++cc)
+#pragma unroll
+                                for (int j = 0; j < 32; ++j) {
+                                    const int32_t c = base0 + cc * 32 + j;
+                                    v[cc][j] = (c >= self_lim || c == self_g) ? -INFINITY : v[cc][j];
+                                }
+                        }
+                    } else if constexpr (kPartial) {               // partial last reference tile: columns >= n_ref -> -inf
                         const int n_left = static_cast<int>(ncols64) - h * (kChunksPerPart * 32);
 #pragma unroll
                         for (int cc = 0; cc < kChunksPerPart; ++cc)
@@ -1246,8 +1293,22 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 ++t_it;
             };
             const int32_t n_full = static_cast<int32_t>(n_ref / kAccN);
-            for (int rt = 0; rt < n_full; ++rt) ref_tile(rt, std::false_type{});
-            if (n_full < n_rt) ref_tile(n_full, std::true_type{});
+            if constexpr (kSelf) {
+                // the masked body runs on the partial last tile and on every tile that holds a row of this CTA pair's candidate
+                // tile (two tiles when the rows straddle a tile boundary: row_begin not a multiple of 256); once per (candidate
+                // tile, reference tile), from the indices alone
+                const int64_t g0 = p.self_row0 + tile * (kTileM * kCG);
+                const int64_t g1 = p.self_row0 + (tile * (kTileM * kCG) + (kTileM * kCG - 1) < p.n_cand
+                                                      ? tile * (kTileM * kCG) + (kTileM * kCG - 1) : p.n_cand - 1);
+                const int32_t rt_end = self_rt_end(p, tile, n_rt);
+                for (int rt = 0; rt < rt_end; ++rt) {
+                    const int64_t c0 = static_cast<int64_t>(rt) * kAccN;
+                    if (rt >= n_full || (c0 <= g1 && c0 + kAccN > g0)) ref_tile(rt, std::true_type{});
+                    else                                               ref_tile(rt, std::false_type{});
+                }
+            }
+            for (int rt = 0; rt < (kSelf ? 0 : n_full); ++rt) ref_tile(rt, std::false_type{});
+            if (!kSelf && n_full < n_rt) ref_tile(n_full, std::true_type{});
             // ---- hand the other column part(s) over, merge, emit.  The merging thread runs ~300 dependent instructions
             // alone on its scheduler (its partner is already in the next tile's loads), so with two parts the ROLE alternates
             // from candidate tile to candidate tile: each warp carries the tail every other tile, and since the reader of
@@ -1343,7 +1404,8 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 }
 
                 RowOut ro[1];
-                ro[0] = classify_row<kEuclid>(p, t, hm, row, delta_row, !(fabsf(s_row) <= 3.4e38f));
+                ro[0] = classify_row<kEuclid, kSelf>(p, t, hm, row, delta_row, !(fabsf(s_row) <= 3.4e38f),
+                                                     kSelf && p.self_mode == FFR_SELF_EARLIER && self_g == 0);
                 append_rows<1>(p, ro, lane);
             }
             }   // !st32
@@ -1474,7 +1536,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                            float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                            RecheckLists lists, int no_recheck, BandArgs band, float* dbg_scores, bool after_k1,
                            const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
-                           const float* euclid_bias, const float* cand_scale, const float* bias_max) {
+                           const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
     if (dim_pad % kBlockK != 0 || dim_pad < kBlockK || dim_pad > 512) {
         set_error("filter_mma: padded dim %d not in {64..512 step 64}", dim_pad);
         return FFR_ERR_UNSUPPORTED;
@@ -1493,6 +1555,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     const bool euclid = euclid_bias != nullptr;
     if (euclid && (cg != 2 || fuse || no_recheck || dbg_scores != nullptr)) {
         set_error("filter_mma: the Euclid kernel exists for cta_group::2, the K1 schedule and the re-checked build only");
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const bool self_mode = self.mode >= 0;
+    if (self_mode && (cg != 2 || fuse || no_recheck || dbg_scores != nullptr || n_ref_dev != nullptr)) {
+        set_error("filter_mma: the self-mode kernel exists for cta_group::2, the K1 schedule and the re-checked build only");
         return FFR_ERR_UNSUPPORTED;
     }
     const int kb = dim_pad / kBlockK;
@@ -1547,6 +1614,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     p.keep = keep; p.best_idx = idx; p.best_val = val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof; p.epi_mode = kn.epi_mode;
     p.band_tol = band.tol; p.band_count = no_recheck ? band.count : nullptr; p.band_rows = band.rows; p.band_cap = band.cap;
     p.ref_bias = euclid_bias; p.cand_scale = cand_scale; p.bias_max = bias_max;
+    p.self_row0 = self.row0; p.self_mode = self.mode;
     p.acc_stages = kn.acc_stages == 1 ? 1 : 2;
     p.cand32 = cand32; p.cand16 = cand16; p.dim = dim;
     p.b_tx_bytes = b_stage / half_b;
@@ -1565,7 +1633,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     // callers always get the exact per-column masks (FFR_GRID_EXACT=1 forces them everywhere).
     p.grid_exact = kn.grid_exact >= 0 ? kn.grid_exact : 0;
     if (no_recheck || dbg_scores != nullptr) p.grid_exact = 1;
-    if (euclid) p.grid_exact = 0;                          // (K3 always runs behind the Euclid kernel)
+    if (euclid || self_mode) p.grid_exact = 0;             // (K3 always runs behind the Euclid and the self-mode kernels)
     p.norm_ahead = kn.norm_ahead < 1 ? 1 : kn.norm_ahead;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const KParams);
@@ -1583,8 +1651,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
 #undef FFR_K_POLICY
 #undef FFR_K
     static const KernelFn euclid2[2] = {filter_mma_kernel<2, 0, 0, 0, false, true>, filter_mma_kernel<2, 0, 0, 1, false, true>};
+    static const KernelFn self2[2][2] = {{filter_mma_kernel<2, 0, 0, 0, false, false, true>, filter_mma_kernel<2, 0, 0, 1, false, false, true>},
+                                         {filter_mma_kernel<2, 0, 0, 0, false, true, true>, filter_mma_kernel<2, 0, 0, 1, false, true, true>}};
     KernelFn fn;
-    if (euclid)       fn = euclid2[p.grid_updates ? 1 : 0];
+    if (self_mode)    fn = self2[euclid ? 1 : 0][p.grid_updates ? 1 : 0];
+    else if (euclid)  fn = euclid2[p.grid_updates ? 1 : 0];
     else if (cg == 2) fn = instr ? instr2[nm] : prod2[nm][(p.grid_exact ? 2 : 0) + (p.grid_updates ? 1 : 0)];
     else              fn = instr ? instr1[nm] : prod1[nm];
     // the opt-in to > 48 KB of dynamic shared memory is a per-DEVICE function attribute: set once per device this process uses
@@ -1601,8 +1672,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                 FFR_CUDA_TRY(cudaFuncSetAttribute(prod1[m], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
                 FFR_CUDA_TRY(cudaFuncSetAttribute(instr1[m], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
             }
-            for (int v = 0; v < 2; ++v)
+            for (int v = 0; v < 2; ++v) {
                 FFR_CUDA_TRY(cudaFuncSetAttribute(euclid2[v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+                FFR_CUDA_TRY(cudaFuncSetAttribute(self2[0][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+                FFR_CUDA_TRY(cudaFuncSetAttribute(self2[1][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+            }
             attr_set[slot] = true;
         }
     }
@@ -1657,10 +1731,10 @@ int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const 
                       float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
                       RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
                       int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
-                      const float* euclid_bias, const float* cand_scale, const float* bias_max) {
+                      const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
     return launch_filter_mma_impl(ref16, n_ref, cand16, cand32, dim, n_cand, dim_pad, thr, delta, thr_band, ref_index_base,
                                   keep, idx, val, lists, no_recheck, BandArgs{band_tol, band_count, band_rows, band_cap}, nullptr,
-                                  after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale, bias_max);
+                                  after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale, bias_max, self);
 }
 
 // true when the fused schedule needs NO fp16 copy of the candidates in the workspace (stage32: the fp16 A tiles only ever
@@ -1683,7 +1757,7 @@ int launch_filter_mma_debug(const __half* ref16, int64_t n_ref, const __half* ca
                             float* scores, cudaStream_t s) {
     return launch_filter_mma_impl(ref16, n_ref, const_cast<__half*>(cand16), nullptr, dim_pad, n_cand, dim_pad, thr, delta, delta, 0, keep, idx,
                                   val, lists, 0, BandArgs{0.f, nullptr, nullptr, 0}, scores, false, nullptr, nullptr, s,
-                                  nullptr, nullptr, nullptr);
+                                  nullptr, nullptr, nullptr, kNoSelf);
 }
 
 }  // namespace ffr

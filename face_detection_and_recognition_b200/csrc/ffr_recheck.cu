@@ -283,12 +283,15 @@ __device__ __forceinline__ void unpack_key(unsigned long long k, float& v, int32
 // warp per record, L LANES PER REFERENCE (the candidate row broadcast from shared memory).  Typically 2-8 references.
 __device__ __forceinline__ int64_t parts_first_item(int64_t warp, int64_t nwarps) { return nwarps - 1 - warp; }
 
+// kSelf: the X / Y masks name a superset of the in-window columns, which can include the row's own column (and, in
+// FFR_SELF_EARLIER, later ones): excluded references are skipped.
+template <bool kSelf>
 __device__ __forceinline__ void
 recheck_parts_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim,
                     float thr, int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                     float* __restrict__ best_val, const RecheckLists& lists, float band_tol, int32_t* band_count,
                     int64_t* band_rows, int64_t band_cap, bool vec, const int32_t* __restrict__ ref_map,
-                    const int32_t* __restrict__ n_unique_dev, int emode) {
+                    const int32_t* __restrict__ n_unique_dev, int emode, SelfArgs self) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     float* c_smem = s_rows + static_cast<size_t>(w) * dim;
     // records are dealt from the LAST warp of the grid downwards: with a short pairs list (dealt from warp 0 upwards) the two
@@ -321,6 +324,7 @@ recheck_parts_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref,
                 } else {
                     ri = rec.idx2;
                 }
+                if constexpr (kSelf) ri = self_eligible(ri, self.row0 + rec.row, self.mode) ? ri : -1;
                 if (ri < 0) continue;
                 const float d = k2s_euclid_dist(c, ref + ri * dim, dim, lane, emode);
                 if (d < best || (d == best && ri < bi)) { best = d; bi = static_cast<int32_t>(ri); }
@@ -351,7 +355,8 @@ recheck_parts_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref,
         __syncwarp();
         const float cc_sqrt = __fsqrt_rn(warp_sum(cc));
         for (int e0 = 0, eb = 0; e0 < n_all; e0 += per, ++eb) {   // `per` references at a time
-            const int64_t ri = ref_of(eb);
+            int64_t ri = ref_of(eb);
+            if constexpr (kSelf) ri = self_eligible(ri, self.row0 + rec.row, self.mode) ? ri : -1;
             float a_acc = 0.f, b_acc = 0.f;
             if (vec) {
                 // eight float4 steps at a time, every load issued before the first FMA: the rows come out of L2 (~600 cycles).
@@ -431,11 +436,13 @@ __device__ __forceinline__ int64_t small_first_item(int64_t warp, int64_t nwarps
     return (warp >= half ? warp - half : warp + (nwarps - half)) * ipw;
 }
 
+// kSelf: the per-candidate bound (!= g, or < g) is applied before the comparison
+template <bool kSelf>
 __device__ __forceinline__ void
 rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim,
                    float thr, int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                    float* __restrict__ best_val, const RecheckLists& lists, int64_t count, float band_tol,
-                   int32_t* band_count, int64_t* band_rows, int64_t band_cap, bool vec, int emode) {
+                   int32_t* band_count, int64_t* band_rows, int64_t band_cap, bool vec, int emode, SelfArgs self) {
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     float* c_smem = s_rows + static_cast<size_t>(w) * dim;
     const int64_t nb = (n_ref + kSmallRefs - 1) / kSmallRefs;
@@ -477,9 +484,11 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
         for (int64_t item = i0; item < i1; ++item) {
             const int64_t slot = item / nb, blk = item - slot * nb;
             if (slot != cur) { flush(); cur = slot; pending = 0; best = -INFINITY; bi = 0x7FFFFFFF; }
-            const float* c = cand + static_cast<int64_t>(lists.full_rows[slot]) * dim;
+            const int32_t crow = lists.full_rows[slot];
+            const float* c = cand + static_cast<int64_t>(crow) * dim;
             const int64_t lo = blk * kSmallRefs, hi = (lo + kSmallRefs < n_ref) ? lo + kSmallRefs : n_ref;
             for (int64_t i = lo; i < hi; ++i) {
+                if constexpr (kSelf) { if (!self_eligible(i, self.row0 + crow, self.mode)) continue; }
                 const float sc = -k2s_euclid_dist(c, ref + i * dim, dim, lane, emode);
                 if (sc > best) { best = sc; bi = static_cast<int32_t>(i); }
             }
@@ -498,6 +507,7 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
         const float4* ref4 = reinterpret_cast<const float4*>(ref);
         const bool live = lane < nvec;
         float4 cv = z4;
+        int64_t g_self = 0;                                        // kSelf: global index of the parked row
         for (int64_t item = i0; item < i1; ++item) {
             const int64_t slot = item / nb, blk = item - slot * nb;
             const int64_t lo = blk * kSmallRefs;
@@ -509,6 +519,7 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
             if (slot != cur) {
                 flush();
                 cv = live ? __ldg(reinterpret_cast<const float4*>(cand) + static_cast<int64_t>(lists.full_rows[slot]) * nvec + lane) : z4;
+                if constexpr (kSelf) g_self = self.row0 + lists.full_rows[slot];
                 float cc = 0.f;
                 cc = fmaf(cv.x, cv.x, cc); cc = fmaf(cv.y, cv.y, cc); cc = fmaf(cv.z, cv.z, cc); cc = fmaf(cv.w, cv.w, cc);
                 cc_sqrt = __fsqrt_rn(warp_sum(cc));
@@ -531,17 +542,19 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
 #pragma unroll
             for (int r = 0; r < kSmallBatch; ++r) {              // ascending + strict '>' = first occurrence
                 const float sc = __fdiv_rn(a[r], __fmul_rn(__fsqrt_rn(b[r]), cc_sqrt));
-                if (r < n_rows && sc > best) { best = sc; bi = static_cast<int32_t>(lo + r); }
+                if (r < n_rows && sc > best && (!kSelf || self_eligible(lo + r, g_self, self.mode))) { best = sc; bi = static_cast<int32_t>(lo + r); }
             }
             ++pending;
         }
         flush();
         return;
     }
+    int64_t g_self = 0;
     for (int64_t item = i0; item < i1; ++item) {
         const int64_t slot = item / nb, blk = item - slot * nb;
         if (slot != cur) {
             flush();
+            if constexpr (kSelf) g_self = self.row0 + lists.full_rows[slot];
             const float* c = cand + static_cast<int64_t>(lists.full_rows[slot]) * dim;
             float cc = 0.f;
             __syncwarp();
@@ -561,7 +574,7 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
             cos_fp32_multi<kSmallBatch>(c_smem, ref + i * dim, n_rows, dim, cc_sqrt, lane, vec, sc);
 #pragma unroll
             for (int r = 0; r < kSmallBatch; ++r)
-                if (r < n_rows && sc[r] > best) { best = sc[r]; bi = static_cast<int32_t>(i + r); }
+                if (r < n_rows && sc[r] > best && (!kSelf || self_eligible(i + r, g_self, self.mode))) { best = sc[r]; bi = static_cast<int32_t>(i + r); }
         }
         ++pending;
     }
@@ -570,33 +583,36 @@ rescan_small_phase(float* s_rows, const float* __restrict__ ref, int64_t n_ref, 
 
 // One launch re-checks everything K2 flagged: phase A = K3a (pairs list), phase B = K3b (full-rescan list; small or
 // tiled walk, chosen from the device-side count, uniform over the grid).  The phases touch disjoint rows.
-template <bool kVec, bool kEuclid>
+// kSelf (ffr_filter_self): cand = rows [self.row0, ...) of ref; the pairs phase needs nothing (its leading references come from
+// K2's masked scores), the parts phase and both full-rescan walks skip the references the row may not match.
+template <bool kVec, bool kEuclid, bool kSelf = false>
 __global__ void __launch_bounds__(kThreads, 2)      // two CTAs per SM (<= 128 registers): the fixed grid of 2 x SMs is ONE wave
 recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim, float thr,
                int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                float* __restrict__ best_val, RecheckLists lists, float band_tol, int32_t* band_count,
                int64_t* band_rows, int64_t band_cap, const int32_t* __restrict__ ref_map,
-               const int32_t* __restrict__ n_unique_dev, int skip, int emode_arg) {
+               const int32_t* __restrict__ n_unique_dev, int skip, int emode_arg, SelfArgs self) {
     const int emode = kEuclid ? emode_arg : -1;           // K2s distance mode (Euclid), -1 = cosine
     extern __shared__ __align__(16) float s_c[];               // kFullGroup x dim candidate rows | staged reference tile
     __shared__ float s_ccs[kFullGroup];
     __shared__ unsigned long long s_key[kWarps][kFullGroup];
     __shared__ int s_last;
+    __shared__ int64_t s_g[kSelf ? kFullGroup : 1];           // kSelf: global indices of the parked full-rescan rows
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     pdl_wait();                 // launched as K2's programmatic dependent: everything below reads K2's lists and outputs
     if (!(skip & 1))
         recheck_pairs_phase(s_c, ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
                             band_rows, band_cap, kVec, emode);
     if (!(skip & 2))
-        recheck_parts_phase(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
-                            band_rows, band_cap, kVec, ref_map, n_unique_dev, emode);
+        recheck_parts_phase<kSelf>(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol,
+                                   band_count, band_rows, band_cap, kVec, ref_map, n_unique_dev, emode, self);
     if (skip & 4) return;
     int64_t count = lists.hdr->full_count;
     if (count > lists.full_cap) count = lists.full_cap;
     if (count == 0) return;
     if (static_cast<long long>(count) * n_ref * dim <= kSmallElems) {
-        rescan_small_phase(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, count, band_tol,
-                           band_count, band_rows, band_cap, kVec, emode);
+        rescan_small_phase<kSelf>(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, count,
+                                  band_tol, band_count, band_rows, band_cap, kVec, emode, self);
         return;
     }
     __syncthreads();                                            // phase A's per-warp rows are dead: the tiled walk reuses s_c
@@ -631,6 +647,7 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                 }
                 cc = warp_sum(cc);
                 if (lane == 0) s_ccs[jw] = __fsqrt_rn(cc);
+                if constexpr (kSelf) { if (lane == 0) s_g[jw] = slot < count ? self.row0 + lists.full_rows[slot] : 0; }
             }
             parked = g;
         }
@@ -751,7 +768,7 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                             for (int j = 0; j < kFullGroup; ++j) {
                                 const float dot = (j & 1) ? acc[r][j >> 1].y : acc[r][j >> 1].x;
                                 const float sc = kEuclid ? -__fsqrt_rn(dot) : __fdiv_rn(dot, __fmul_rn(rs, s_ccs[j]));
-                                if (sc > best[j]) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
+                                if (sc > best[j] && (!kSelf || self_eligible(i, s_g[j], self.mode))) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
                             }
                         }
                     }
@@ -779,7 +796,7 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
 #pragma unroll
                 for (int j = 0; j < kFullGroup; ++j) {
                     const float sc = kEuclid ? -__fsqrt_rn(acc[j]) : __fdiv_rn(acc[j], __fmul_rn(rs, s_ccs[j]));
-                    if (sc > best[j]) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
+                    if (sc > best[j] && (!kSelf || self_eligible(i, s_g[j], self.mode))) { best[j] = sc; bidx[j] = static_cast<int32_t>(i); }
                 }
             }
         }
@@ -854,7 +871,7 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
                    const float* /*ref_norm*/, const float* /*cand_norm*/, float thr, int64_t ref_index_base,
                    uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode) {
+                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode, SelfArgs self) {
     if (n_cand == 0) return FFR_OK;
     const bool euclid = euclid_mode >= 0;
     static_assert(kFullGroup % kWarps == 0, "every warp parks kFullGroup / kWarps candidate rows of a full-rescan group");
@@ -877,6 +894,10 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
             FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
             FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
             FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
+            FFR_CUDA_TRY(cudaFuncSetAttribute(recheck_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 148 * 1024));
             attr_set[slot] = true;
         }
     }
@@ -891,10 +912,13 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
     cfg.attrs = attr;
     cfg.numAttrs = (knobs().pdl & 2) != 0 ? 1 : 0;        // FFR_PDL bit 1 (bit 0: K1 -> K2)
     const int skip = knobs().k3_skip;                     // timing experiments only (FFR_K3_SKIP: phases left out, WRONG results)
-    auto* fn = euclid ? (vec ? recheck_kernel<true, true> : recheck_kernel<false, true>)
-                      : (vec ? recheck_kernel<true, false> : recheck_kernel<false, false>);
+    auto* fn = self.mode >= 0
+                   ? (euclid ? (vec ? recheck_kernel<true, true, true> : recheck_kernel<false, true, true>)
+                             : (vec ? recheck_kernel<true, false, true> : recheck_kernel<false, false, true>))
+                   : (euclid ? (vec ? recheck_kernel<true, true> : recheck_kernel<false, true>)
+                             : (vec ? recheck_kernel<true, false> : recheck_kernel<false, false>));
     FFR_CUDA_TRY(cudaLaunchKernelEx(&cfg, fn, ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val, lists, band_tol,
-                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, skip, euclid_mode));
+                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, skip, euclid_mode, self));
     FFR_LAUNCH_CHECK("recheck");
     return FFR_OK;
 }

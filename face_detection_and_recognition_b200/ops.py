@@ -18,15 +18,16 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import (DTYPE_F16, DTYPE_F32, FLAG_FORCE_FP32, FLAG_FORCE_MMA, FLAG_NO_RECHECK, METRIC_COSINE,
-                   METRIC_EUCLID, check)
+from ._lib import (DTYPE_F16, DTYPE_F32, ERR_UNSUPPORTED, FLAG_FORCE_FP32, FLAG_FORCE_MMA, FLAG_NO_RECHECK, METRIC_COSINE,
+                   METRIC_EUCLID, SELF_EARLIER, SELF_OTHERS, FfrError, check)
 
-__all__ = ["l2norm_rows", "face_filter", "cosine_filter", "ref_mean_and_thres", "FilterResult", "HostFilter", "GraphedFilter",
+__all__ = ["l2norm_rows", "face_filter", "self_filter", "cosine_filter", "ref_mean_and_thres", "FilterResult", "HostFilter", "GraphedFilter",
            "ResultGather", "launch_count", "METRIC_COSINE", "METRIC_EUCLID", "FLAG_FORCE_FP32", "FLAG_FORCE_MMA",
-           "FLAG_NO_RECHECK"]
+           "FLAG_NO_RECHECK", "SELF_OTHERS", "SELF_EARLIER"]
 
 _METRICS = {"cosine": METRIC_COSINE, "euclid": METRIC_EUCLID, "euclidean": METRIC_EUCLID,
             METRIC_COSINE: METRIC_COSINE, METRIC_EUCLID: METRIC_EUCLID}
+_SELF_MODES = {"others": SELF_OTHERS, "earlier": SELF_EARLIER, SELF_OTHERS: SELF_OTHERS, SELF_EARLIER: SELF_EARLIER}
 
 
 def _stream_ptr(dev: torch.device) -> int:
@@ -154,16 +155,71 @@ def face_filter(ref: torch.Tensor, cand: torch.Tensor, thr: float, metric="cosin
             n = int(band_count.item())
             res.band_rows = torch.sort(band_rows[:min(n, n_cand)]).values
         if want_stats:
-            arr = (C.c_int64 * 8)()
-            check(lib.ffr_filter_stats(ws.data_ptr(), arr, _stream_ptr(dev)))
-            res.stats = {"rechecked": arr[0], "part_rescans": arr[4], "full_rescans": arr[1],
-                         "path": "tcgen05" if arr[2] == 1 else "fp32", "launches": arr[3], "refs_scanned": arr[5]}
-            if arr[2] == 1:
-                cfg = (C.c_int32 * 8)()
-                lib.ffr_debug_last_k2_config(cfg)
-                res.stats["k2"] = {"cta_group": cfg[0], "grid_exact": cfg[1], "grid_updates": cfg[2],
-                                   "normalise": ("k1", "fused_scratch", "stage32+tail_offload", "stage32")[cfg[3]], "a_stages": cfg[4],
-                                   "b_stages": cfg[5], "grid": cfg[6]}
+            res.stats = _stats(lib, ws, dev)
+    return res
+
+
+def _stats(lib, ws, dev) -> dict:
+    arr = (C.c_int64 * 8)()
+    check(lib.ffr_filter_stats(ws.data_ptr(), arr, _stream_ptr(dev)))
+    stats = {"rechecked": arr[0], "part_rescans": arr[4], "full_rescans": arr[1],
+             "path": "tcgen05" if arr[2] == 1 else "fp32", "launches": arr[3], "refs_scanned": arr[5]}
+    if arr[2] == 1:
+        cfg = (C.c_int32 * 8)()
+        lib.ffr_debug_last_k2_config(cfg)
+        stats["k2"] = {"cta_group": cfg[0], "grid_exact": cfg[1], "grid_updates": cfg[2],
+                       "normalise": ("k1", "fused_scratch", "stage32+tail_offload", "stage32")[cfg[3]], "a_stages": cfg[4],
+                       "b_stages": cfg[5], "grid": cfg[6]}
+    return stats
+
+
+def self_filter(x: torch.Tensor, thr: float, metric="cosine", mode="others", rows: Optional[Tuple[int, int]] = None,
+                band_tol: Optional[float] = None, flags: int = 0, want_stats: bool = False,
+                out: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> FilterResult:
+    """Each row's best match among the OTHER rows of the same set ``x`` [N, D] (float32 CUDA): near-duplicates, repeated
+    enrolments, a face that matches none of its classmates.
+
+    ``mode="others"``: best over every row i != j.  ``mode="earlier"``: best over i < j -- with keep = 1 row j is a near-duplicate
+    of an earlier row, so dropping exactly the kept rows leaves the first occurrence of every group.  ``rows=(begin, end)``
+    filters only those candidate rows against all N (candidate-axis sharding); results are local to the range, ``best_idx`` is a
+    global row of ``x``.  A row with no eligible reference (row 0 in "earlier", or N = 1) gets keep 0, index -1 and -inf (cosine)
+    / +inf (Euclid).  Metric, threshold, band and precision contract are ``face_filter``'s on the masked problem; bit-identical
+    rows are not folded.  fp16 rows and ``FLAG_NO_RECHECK`` are refused."""
+    lib = _lib.load()
+    m = _METRICS[metric]
+    md = _SELF_MODES[mode]
+    if isinstance(x, torch.Tensor) and x.dtype == torch.float16:
+        raise FfrError(ERR_UNSUPPORTED, "self_filter takes float32 embeddings (fp16 rows are not supported)")
+    x = _require_cuda(x, "x")
+    if x.dim() != 2:
+        raise ValueError(f"x {tuple(x.shape)} must be [N, D]")
+    n, dim = x.shape
+    begin, end = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
+    n_rows = max(end - begin, 0)
+    dev = x.device
+    if out is None:
+        keep = torch.empty((n_rows,), dtype=torch.uint8, device=dev)
+        idx = torch.empty((n_rows,), dtype=torch.int32, device=dev)
+        val = torch.empty((n_rows,), dtype=torch.float32, device=dev)
+    else:
+        keep, idx, val = out
+    ws = _workspace(dev, int(lib.ffr_filter_self_workspace_bytes(n, n_rows, dim, m)))
+    band_count = band_rows = None
+    if band_tol is not None:
+        band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
+        band_rows = torch.empty((max(n_rows, 1),), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib.ffr_filter_self(x.data_ptr(), n, begin, end - begin, dim, m, md, float(thr),
+                                  keep.data_ptr() if n_rows else None, idx.data_ptr() if n_rows else None,
+                                  val.data_ptr() if n_rows else None,
+                                  float(band_tol or 0.0), band_count.data_ptr() if band_count is not None else None,
+                                  band_rows.data_ptr() if band_rows is not None else None, n_rows, int(flags),
+                                  ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
+        res = FilterResult(keep, idx, val)
+        if band_tol is not None:
+            res.band_rows = torch.sort(band_rows[:min(int(band_count.item()), n_rows)]).values
+        if want_stats:
+            res.stats = _stats(lib, ws, dev)
     return res
 
 

@@ -86,7 +86,19 @@ class CandidateSharder:
         start, stop, m_local = self.local_range(n_cand_total)
         if cand_local.shape[0] != stop - start:
             raise ValueError(f"rank {self.rank} expects {stop - start} local candidates, got {cand_local.shape[0]}")
-        res = self.filter_fn(ref, cand_local, thr, metric=metric)
+        return self._gather(self.filter_fn(ref, cand_local, thr, metric=metric), m_local, n_cand_total)
+
+    def self_filter(self, x: torch.Tensor, thr: float, metric="cosine", mode="others"):
+        """Self mode (``ops.self_filter``) sharded over the candidate axis: every rank passes the FULL ``x`` and filters its
+        ``shard_range`` of the rows against all of them.  Returns (keep, best_idx) for all rows on every rank, plus this rank's
+        local result object."""
+        from . import ops
+        start, stop, m_local = self.local_range(x.shape[0])
+        res = ops.self_filter(x, thr, metric=metric, mode=mode, rows=(start, stop))
+        return self._gather(res, m_local, x.shape[0])
+
+    def _gather(self, res, m_local: int, n_cand_total: int):
+        """Every rank's (keep, best_idx) for all ``n_cand_total`` candidates, from this rank's local result ``res``."""
         if self.world == 1:
             return res.keep, res.best_idx, res
         if self.gather == "nccl":

@@ -112,6 +112,29 @@ int ffr_filter_ex(const void* ref, int64_t n_ref, const void* cand, int64_t n_ca
                   float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
                   int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
 
+/* ---- self mode: each row's best match among the OTHER rows of the same set ------------------------------------
+ * Near-duplicate search inside one embedding set (the IMDB-WIKI cleaner's question; the tracker's check_if_face_exists asked
+ * one query at a time).  x[n, dim] fp32 (device) is both the candidate and the reference matrix: the candidates are rows
+ * [row_begin, row_begin + n_rows) (so candidate-axis sharding works unchanged), the references all n rows, and best_idx is a
+ * global row index of x.  keep / best_idx / best_val / the band hold n_rows entries, local to the row range.
+ *   FFR_SELF_OTHERS   best over every reference i != j (leave-one-out)
+ *   FFR_SELF_EARLIER  best over i < j: with keep = 1 row j is a near-duplicate of an EARLIER row, so dropping exactly the kept
+ *                     rows leaves the first occurrence of every group
+ * A row with no eligible reference (row 0 in EARLIER, or n = 1): keep = 0, best_idx = -1, best_val = -inf (cosine) / +inf
+ * (Euclid), never in the band.  Bit-identical rows are NOT folded: they are what the caller is looking for.
+ * Metric, threshold, first-occurrence ties, band and precision contract are ffr_filter_ex's applied to the masked problem
+ * (the Euclid rule included: best_idx equals the FFR_FLAG_FORCE_FP32 result except on fp32 ties, keep / best_val bit-identical
+ * to it wherever best_idx agrees).  Tensor cores when n > 8, dim <= 512, the re-check is on and the GPU runs cta_group::2;
+ * otherwise (and with FFR_FLAG_FORCE_FP32) the exact fp32 kernel K2s in its self form.  FFR_FLAG_NO_RECHECK is refused
+ * (FFR_ERR_UNSUPPORTED), a row range outside [0, n) too (FFR_ERR_INVALID).  ffr_filter_stats works on this workspace. */
+#define FFR_SELF_OTHERS  0
+#define FFR_SELF_EARLIER 1
+size_t ffr_filter_self_workspace_bytes(int64_t n, int64_t n_rows, int32_t dim, int metric);
+int ffr_filter_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, int mode,
+                    float thr, uint8_t* keep, int32_t* best_idx, float* best_val,
+                    float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
+                    int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
+
 /* statistics of the last ffr_filter* call that used this workspace (device->host copy, synchronises
  * the stream): out[0] = rows re-checked in fp32 against their two or three leading references (near-tie or
  * near-threshold), out[1] = rows that needed the full fp32 rescan, out[2] = path taken (0 fp32 CUDA-core,
