@@ -60,6 +60,9 @@ SIGNATURES = {
     "ffr_allgather_workspace_bytes": (_sz, [C.c_int, _i64]),
     "ffr_allgather_results": (C.c_int, [_vp, _vp, _vp, _i64, _vp, _vp, _vp, _sz, _vp]),
     "ffr_allgather_results_inplace": (C.c_int, [_vp, _vp, _vp, _i64, _vp]),
+    "ffr_allreduce_best_workspace_bytes": (_sz, [_i64]),
+    "ffr_allreduce_best": (C.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i32, C.c_int, _f32, _vp, _vp, _vp,
+                                     _f32, _vp, _vp, _i64, _vp, _sz, _vp]),
 }
 # test / tuning hooks that are not part of the public header
 HOOKS = {

@@ -1,6 +1,7 @@
 // C-ABI entry points of libffr_b200.so (declared in include/ffr.h): argument checking, dispatch between
 // the exact fp32 CUDA-core kernel and the tcgen05 kernel, workspace carving, the host-buffer pipeline
-// (ffr_ctx_*) and the NCCL gather (ffr_comm_*, NCCL dlopen'ed so the library loads without it).
+// (ffr_ctx_*), the NCCL gather (ffr_comm_*, NCCL dlopen'ed so the library loads without it) and the merge of a gallery
+// sharded over ranks (ffr_allreduce_best).
 #include <dlfcn.h>
 #include <stdlib.h>
 #include <string.h>
@@ -749,6 +750,7 @@ typedef void* nccl_comm_t;
 typedef int (*pfn_get_uid)(nccl_uid*);
 typedef int (*pfn_init_rank)(nccl_comm_t*, int, nccl_uid, int);
 typedef int (*pfn_allgather)(const void*, void*, size_t, int, nccl_comm_t, cudaStream_t);
+typedef int (*pfn_allreduce)(const void*, void*, size_t, int, int, nccl_comm_t, cudaStream_t);
 typedef int (*pfn_destroy)(nccl_comm_t);
 typedef const char* (*pfn_errstr)(int);
 typedef int (*pfn_group)(void);
@@ -757,6 +759,7 @@ struct NcclApi {
     pfn_get_uid get_uid = nullptr;
     pfn_init_rank init_rank = nullptr;
     pfn_allgather allgather = nullptr;
+    pfn_allreduce allreduce = nullptr;
     pfn_destroy destroy = nullptr;
     pfn_errstr errstr = nullptr;
     pfn_group group_start = nullptr, group_end = nullptr;
@@ -776,11 +779,12 @@ int nccl_load() {
     g_nccl.get_uid = reinterpret_cast<pfn_get_uid>(dlsym(g_nccl.h, "ncclGetUniqueId"));
     g_nccl.init_rank = reinterpret_cast<pfn_init_rank>(dlsym(g_nccl.h, "ncclCommInitRank"));
     g_nccl.allgather = reinterpret_cast<pfn_allgather>(dlsym(g_nccl.h, "ncclAllGather"));
+    g_nccl.allreduce = reinterpret_cast<pfn_allreduce>(dlsym(g_nccl.h, "ncclAllReduce"));
     g_nccl.destroy = reinterpret_cast<pfn_destroy>(dlsym(g_nccl.h, "ncclCommDestroy"));
     g_nccl.errstr = reinterpret_cast<pfn_errstr>(dlsym(g_nccl.h, "ncclGetErrorString"));
     g_nccl.group_start = reinterpret_cast<pfn_group>(dlsym(g_nccl.h, "ncclGroupStart"));
     g_nccl.group_end = reinterpret_cast<pfn_group>(dlsym(g_nccl.h, "ncclGroupEnd"));
-    if (!g_nccl.get_uid || !g_nccl.init_rank || !g_nccl.allgather || !g_nccl.destroy || !g_nccl.group_start || !g_nccl.group_end) {
+    if (!g_nccl.get_uid || !g_nccl.init_rank || !g_nccl.allgather || !g_nccl.allreduce || !g_nccl.destroy || !g_nccl.group_start || !g_nccl.group_end) {
         set_error("libnccl is missing expected symbols");
         return FFR_ERR_NCCL;
     }
@@ -872,6 +876,50 @@ int ffr_allgather_results_inplace(ffr_comm* c, uint8_t* keep_all, int32_t* idx_a
     if (e != 0) return nccl_fail(e, "ncclAllGather (in place)");
     if (e2 != 0) return nccl_fail(e2, "ncclGroupEnd");
     return FFR_OK;
+}
+
+size_t ffr_allreduce_best_workspace_bytes(int64_t n_cand) {
+    if (n_cand < 0) return 0;
+    const size_t b = align_up(static_cast<size_t>(n_cand) * sizeof(unsigned long long), 256);
+    return b > 0 ? b : 256;
+}
+
+int ffr_allreduce_best(ffr_comm* c, const float* ref_local, int64_t n_ref_local, int64_t ref_index_base, const float* cand,
+                       int64_t n_cand, int32_t dim, int metric, float thr, uint8_t* keep, int32_t* best_idx, float* best_val,
+                       float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, void* workspace,
+                       size_t ws_bytes, ffr_stream_t stream) {
+    if (c == nullptr) { set_error("allreduce_best: comm is null"); return FFR_ERR_INVALID; }
+    if (n_ref_local < 0 || n_cand < 0 || dim <= 0) {
+        set_error("allreduce_best: need n_ref_local >= 0, n_cand >= 0, dim > 0 (got %lld, %lld, %d)", (long long)n_ref_local,
+                  (long long)n_cand, dim);
+        return FFR_ERR_INVALID;
+    }
+    if (ref_index_base < 0 || ref_index_base + n_ref_local > static_cast<int64_t>(INT32_MAX)) {
+        set_error("allreduce_best: global reference indices [%lld, %lld) do not fit int32", (long long)ref_index_base,
+                  (long long)(ref_index_base + n_ref_local));
+        return FFR_ERR_INVALID;
+    }
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) { set_error("unknown metric %d", metric); return FFR_ERR_INVALID; }
+    if ((n_ref_local > 0 && ref_local == nullptr) ||
+        (n_cand > 0 && (cand == nullptr || keep == nullptr || best_idx == nullptr))) {
+        set_error("allreduce_best: null pointer argument");
+        return FFR_ERR_INVALID;
+    }
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    if (band_count != nullptr) FFR_CUDA_TRY(cudaMemsetAsync(band_count, 0, sizeof(int32_t), s));
+    if (n_cand == 0) return FFR_OK;
+    const size_t need = ffr_allreduce_best_workspace_bytes(n_cand);
+    if (workspace == nullptr || ws_bytes < need) {
+        set_error("allreduce_best: workspace needs %zu bytes, got %zu", need, workspace ? ws_bytes : (size_t)0);
+        return FFR_ERR_WORKSPACE;
+    }
+    if (reinterpret_cast<uintptr_t>(workspace) & 7) { set_error("allreduce_best: workspace must be 8-byte aligned"); return FFR_ERR_INVALID; }
+    unsigned long long* keys = static_cast<unsigned long long*>(workspace);
+    int rc = launch_best_keys(ref_local, n_ref_local, ref_index_base, cand, n_cand, dim, metric, best_idx, keys, s);
+    if (rc != FFR_OK) return rc;
+    const int e = g_nccl.allreduce(keys, keys, static_cast<size_t>(n_cand), /*ncclUint64*/ 5, /*ncclMax*/ 2, c->comm, s);
+    if (e != 0) return nccl_fail(e, "ncclAllReduce");
+    return launch_emit_keys(keys, n_cand, metric, thr, keep, best_idx, best_val, band_tol, band_count, band_rows, band_cap, s);
 }
 
 }  // extern "C"

@@ -381,6 +381,11 @@ void set_mma_prof_buffer(unsigned long long* dev_ptr);   // diagnostics: [grid][
 int launch_ref_stats(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres, cudaStream_t s);
 int k2s_dist_mode(const float* rows, int32_t dim);       // which K2s form scores (n_ref = 1, Euclid) rows of this width / alignment
 int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim);   // ... and which form K2s uses for n_ref > 2
+// gallery over ranks (ffr_recheck.cu): the merge key of each row's winner on this rank, and the outputs from the reduced keys
+int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, const float* cand, int64_t n_cand, int32_t dim,
+                     int metric, const int32_t* best_idx, unsigned long long* keys, cudaStream_t s);
+int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, uint8_t* keep, int32_t* best_idx,
+                     float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s);
 int launch_pack_results(const uint8_t* keep, const int32_t* idx, int64_t m, int64_t m_pad, uint8_t* packed,
                         cudaStream_t s);
 int launch_unpack_results(const uint8_t* packed, int64_t m, int64_t m_pad, int nranks, uint8_t* keep, int32_t* idx,

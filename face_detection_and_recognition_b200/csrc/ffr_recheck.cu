@@ -262,6 +262,9 @@ recheck_pairs_phase(float* s_rows, const float* __restrict__ ref, const float* _
 // reused for all kFullGroup candidates), keeps a per-candidate best with strict '>' in ascending order, and the
 // block/ slice results are merged with a 64-bit atomicMax on (orderable(score) << 32 | ~index), which implements
 // "largest score, then smallest index" = np.argmax.  The last slice to arrive writes the outputs.
+// The same key merges a gallery sharded over ranks (ffr_allreduce_best: one ncclMax over uint64, v = -distance for Euclid, key 0
+// = no reference).  sharding.pack_best_keys is its Python twin for torch.distributed, with the top bit flipped so that a SIGNED
+// int64 max orders the keys the same way.
 __device__ __forceinline__ unsigned long long pack_key(float v, int32_t idx) {
     uint32_t u = __float_as_uint(v);
     u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -865,7 +868,104 @@ __global__ void unpack_results_kernel(const uint8_t* __restrict__ packed, int64_
     }
 }
 
+// ---- gallery over ranks (ffr_allreduce_best) --------------------------------------------------------------------------
+// Merge / value pass: the fp32 value of each row's winner on this rank, packed into the merge key with pack_key (above) --
+// (orderable(v) << 32) | ~global_idx, v = cosine score or -distance, so "largest key" = best value, then smallest global index
+// (the first occurrence, np.argmax / np.argmin over the whole gallery).  Key 0 is the identity: a rank without references, or
+// a row whose index lies outside this rank's shard, contributes nothing.  Cosine uses K3's fp32 arithmetic (cos_fp32 on the
+// row's own |c|, lane-strided as in the parked-row form), Euclid K2s's (k2s_euclid_dist in mode emode), so that a rank's value
+// equals what the one-GPU call computes for that same pair.  One warp per row.
+__global__ void __launch_bounds__(kThreads)
+best_key_kernel(const float* __restrict__ ref, int64_t n_ref, int64_t ref_index_base, const float* __restrict__ cand,
+                int64_t n_cand, int32_t dim, const int32_t* __restrict__ best_idx, unsigned long long* __restrict__ keys,
+                bool vec, int emode) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = static_cast<int64_t>(blockIdx.x) * kWarps + (threadIdx.x >> 5);
+    const int64_t nwarps = static_cast<int64_t>(gridDim.x) * kWarps;
+    for (int64_t row = warp; row < n_cand; row += nwarps) {
+        const int32_t g = __ldg(best_idx + row);
+        const int64_t ri = static_cast<int64_t>(g) - ref_index_base;
+        if (ri < 0 || ri >= n_ref) {
+            if (lane == 0) keys[row] = 0ull;
+            continue;
+        }
+        const float* c = cand + row * dim;
+        const float* r = ref + ri * dim;
+        float v;
+        if (emode >= 0) {
+            v = -k2s_euclid_dist(c, r, dim, lane, emode);
+        } else {
+            float cc = 0.f;
+            if (vec) {
+                const float4* c4 = reinterpret_cast<const float4*>(c);
+                for (int k = lane; k < (dim >> 2); k += 32) {
+                    const float4 t = __ldg(c4 + k);
+                    cc = fmaf(t.x, t.x, cc); cc = fmaf(t.y, t.y, cc); cc = fmaf(t.z, t.z, cc); cc = fmaf(t.w, t.w, cc);
+                }
+            } else {
+                for (int d = lane; d < dim; d += 32) { const float t = __ldg(c + d); cc = fmaf(t, t, cc); }
+            }
+            v = cos_fp32(c, r, dim, __fsqrt_rn(warp_sum(cc)), lane, vec);
+        }
+        if (lane == 0) keys[row] = pack_key(v, g);
+    }
+}
+
+// After the all-reduce: global best_idx / best_val, keep from thr and the band, from the winning key.  A row no rank had a
+// reference for (key 0) gets keep 0, index -1 and -inf (cosine) / +inf (Euclid), never in the band.
+__global__ void emit_keys_kernel(const unsigned long long* __restrict__ keys, int64_t n_cand, bool euclid, float thr,
+                                 uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
+                                 float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap) {
+    for (int64_t row = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; row < n_cand;
+         row += static_cast<int64_t>(gridDim.x) * blockDim.x) {
+        const unsigned long long k = keys[row];
+        if (k == 0ull) {
+            keep[row] = 0;
+            best_idx[row] = -1;
+            if (best_val != nullptr) best_val[row] = euclid ? INFINITY : -INFINITY;
+            continue;
+        }
+        float v;
+        int32_t g;
+        unpack_key(k, v, g);
+        const float best = euclid ? -v : v;
+        keep[row] = (euclid ? best <= thr : best >= thr) ? 1 : 0;
+        best_idx[row] = g;
+        if (best_val != nullptr) best_val[row] = best;
+        if (band_count != nullptr && fabsf(best - thr) <= band_tol) {
+            const int32_t slot = atomicAdd(band_count, 1);
+            if (band_rows != nullptr && slot < band_cap) band_rows[slot] = row;
+        }
+    }
+}
+
 }  // namespace
+
+int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, const float* cand, int64_t n_cand, int32_t dim,
+                     int metric, const int32_t* best_idx, unsigned long long* keys, cudaStream_t s) {
+    if (n_cand == 0) return FFR_OK;
+    // K3's choice (launch_recheck) wherever K3 runs: its candidates are always 16-byte aligned there, these need not be
+    const bool vec = (dim % 4 == 0) && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
+                     ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
+    const int emode = metric == FFR_METRIC_EUCLID ? k2s_dist_mode_gallery(ref, cand, dim) : -1;
+    int64_t grid = (n_cand + kWarps - 1) / kWarps;
+    if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
+    best_key_kernel<<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, ref_index_base, cand, n_cand, dim, best_idx,
+                                                                      keys, vec, emode);
+    FFR_LAUNCH_CHECK("best_keys");
+    return FFR_OK;
+}
+
+int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, uint8_t* keep, int32_t* best_idx,
+                     float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s) {
+    if (n_cand == 0) return FFR_OK;
+    int64_t grid = (n_cand + 255) / 256;
+    if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
+    emit_keys_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(keys, n_cand, metric == FFR_METRIC_EUCLID, thr, keep, best_idx,
+                                                                best_val, band_tol, band_count, band_rows, band_cap);
+    FFR_LAUNCH_CHECK("emit_keys");
+    return FFR_OK;
+}
 
 int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim,
                    const float* /*ref_norm*/, const float* /*cand_norm*/, float thr, int64_t ref_index_base,

@@ -407,7 +407,8 @@ class HostFilter:
 
 
 class ResultGather:
-    """K4: one NCCL allgather of the packed per-candidate {best_idx, keep} over NVLink (ffr_comm_*).
+    """K4: one NCCL allgather of the packed per-candidate {best_idx, keep} over NVLink (ffr_comm_*); for a gallery sharded
+    over the ranks, one uint64 max all-reduce of each row's packed best match (``allreduce_best``).
 
     The 128-byte NCCL unique id is created on rank 0 and broadcast through ``torch.distributed`` (any backend)."""
 
@@ -452,6 +453,54 @@ class ResultGather:
             check(self._lib.ffr_allgather_results_inplace(self._h, keep_all.data_ptr(), idx_all.data_ptr(), m,
                                                           _stream_ptr(dev)))
         return keep_all, idx_all
+
+    def allreduce_best(self, ref_local: Optional[torch.Tensor], cand: torch.Tensor, thr: float, best_idx: torch.Tensor,
+                       ref_index_base: int = 0, metric="cosine", band_tol: Optional[float] = None,
+                       out: Optional[Tuple[torch.Tensor, torch.Tensor, torch.Tensor]] = None) -> FilterResult:
+        """Gallery sharded over the ranks (ffr_allreduce_best): ``best_idx`` is this rank's ``face_filter(ref_local, cand, thr,
+        ref_index_base=ref_index_base).best_idx`` (global indices; ``ref_local`` None or empty: this rank has no references
+        and ran no filter).  Returns the result for the whole gallery, identical on every rank: the fp32 value of each rank's
+        winner is recomputed, the best (then the smallest global index) wins one uint64 max all-reduce, and keep / band follow
+        from ``thr``.  A row no rank had a reference for gets keep 0, index -1 and -inf (cosine) / +inf (Euclid)."""
+        m = _METRICS[metric]
+        cand = _require_cuda(cand, "cand")
+        if cand.dim() != 2:
+            raise ValueError(f"cand {tuple(cand.shape)} must be [M, D]")
+        n_cand, dim = cand.shape
+        dev = cand.device
+        n_ref = 0 if ref_local is None else int(ref_local.shape[0])
+        if n_ref:
+            ref_local = _require_cuda(ref_local, "ref_local")
+            if ref_local.dim() != 2 or ref_local.shape[1] != dim or ref_local.device != dev:
+                raise ValueError(f"ref_local {tuple(ref_local.shape)} must be [N, {dim}] on {dev}")
+        if (not isinstance(best_idx, torch.Tensor) or best_idx.dtype != torch.int32 or best_idx.device != dev
+                or tuple(best_idx.shape) != (n_cand,)):
+            raise ValueError(f"best_idx must be an int32 tensor of shape ({n_cand},) on {dev}, got "
+                             f"{getattr(best_idx, 'dtype', type(best_idx))} {tuple(getattr(best_idx, 'shape', ()))} "
+                             f"on {getattr(best_idx, 'device', None)}")
+        if out is None:
+            out = (torch.empty((n_cand,), dtype=torch.uint8, device=dev), torch.empty((n_cand,), dtype=torch.int32, device=dev),
+                   torch.empty((n_cand,), dtype=torch.float32, device=dev))
+        keep, idx, val = out
+        if idx.data_ptr() != best_idx.data_ptr():
+            idx.copy_(best_idx)
+        band_count = band_rows = None
+        if band_tol is not None:
+            band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
+            band_rows = torch.empty((max(n_cand, 1),), dtype=torch.int64, device=dev)
+        ws = _workspace(dev, int(self._lib.ffr_allreduce_best_workspace_bytes(n_cand)))
+        with torch.cuda.device(dev):
+            check(self._lib.ffr_allreduce_best(self._h, ref_local.data_ptr() if n_ref else None, n_ref, int(ref_index_base),
+                                               cand.data_ptr() if n_cand else None, n_cand, dim, m, float(thr),
+                                               keep.data_ptr() if n_cand else None, idx.data_ptr() if n_cand else None,
+                                               val.data_ptr() if n_cand else None, float(band_tol or 0.0),
+                                               band_count.data_ptr() if band_count is not None else None,
+                                               band_rows.data_ptr() if band_rows is not None else None, n_cand,
+                                               ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
+        res = FilterResult(keep, idx, val)
+        if band_tol is not None:
+            res.band_rows = torch.sort(band_rows[:min(int(band_count.item()), n_cand)]).values
+        return res
 
     def all_gather(self, keep_local: torch.Tensor, idx_local: torch.Tensor):
         m = keep_local.numel()

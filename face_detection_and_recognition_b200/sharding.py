@@ -1,4 +1,4 @@
-"""Candidate-axis sharding across the GPUs of one box (SURVEY.md §8e).
+"""Candidate-axis and gallery (reference-axis) sharding across the GPUs of one box (SURVEY.md §8e, DESIGN.md §7).
 
 Every candidate's result depends only on that candidate and the (replicated) reference set, so candidates are split
 into contiguous, equal ranges -- ``m_local = ceil(M / G)`` rows per rank, the last range padded -- each rank runs the
@@ -12,6 +12,11 @@ to 16):
     arrays, one grouped in-place ncclAllGather fills in the others), used on GPUs;
   * ``"dist"``  ``torch.distributed.all_gather_into_tensor`` on the process group the caller initialised -- this is
     what the world_size-2 ``gloo`` tests exercise on CPU (host-side plumbing only; the filter itself is injected).
+
+``GallerySharder`` splits the REFERENCES instead (a gallery too large for one GPU, or a probe batch too small to keep every
+GPU busy streaming the whole gallery): each rank filters the replicated candidates against its contiguous gallery range with
+``ref_index_base`` = the range's start, and one max all-reduce of a 64-bit key per candidate -- the winner's value, then
+its smallest global index -- merges the ranks (``ops.ResultGather.allreduce_best``; ``pack_best_keys`` for ``"dist"``).
 """
 from __future__ import annotations
 
@@ -19,7 +24,8 @@ from typing import Callable, Optional, Tuple
 
 import torch
 
-__all__ = ["shard_range", "pack_results", "unpack_results", "CandidateSharder"]
+__all__ = ["shard_range", "pack_results", "unpack_results", "CandidateSharder", "pack_best_keys", "unpack_best_keys",
+           "GallerySharder"]
 
 
 def shard_range(n_cand: int, world: int, rank: int) -> Tuple[int, int, int]:
@@ -116,6 +122,110 @@ class CandidateSharder:
         dist.all_gather_into_tensor(recv, send)
         keep_all, idx_all = unpack_results(recv, self.world, m_local, n_cand_total)
         return keep_all, idx_all, res
+
+    def close(self):
+        if self._rg is not None:
+            self._rg.close()
+            self._rg = None
+
+
+_EUCLID = ("euclid", "euclidean", 1)
+_U32 = 0xFFFFFFFF
+_KEY_EMPTY = -(1 << 63)
+
+
+def pack_best_keys(val: torch.Tensor, idx: torch.Tensor, metric="cosine") -> torch.Tensor:
+    """int64 merge key of each row's best match: the C key of ffr_allreduce_best, ``(orderable(v) << 32) | ~idx`` with
+    v = score (cosine) or -distance (Euclid), with its top bit flipped so that a SIGNED max orders it like the unsigned C
+    key: the larger value wins, then the smaller index.  ``idx < 0`` (no reference on this rank) packs the identity,
+    the smallest int64."""
+    v = val.to(torch.float32).contiguous()
+    if metric in _EUCLID:
+        v = -v
+    u = v.view(torch.int32).to(torch.int64) & _U32
+    o = torch.where(u >= (1 << 31), (~u) & _U32, u | (1 << 31))
+    idx = idx.to(torch.int64)
+    keys = ((o - (1 << 31)) << 32) | (_U32 - (idx & _U32))
+    return torch.where(idx >= 0, keys, torch.full_like(keys, _KEY_EMPTY))
+
+
+def unpack_best_keys(keys: torch.Tensor, metric="cosine") -> Tuple[torch.Tensor, torch.Tensor]:
+    """Inverse of ``pack_best_keys``: (best_val f32, best_idx i32); the identity gives index -1 and -inf (cosine) /
+    +inf (Euclid)."""
+    o = (keys >> 32) + (1 << 31)
+    u = torch.where(o >= (1 << 31), o & 0x7FFFFFFF, (~o) & _U32)
+    v = (u - (u >= (1 << 31)).to(torch.int64) * (1 << 32)).to(torch.int32).view(torch.float32)
+    idx = (_U32 - (keys & _U32)).to(torch.int64)
+    idx = (idx - (idx >= (1 << 31)).to(torch.int64) * (1 << 32)).to(torch.int32)
+    euclid = metric in _EUCLID
+    if euclid:
+        v = -v
+    empty = keys == _KEY_EMPTY
+    v = torch.where(empty, torch.full_like(v, float("inf") if euclid else float("-inf")), v)
+    return v, torch.where(empty, torch.full_like(idx, -1), idx)
+
+
+class GallerySharder:
+    """Gallery (reference-axis) sharding: rank r holds references ``shard_range(n_ref, world, r)`` and every rank the same
+    candidates (probes); ``filter`` returns the result for the whole gallery, identical on every rank.
+
+    ``reduce="nccl"``: the library's communicator (``ops.ResultGather.allreduce_best``: the fp32 value of every rank's
+    winner is recomputed on the GPU before the merge, so ``face_filter``'s fp16-operand scores are never compared).
+    ``reduce="dist"``: the same keys packed in torch and ``torch.distributed.all_reduce(MAX)`` on int64 over the caller's
+    process group; it merges ``filter_fn``'s ``best_val`` as it is, so it needs an injected fp32 ``filter_fn`` (the CPU
+    ``gloo`` tests inject the oracle).  ``filter_fn(ref_local, cand, thr, metric=..., ref_index_base=...)`` returns an
+    object with ``.best_idx`` (and ``.best_val`` for ``"dist"``)."""
+
+    def __init__(self, rank: int, world: int, device: Optional[int] = None, reduce: str = "nccl",
+                 filter_fn: Optional[Callable] = None):
+        if reduce not in ("nccl", "dist"):
+            raise ValueError("reduce must be 'nccl' or 'dist'")
+        if reduce == "dist" and filter_fn is None:
+            raise ValueError("reduce='dist' merges filter_fn's best_val as it is: inject an fp32 filter_fn")
+        self.rank, self.world, self.device, self.reduce = rank, world, device, reduce
+        if filter_fn is None:
+            from . import ops
+            filter_fn = ops.face_filter
+        self.filter_fn = filter_fn
+        self._rg = None
+        if reduce == "nccl":
+            from . import ops
+            self._rg = ops.ResultGather(rank, world, device if device is not None else 0)
+
+    def shard_range(self, n_ref: int) -> Tuple[int, int]:
+        """[start, stop) of this rank's references; ``start`` is its ``ref_index_base``."""
+        start, stop, _ = shard_range(n_ref, self.world, self.rank)
+        return start, stop
+
+    def filter(self, ref_local: Optional[torch.Tensor], cand: torch.Tensor, thr: float, n_ref_total: int,
+               metric="cosine", band_tol: Optional[float] = None):
+        """``ref_local`` = rows ``shard_range(n_ref_total)`` of the gallery (None or empty on a rank without any), ``cand``
+        the full candidate set.  Returns an ``ops.FilterResult`` for the whole gallery, the same on every rank."""
+        if n_ref_total <= 0:
+            raise ValueError("the gallery is empty")
+        start, stop = self.shard_range(n_ref_total)
+        n_local = 0 if ref_local is None else int(ref_local.shape[0])
+        if n_local != stop - start:
+            raise ValueError(f"rank {self.rank} expects {stop - start} gallery rows, got {n_local}")
+        n_cand = cand.shape[0]
+        res = self.filter_fn(ref_local, cand, thr, metric=metric, ref_index_base=start) if n_local else None
+        if self.reduce == "nccl":
+            idx = res.best_idx if res is not None else torch.full((n_cand,), -1, dtype=torch.int32, device=cand.device)
+            return self._rg.allreduce_best(ref_local if n_local else None, cand, thr, idx, ref_index_base=start,
+                                           metric=metric, band_tol=band_tol)
+        import torch.distributed as dist
+        from .ops import FilterResult
+        if res is not None:
+            keys = pack_best_keys(res.best_val, res.best_idx, metric)
+        else:
+            keys = torch.full((n_cand,), _KEY_EMPTY, dtype=torch.int64, device=cand.device)
+        dist.all_reduce(keys, op=dist.ReduceOp.MAX)
+        val, idx = unpack_best_keys(keys, metric)
+        keep = ((val <= thr) if metric in _EUCLID else (val >= thr)).to(torch.uint8)
+        out = FilterResult(keep, idx, val)
+        if band_tol is not None:
+            out.band_rows = torch.nonzero((val - thr).abs() <= band_tol).reshape(-1)
+        return out
 
     def close(self):
         if self._rg is not None:

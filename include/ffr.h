@@ -197,6 +197,29 @@ int  ffr_allgather_results(ffr_comm* comm, const uint8_t* keep_local, const int3
 int  ffr_allgather_results_inplace(ffr_comm* comm, uint8_t* keep_all, int32_t* idx_all, int64_t m_local,
                                    ffr_stream_t stream);
 
+/* ---- gallery sharded over ranks: merge of the per-rank best matches ---------------------------------------------
+ * The references (the gallery) are split across ranks, the candidates (probes) replicated.  Each rank has run ffr_filter* on
+ * its shard ref_local[n_ref_local, dim] with ref_index_base = the global index of its row 0, and passes that result's best_idx
+ * (device i32[n_cand], global indices) in; on return every rank holds the identical result for the WHOLE gallery in keep,
+ * best_idx and best_val (best_val may be NULL), plus the band (|best - thr| <= band_tol, as ffr_filter_ex).
+ *   1. one kernel recomputes the fp32 value of the rank's winner from ref_local and cand (cosine: K3's arithmetic; Euclid: the
+ *      distance K2s computes) -- the filter's best_val may be an fp16-operand score, which cannot be compared across ranks --
+ *      and packs the key (orderable(v) << 32) | ~idx, v = score (cosine) or -distance (Euclid);
+ *   2. one in-place ncclAllReduce(ncclUint64, ncclMax) over n_cand keys: best value, then the smallest global index (the first
+ *      occurrence over the whole gallery);
+ *   3. one kernel writes best_idx / best_val, decides keep from thr and appends the band.
+ * A rank with an empty shard (n_ref_local = 0, ref_local may be NULL; it runs no filter) contributes the identity key 0, as does
+ * a row whose best_idx lies outside [ref_index_base, ref_index_base + n_ref_local).  A row no rank has a reference for gets
+ * keep 0, best_idx -1, best_val -inf (cosine) / +inf (Euclid).  Precision: the one-GPU gallery contract over the whole gallery
+ * (best_idx equal except on fp32 ties, keep exact outside |best - thr| < 1e-6, Euclid keep / best_val bit-identical to the
+ * one-GPU call wherever best_idx agrees); best_val is always the fp32 value of the returned reference.  Every rank must call
+ * with the same n_cand, metric, thr and band arguments.  The workspace holds n_cand 64-bit keys. */
+size_t ffr_allreduce_best_workspace_bytes(int64_t n_cand);
+int  ffr_allreduce_best(ffr_comm* comm, const float* ref_local, int64_t n_ref_local, int64_t ref_index_base, const float* cand,
+                        int64_t n_cand, int32_t dim, int metric, float thr, uint8_t* keep, int32_t* best_idx, float* best_val,
+                        float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
+                        void* workspace, size_t ws_bytes, ffr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
