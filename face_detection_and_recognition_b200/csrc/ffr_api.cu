@@ -69,30 +69,12 @@ int env_int(const char* name, int dflt) {
 const Knobs* read_knobs() {
     Knobs* k = new Knobs();
     k->cta_group = env_int("FFR_CTA_GROUP", 2);
-    k->a_stages = env_int("FFR_A_STAGES", 0);
-    k->b_stages = env_int("FFR_B_STAGES", 0);
-    k->acc_stages = env_int("FFR_ACC_STAGES", 2);
-    k->diag_half_b = env_int("FFR_DIAG_HALF_B", 0);
-    k->epi_mode = env_int("FFR_EPI_MODE", 0);
-    k->discard_a = env_int("FFR_DISCARD_A", 1);
-    k->decouple_a = env_int("FFR_DECOUPLE_A", 1);
-    k->norm_evict_first = env_int("FFR_NORM_EVICT_FIRST", 1);
-    k->norm_diag = env_int("FFR_NORM_DIAG", 0);
     k->grid_update_refs = env_int("FFR_GRID_UPDATE_REFS", 8192);
     k->grid_exact = env_int("FFR_GRID_EXACT", -1);
-    k->norm_ahead = env_int("FFR_NORM_AHEAD", 2);
     k->fuse_k1 = env_int("FFR_FUSE_K1", -1);
     k->stage32 = env_int("FFR_STAGE32", 1);
-    k->k1_blocks_per_sm = env_int("FFR_K1_BLOCKS_PER_SM", 8);
-    k->k1_subwarp = env_int("FFR_K1_SUBWARP", 1);
-    k->k1_rows = env_int("FFR_K1_ROWS", 8);
-    k->k2s_subwarp = env_int("FFR_K2S_SUBWARP", 1);
     k->dedup_refs = env_int("FFR_DEDUP_REFS", 1);
     k->tail_offload = env_int("FFR_TAIL_OFFLOAD", -1);
-    k->pdl = env_int("FFR_PDL", 1);
-    k->cand_l2_mb = env_int("FFR_CAND_L2_MB", 0);      // stage32: candidate matrices up to this size (MiB) are loaded WITHOUT evict-first (measured: slower)
-    k->last_inline = env_int("FFR_LAST_INLINE", 1);    // stage32 with the offloaded tail: the CTA's last candidate tile is finished by the epilogue warps
-    k->k3_skip = env_int("FFR_K3_SKIP", 0);            // timing experiments: K3 phases left out (1 pairs, 2 parts, 4 full) -- WRONG results
     return k;
 }
 }  // namespace

@@ -33,13 +33,12 @@ int num_sms();                                             // SM count of the cu
 int current_device_slot();                                 // cudaGetDevice clamped to [0, kMaxDevices): index of per-device caches
 constexpr int kMaxDevices = 64;
 
-// ---- tuning / experiment knobs (FFR_* environment variables, DESIGN.md §10) -------------------------
-// Read from the environment ONCE per process (first use); the hot path never calls getenv.  Tests that flip a knob
-// between calls use the non-ABI hook ffr_debug_reload_env().  -1 = "auto" where a knob has a shape-dependent default.
+// ---- dispatch overrides (FFR_* environment variables, DESIGN.md §10) ------------------------------------
+// Each one forces a choice the dispatcher also makes by itself on some shape or platform (tests use them to reach those
+// paths at small sizes).  Read from the environment ONCE per process (first use); the hot path never calls getenv.  Tests
+// that flip one between calls use the non-ABI hook ffr_debug_reload_env().  -1 = "auto" where the default depends on the shape.
 struct Knobs {
-    int cta_group, a_stages, b_stages, acc_stages, diag_half_b, epi_mode, discard_a, decouple_a,
-        norm_evict_first, norm_diag, grid_update_refs, grid_exact, norm_ahead, fuse_k1, stage32, k1_blocks_per_sm,
-        k1_subwarp, k1_rows, k2s_subwarp, dedup_refs, tail_offload, pdl, cand_l2_mb, k3_skip, last_inline;
+    int cta_group, grid_update_refs, grid_exact, fuse_k1, stage32, dedup_refs, tail_offload;
 };
 const Knobs& knobs();
 void reload_knobs();
@@ -223,7 +222,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const void* desc, ui
         ::"r"(smem_u32(smem_dst)), "l"(desc), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "l"(cache_hint)
         : "memory");
 }
-constexpr uint64_t kEvictNormal = 0x1000000000000000ull;
 constexpr uint64_t kEvictFirst  = 0x12F0000000000000ull;
 constexpr uint64_t kEvictLast   = 0x14F0000000000000ull;
 

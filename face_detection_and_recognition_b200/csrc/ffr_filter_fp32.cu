@@ -400,7 +400,7 @@ int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64
         FFR_LAUNCH_CHECK("filter_fp32_generic");
         return FFR_OK;
     }
-    if (n_ref <= 2 && (dim == 128 || dim == 256) && knobs().k2s_subwarp != 0) {
+    if (n_ref <= 2 && (dim == 128 || dim == 256)) {
         const int64_t rows_per_warp = (dim == 128 ? 4 : 2) * 2;
         const int64_t w_needed = (n_cand + rows_per_warp - 1) / rows_per_warp;
         int64_t gsub = (w_needed + (kThreads / 32) - 1) / (kThreads / 32);
@@ -432,7 +432,7 @@ int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64
 int k2s_dist_mode(const float* rows, int32_t dim) {
     const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(rows) & 15) == 0);
     if (!vec_ok) return 0;
-    if ((dim == 128 || dim == 256) && knobs().k2s_subwarp != 0) return dim == 128 ? 16 : 32;
+    if (dim == 128 || dim == 256) return dim == 128 ? 16 : 32;
     const int nv = (dim + 127) / 128;
     return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
 }

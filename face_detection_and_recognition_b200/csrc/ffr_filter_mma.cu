@@ -45,10 +45,6 @@
 
 #include "ffr_common.cuh"
 
-#ifndef FFR_OOB_CLAMP
-#define FFR_OOB_CLAMP 1
-#endif
-
 namespace ffr {
 
 namespace {
@@ -452,23 +448,12 @@ struct KParams {
     const float* cand32;           // kNorm: original fp32 candidate rows [n_cand, dim]
     __half* cand16;                // kNorm: where the normalised fp16 rows go (leading dimension kb_count * 64)
     int32_t dim;                   // kNorm: true embedding size (row pitch of cand32)
-    int acc_stages;                // TMEM accumulator stages in use (2 = MMA of tile t+1 overlaps the epilogue of t)
     int grid_updates;              // epilogue: unconditional grid update path (n_ref <= FFR_GRID_UPDATE_REFS, default 8192)
     int grid_exact;                // update_grid: a part with several in-window columns takes the exact per-column path (1) or only
                                    // flags the row for the full fp32 rescan (0: branch-free; default for dim <= 256, FFR_GRID_EXACT)
-    int norm_diag;                 // kNorm diagnostics (timing only, wrong results): 1 = no loads, 2 = no stores (FFR_NORM_DIAG)
-    int norm_evict_first;          // kNorm: fp32 loads carry the L2 evict-first policy (FFR_NORM_EVICT_FIRST)
-    int norm_ahead;                // kNorm: tiles the normaliser warps may run ahead of the A loads (FFR_NORM_AHEAD, default 2)
-    int decouple_a;                // producer: A loads issued opportunistically while the B stream runs (FFR_DECOUPLE_A, default on)
     int stage32;                   // kNorm, dim_pad == 128: fp32 candidate rows are staged through shared memory by TMA and the normaliser
                                    // warps write the swizzled fp16 A tile directly (no global scratch, no K1 pass at ANY n_ref)
     int s_bufs;                    // stage32: staging ring depth (buffers of kStageRows rows)
-    int last_inline;               // kNormMode 2: the CTA's LAST candidate tile is merged + emitted by the epilogue warps themselves (FFR_LAST_INLINE)
-    int discard_a;                 // kNorm: discard the consumed fp16 rows from L2 (FFR_DISCARD_A, default on)
-    uint64_t cand32_policy;        // stage32: L2 policy of the fp32 candidate loads -- evict-first for a stream larger than L2, plain when the
-                                   // whole candidate matrix fits (K3's fp32 re-check then finds its rows in L2 instead of HBM)
-    uint32_t b_tx_bytes;           // bytes one CTA's B-stage TMA load delivers (diagnostics can halve the box: FFR_DIAG_HALF_B)
-    int epi_mode;                  // diagnostics: 1 = epilogue only loads TMEM (no max tree), results invalid
     unsigned long long* prof;      // optional [gridDim.x][32] stall-cycle counters (diagnostics)
     // kEuclid: score = acc + ref_bias[col] * cand_scale[row] (DESIGN.md section 4, "Euclid on the tensor cores")
     const float* ref_bias;         // -|r|^2 * 2^-f / 2 per (compact) reference column, zero padded to a multiple of kTileN
@@ -635,7 +620,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                   const __grid_constant__ CUtensorMap tmap_cand32, const KParams p) {
     // kNormMode: 0 = the candidates' fp16 rows come from K1, 1 = normaliser warps with global loads + fp16 scratch, 2 = stage32.
     // (Separate instantiations: with stage32 as a run-time branch its mere presence cost the dim-512 kernel 1.5 % of wall clock.)
-    // kInstr: the instrumented build (in-kernel cycle counters, score dump, epilogue diagnostics).  The production
+    // kInstr: the instrumented build (in-kernel cycle counters, score dump).  The production
     // instantiation contains none of it: the counters alone were half a dozen spilled 64-bit values per role.
     static_assert(!kSelf || (kCG == 2 && kNormMode == 0 && !kInstr), "self mode runs on the K1 schedule, cta_group::2, production build");
     constexpr bool kNorm = kNormMode != 0;
@@ -708,9 +693,6 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
     if (kCG == 2) cluster_sync_all(); else __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    // K3 is launched as a programmatic dependent: its blocks may be scheduled as soon as SMs free up and wait (pdl_wait) for
-    // this whole grid to finish -- the launch latency disappears behind our tail.  All our CTAs are already resident.
-    pdl_launch_dependents();
     if (prof_on != nullptr && threadIdx.x == 0) {
         unsigned long long ts;
         asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(ts));
@@ -757,7 +739,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
 #pragma unroll
                     for (int g = 0; g < 4; ++g)               // four 32-float (128-byte, swizzled) column groups of the rows
                         if (g < n_groups)
-                            tma_load_2d(smem_s + sb * kStageBytes + g * (kStageBytes / 4), &tmap_cand32, &s_full[sb], g * 32, r0, p.cand32_policy);
+                            tma_load_2d(smem_s + sb * kStageBytes + g * (kStageBytes / 4), &tmap_cand32, &s_full[sb], g * 32, r0, kEvictFirst);
                     ++s_next;
                     if (++sb == static_cast<uint32_t>(p.s_bufs)) { sb = 0; sph ^= 1; }
                 }
@@ -788,7 +770,6 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     need_a = false;
                 };
                 try_issue_a();
-                if (!p.decouple_a && !st32) { while (need_a) try_issue_a(); }      // (A/B knob: the old blocking order)
                 if (!k1_done) { pdl_wait(); k1_done = true; }
                 for (int rt = 0; rt < (kSelf ? self_rt_end(p, tile, n_rt) : n_rt); ++rt) {
                     int32_t rrow0 = rt * kAccN + static_cast<int32_t>(cta_rank * kBRows);
@@ -797,7 +778,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     // thread waits for b_full ~60 % of its time; cta_group::1, whose box is only partly out of bounds, and 129
                     // references do not show it).  Its columns are >= n_ref, i.e. masked to -inf by index whatever they hold,
                     // so the last in-bounds rows are loaded in its place.
-                    if (kCG == 2 && FFR_OOB_CLAMP && rrow0 >= n_ref) rrow0 = n_ref > static_cast<int64_t>(kBRows) ? static_cast<int32_t>(n_ref) - static_cast<int32_t>(kBRows) : 0;
+                    if (kCG == 2 && rrow0 >= n_ref) rrow0 = n_ref > static_cast<int64_t>(kBRows) ? static_cast<int32_t>(n_ref) - static_cast<int32_t>(kBRows) : 0;
                     for (int kb = 0; kb < p.kb_count; ++kb) {
                         if (need_a) {
                             const long long tw0 = pr ? clock64() : 0;
@@ -806,7 +787,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                         } else {
                             mbar_wait_timed(&b_empty[bs], bph ^ 1, pr, w_bempty);
                         }
-                        if (leader) mbar_expect_tx(&b_full[bs], p.b_tx_bytes * kCG);
+                        if (leader) mbar_expect_tx(&b_full[bs], kBStageBytes * kCG);
                         uint8_t* dst = smem_b + bs * kBStageBytes;
                         if (kCG == 2) tma_load_2d_cg2(dst, &tmap_ref, &b_full[bs], kb * kBlockK, rrow0, kEvictLast);
                         else          tma_load_2d(dst, &tmap_ref, &b_full[bs], kb * kBlockK, rrow0, kEvictLast);
@@ -880,7 +861,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                         if (++bs == static_cast<uint32_t>(p.b_stages)) { bs = 0; bph ^= 1; }
                     }
                     if (kCG == 2) umma_commit_cg2(&t_full[acc]); else umma_commit(&t_full[acc]);       // accumulator ready
-                    if (p.acc_stages == 2) { acc ^= 1u; if (acc == 0u) tph ^= 1u; } else { tph ^= 1u; }
+                    acc ^= 1u; if (acc == 0u) tph ^= 1u;
                     ++t_it;
                 }
                 if (kCG == 2) umma_commit_cg2(&a_empty[as]); else umma_commit(&a_empty[as]);           // A stage reusable
@@ -990,17 +971,13 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     // warp, IPC 0.34, two thirds of the instructions on the FMA pipe), so the 128 squares and the 128 scalings are
                     // issued two per instruction.  Products and the scaled values are the same IEEE results; the sum of squares is
                     // kept in eight partial sums instead of four (1 / |x| can differ in the last place from the earlier form).
-                    // The timing-only knobs (no loads / no stores) exist in the instrumented build alone: as a run-time select they
-                    // cost 63 register-clearing instructions per buffer.
-                    const bool diag_noload = kInstr && (p.norm_diag & 1), diag_nostore = kInstr && (p.norm_diag & 2);
                     float4 x[32];
 #pragma unroll
                     for (int g = 0; g < 4; ++g) {
                         const uint8_t* sg = src + g * (kStageBytes / 4);
 #pragma unroll
                         for (int c = 0; c < 8; ++c)
-                            x[g * 8 + c] = diag_noload ? make_float4(0.f, 0.f, 0.f, 0.f)
-                                                       : *reinterpret_cast<const float4*>(sg + ((static_cast<uint32_t>(c) << 4) ^ sw));
+                            x[g * 8 + c] = *reinterpret_cast<const float4*>(sg + ((static_cast<uint32_t>(c) << 4) ^ sw));
                     }
                     float2 q0 = make_float2(0.f, 0.f), q1 = q0, q2 = q0, q3 = q0;
 #pragma unroll
@@ -1035,13 +1012,13 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                             pk.y = *reinterpret_cast<const uint32_t*>(&h1);
                             pk.z = *reinterpret_cast<const uint32_t*>(&h2);
                             pk.w = *reinterpret_cast<const uint32_t*>(&h3);
-                            if (!diag_nostore) *reinterpret_cast<uint4*>(dg + ((static_cast<uint32_t>(4 * (g & 1) + c) << 4) ^ sw)) = pk;
+                            *reinterpret_cast<uint4*>(dg + ((static_cast<uint32_t>(4 * (g & 1) + c) << 4) ^ sw)) = pk;
                         }
                     }
                     __syncwarp();
                     if (lane == 0) mbar_arrive(&s_empty[sb]);                             // the buffer can be refilled
                 }
-                if (!(p.norm_diag & 4)) fence_proxy_async_smem();   // generic-proxy writes of the A tile -> visible to the MMAs (async proxy)
+                fence_proxy_async_smem();                     // generic-proxy writes of the A tile -> visible to the MMAs (async proxy)
                 __syncwarp();
                 if (lane == 0) {
                     if (kCG == 2 && !leader) mbar_arrive_leader_cta(&a_full[as]);
@@ -1054,8 +1031,8 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 if (++as == static_cast<uint32_t>(p.a_stages)) { as = 0; aph ^= 1; }
             }
             if (kOffload)
-                // drain: the last two tiles (the very last one is merged by the epilogue warps themselves: last_inline)
-                for (uint32_t u = n_done >= 2u ? n_done - 2u : 0u; u + (p.last_inline != 0 ? 1u : 0u) < n_done; ++u) merge_tile(u);
+                // drain: the last two tiles (the very last one is merged by the epilogue warps themselves: inline_last)
+                for (uint32_t u = n_done >= 2u ? n_done - 2u : 0u; u + 1u < n_done; ++u) merge_tile(u);
             if (pr && lane == 0) {
                 p.prof[blockIdx.x * 32 + 13] = static_cast<unsigned long long>(clock64() - t_nv_begin);
                 p.prof[blockIdx.x * 32 + 14] = n_done;
@@ -1067,6 +1044,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
         const int nvec = p.dim >> 2;                                   // float4 per row (dim % 4 == 0 checked on the host)
         const int ld16 = p.kb_count * kBlockK;
         constexpr int kR = 4;                                         // rows in flight per warp
+        constexpr uint32_t kNormAhead = 2;                            // tiles the warps may run ahead of the A loads
         const bool pr = prof_on != nullptr && nw == 0;
         const long long t_nv_begin = clock64();
         uint32_t n_done = 0;
@@ -1074,13 +1052,13 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             const int64_t row0 = tile * (kTileM * kCG) + cta_rank * kTileM;
             // at most two tiles ahead of the TMA loads: the fp16 rows then stay in L2 until they are consumed (running
             // free, the warps finished ALL tiles in a third of the kernel and every row made an HBM round trip)
-            while (n_done >= ld_acquire_shared(cons_count) + static_cast<uint32_t>(p.norm_ahead)) __nanosleep(200);
+            while (n_done >= ld_acquire_shared(cons_count) + kNormAhead) __nanosleep(200);
             // The fp16 rows are scratch: once a tile has been consumed nobody reads them again, and dropping the dirty L2
             // lines spares their write-back to HBM.  Passing the wait above means the A loads of tile n_done - 2 (or later)
             // have been issued, which needs that tile's A stage free, i.e. every MMA of tile n_done - 2 - a_stages retired --
             // and with them that tile's A loads.  (Done here, not by the TMA thread: 1024 discards per tile in the one
             // thread that feeds the B ring cost 7 % of the kernel.)
-            if (p.discard_a && n_done >= 2u + static_cast<uint32_t>(p.a_stages)) {
+            if (n_done >= 2u + static_cast<uint32_t>(p.a_stages)) {
                 const int64_t old_tile = tile - static_cast<int64_t>(2 + p.a_stages) * tile_stride;
                 const int64_t old_row0 = old_tile * (kTileM * kCG) + cta_rank * kTileM;
                 const int64_t bytes = static_cast<int64_t>(kTileM) * ld16 * 2;          // a full tile: it is not the last one
@@ -1099,8 +1077,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
                         const int f = lane + 32 * j;
-                        v[u][j] = (f < nvec && !(p.norm_diag & 1)) ? (p.norm_evict_first ? ldg_stream_evict_first_f4(src + f) : ldg_stream_f4(src + f))
-                                                                   : make_float4(0.f, 0.f, 0.f, 0.f);
+                        v[u][j] = f < nvec ? ldg_stream_evict_first_f4(src + f) : make_float4(0.f, 0.f, 0.f, 0.f);
                     }
                 }
 #pragma unroll
@@ -1129,7 +1106,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                                     pk.x = *reinterpret_cast<const uint32_t*>(&h0);
                                     pk.y = *reinterpret_cast<const uint32_t*>(&h1);
                                 }
-                                if (!(p.norm_diag & 2)) reinterpret_cast<uint2*>(dst)[f] = pk;
+                                reinterpret_cast<uint2*>(dst)[f] = pk;
                             }
                         }
                     }
@@ -1155,8 +1132,8 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
         bool first_tile = true;
         const bool pr = prof_on != nullptr && warp == 4;                 // one part-0 warp reports
         unsigned long long w_tfull = 0, c_hot = 0, c_gen = 0, c_bar1 = 0, c_tail = 0;
-        // diagnostics (score dump, epilogue modes) only exist in the general loop
-        const bool hot_ok = !kInstr || (p.dbg_scores == nullptr && p.epi_mode == 0);
+        // the score dump only exists in the general loop
+        const bool hot_ok = !kInstr || p.dbg_scores == nullptr;
         // the two epilogue policies: compile-time constants in the production instantiations
         const bool grid_updates = kAlways == 2 ? p.grid_updates != 0 : kAlways == 1;     // unconditional update path
         const bool grid_exact = kExact == 2 ? p.grid_exact != 0 : kExact == 1;           // several in-window columns in one part: exact masks, or flag the row
@@ -1192,8 +1169,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             // tile -- the body is what has to stream through the instruction cache.
             auto ref_tile = [&](const int rt, auto partial_tag) {
                 constexpr bool kPartial = decltype(partial_tag)::value;
-                const uint32_t acc = p.acc_stages == 2 ? (t_it & 1) : 0u;
-                const uint32_t tph = p.acc_stages == 2 ? ((t_it >> 1) & 1) : (t_it & 1);
+                const uint32_t acc = t_it & 1, tph = (t_it >> 1) & 1;
                 mbar_wait_timed(&t_full[acc], tph, pr, w_tfull);
                 const long long tp0 = pr ? clock64() : 0;
                 tc_fence_after();
@@ -1263,7 +1239,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     if (grid_updates || m >= gate) update_grid<kChunksPerPart>(v, sx, cm, m, base0, kEuclid ? delta_row : p.delta, grid_exact, t, gate, hid);
                     if (pr) c_hot += static_cast<unsigned long long>(clock64() - tp0);
                 } else {
-                    // ---- general loop, one chunk at a time: diagnostics only (score dump, epilogue modes)
+                    // ---- general loop, one chunk at a time: the score dump only
                     const int ncols = ncols64 > kAccN ? kAccN : static_cast<int>(ncols64);
                     const int n_left = ncols - h * (kChunksPerPart * 32);             // live columns of this warp's part
                     float va[32];
@@ -1277,9 +1253,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                             for (int j = 0; j < 32; ++j)
                                 if (base0 + cc * 32 + j < p.n_ref) p.dbg_scores[row * p.n_ref + base0 + cc * 32 + j] = va[j];
                         }
-                        if (p.epi_mode == 1) { t.b1 = fmax3(t.b1, va[0], va[31]); continue; }
                         const float cmx = chunk_max(va);
-                        if (p.epi_mode == 2) { t.b1 = fmaxf(t.b1, cmx); continue; }
                         if (cmx >= gate) update_chunk(va, cmx, base0 + cc * 32, p.delta, t, gate, hid.amb2);
                     }
                     tc_fence_before();
@@ -1318,7 +1292,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             const long long t_tail0 = pr ? clock64() : 0;
             // ... except for the CTA's LAST candidate tile: nothing is left to overlap its tail with, and four merger warps (32 rows
             // each) finish it in half the time the two helper warps (64 rows each) need -- the kernel's drain.
-            const bool inline_last = kOffload && p.last_inline != 0 && tile + tile_stride >= n_tiles;
+            const bool inline_last = kOffload && tile + tile_stride >= n_tiles;
             if (kOffload && !inline_last) {
                 // stage32 with several reference tiles per candidate tile: the tail is NOT run here.  Merging the two column halves, classifying the row and appending to K3's
                 // lists is ~300 dependent instructions that used to stall this warp for as long as a reference tile's hot loop
@@ -1545,7 +1519,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
         set_error("filter_mma: n_ref / n_cand must be < 2^31");
         return FFR_ERR_UNSUPPORTED;
     }
-    const Knobs& kn = knobs();                         // FFR_* experiment knobs, read once per process (DESIGN.md §10)
+    const Knobs& kn = knobs();                         // FFR_* dispatch overrides, read once per process (DESIGN.md §10)
     const int sms = num_sms();
     // cta_group::2 everywhere: half the B bytes per SM and 8 KB instead of 12 KB of shared-memory operand reads per MMA
     // (measured: dim 128 1292 vs 1152 TFLOP/s, dim 256 1207 vs 1010, dim 512 1429 vs 1212)
@@ -1566,9 +1540,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     constexpr int acc_n = kTileN;
     const uint32_t a_stage = kb * kABlockBytes;
     const uint32_t b_stage = (acc_n / cg) * kBlockK * 2;
-    int a_stages = kn.a_stages > 0 ? kn.a_stages : a_stage_count(dim_pad);
-    if (a_stages < 1) a_stages = 1;
-    if (a_stages > kMaxAStages) a_stages = kMaxAStages;
+    int a_stages = a_stage_count(dim_pad);
     constexpr int ew = 8;                                  // epilogue warps: 4 TMEM lane quadrants x 2 column halves
     // stage32 (fused normalisation, 128-d rows): fp32 rows staged by TMA, two A stages (the normaliser fills one while the
     // MMAs read the other), the B ring gets what is left (>= 2 stages); the tail's hand-over buffer is two slots x two halves
@@ -1586,14 +1558,10 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     if (a_stages * a_stage + 2 * b_stage > budget) { set_error("filter_mma: not enough shared memory for dim %d", dim_pad); return FFR_ERR_UNSUPPORTED; }
     int b_stages = static_cast<int>((budget - a_stages * a_stage) / b_stage);
     if (b_stages > kMaxBStages) b_stages = kMaxBStages;
-    if (kn.b_stages >= 2 && kn.b_stages < b_stages) b_stages = kn.b_stages;
     const uint32_t smem = a_stages * a_stage + b_stages * b_stage + s_bufs * kStageBytes + extra;
 
     CUtensorMap tm_c, tm_r;
-    // FFR_DIAG_HALF_B=1 (timing experiments only, results are wrong): every B load fetches half its rows -- half the L2 -> SM
-    // traffic with the same MMA work, to tell an L2-bandwidth bound from a latency bound
-    const int half_b = kn.diag_half_b ? 2 : 1;
-    int rc = make_tmap(&tm_r, ref16, n_ref, dim_pad, acc_n / cg / half_b);
+    int rc = make_tmap(&tm_r, ref16, n_ref, dim_pad, acc_n / cg);
     if (rc != FFR_OK) return rc;
     if (st32) {
         tm_c = tm_r;                                           // (unused placeholder: stage32 has no fp16 candidate matrix)
@@ -1611,21 +1579,13 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     KParams p;
     p.n_ref = n_ref; p.n_ref_dev = n_ref_dev; p.ref_map = ref_map; p.n_cand = n_cand; p.kb_count = kb; p.a_stages = a_stages; p.b_stages = b_stages;
     p.thr = thr; p.delta = delta; p.thr_band = thr_band; p.ref_index_base = ref_index_base;
-    p.keep = keep; p.best_idx = idx; p.best_val = val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof; p.epi_mode = kn.epi_mode;
+    p.keep = keep; p.best_idx = idx; p.best_val = val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof;
     p.band_tol = band.tol; p.band_count = no_recheck ? band.count : nullptr; p.band_rows = band.rows; p.band_cap = band.cap;
     p.ref_bias = euclid_bias; p.cand_scale = cand_scale; p.bias_max = bias_max;
     p.self_row0 = self.row0; p.self_mode = self.mode;
-    p.acc_stages = kn.acc_stages == 1 ? 1 : 2;
     p.cand32 = cand32; p.cand16 = cand16; p.dim = dim;
-    p.b_tx_bytes = b_stage / half_b;
-    p.discard_a = kn.discard_a;
-    p.decouple_a = kn.decouple_a;
     p.stage32 = st32 ? 1 : 0;
     p.s_bufs = s_bufs;
-    p.last_inline = kn.last_inline;
-    p.cand32_policy = static_cast<double>(n_cand) * dim * 4.0 <= kn.cand_l2_mb * 1048576.0 ? kEvictNormal : kEvictFirst;
-    p.norm_evict_first = kn.norm_evict_first;
-    p.norm_diag = kn.norm_diag;
     p.grid_updates = n_ref <= kn.grid_update_refs ? 1 : 0;
     // The flag-only form hands every same-part near tie to K3, which rescans the 128 references of that part in fp32 (round
     // 1 rescanned ALL references, which only paid for 128-d x >= 32 k references).  It RELIES on K3: without the re-check
@@ -1634,13 +1594,12 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     p.grid_exact = kn.grid_exact >= 0 ? kn.grid_exact : 0;
     if (no_recheck || dbg_scores != nullptr) p.grid_exact = 1;
     if (euclid || self_mode) p.grid_exact = 0;             // (K3 always runs behind the Euclid and the self-mode kernels)
-    p.norm_ahead = kn.norm_ahead < 1 ? 1 : kn.norm_ahead;
 
     typedef void (*KernelFn)(const CUtensorMap, const CUtensorMap, const CUtensorMap, const KParams);
     // Instantiations: cta_group::2 production kernels carry the two epilogue policies as compile-time constants (no dead
     // fall-back code in the hot loop); the instrumented build (tools/diag_mma.py, the tests' score dump) and the
     // cta_group::1 fall-back (odd SM counts, FFR_CTA_GROUP=1) read them at run time.
-    const bool instr = prof != nullptr || dbg_scores != nullptr || p.epi_mode != 0;
+    const bool instr = prof != nullptr || dbg_scores != nullptr;
     const int nm = st32 ? (offload ? 2 : 3) : (fuse ? 1 : 0);
 #define FFR_K(CG, NM, E, A, I) filter_mma_kernel<CG, NM, E, A, I>
 #define FFR_K_POLICY(NM) {FFR_K(2, NM, 0, 0, false), FFR_K(2, NM, 0, 1, false), FFR_K(2, NM, 1, 0, false), FFR_K(2, NM, 1, 1, false)}
@@ -1695,7 +1654,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     attr[0].val.clusterDim.x = cg; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    if (after_k1 && n_ref_dev == nullptr && (kn.pdl & 1) != 0) {   // the previous launch of this stream is K1 (it triggers its dependents at entry)
+    if (after_k1 && n_ref_dev == nullptr) {   // the previous launch of this stream is K1 (it triggers its dependents at entry)
         attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         attr[1].val.programmaticStreamSerializationAllowed = 1;
         cfg.numAttrs = 2;

@@ -198,8 +198,7 @@ static int launch_l2norm_impl(const float* x, int64_t rows, int32_t dim, __half*
     const int64_t warps_needed = (rows + sec.rows + kRowsPerIter - 1) / kRowsPerIter;
     const int64_t blocks_needed = (warps_needed + (kThreads / 32) - 1) / (kThreads / 32);
     // up to 8 resident CTAs per SM (2048 threads); whole multiples of the SM count when the matrix is big
-    const int k1_bps = knobs().k1_blocks_per_sm;
-    int64_t grid = blocks_needed < static_cast<int64_t>(sms) * k1_bps ? blocks_needed : static_cast<int64_t>(sms) * k1_bps;
+    int64_t grid = blocks_needed < static_cast<int64_t>(sms) * 8 ? blocks_needed : static_cast<int64_t>(sms) * 8;
     if (grid < 1) grid = 1;
     const bool vec_ok = (dim % 128 == 0) && (y16 == nullptr || (ld16 % 4 == 0)) &&
                         ((reinterpret_cast<uintptr_t>(x) & 15) == 0) &&
@@ -208,8 +207,7 @@ static int launch_l2norm_impl(const float* x, int64_t rows, int32_t dim, __half*
                         (sec.rows == 0 || ((reinterpret_cast<uintptr_t>(sec.x) & 15) == 0 &&
                                            (reinterpret_cast<uintptr_t>(sec.y16) & 7) == 0));
     const dim3 g(static_cast<unsigned>(grid)), b(kThreads);
-    const bool sub_ok = vec_ok && y32 == nullptr && norms == nullptr && y16 != nullptr && ld16 == dim &&
-                        knobs().k1_subwarp != 0;
+    const bool sub_ok = vec_ok && y32 == nullptr && norms == nullptr && y16 != nullptr && ld16 == dim;
     if (sub_ok && (dim == 128 || dim == 256)) {
         // 8 rows (dim 128) / 4 rows (dim 256) per warp iteration
         const int64_t rows_per_warp = (dim == 128 ? 4 : 2) * 2;
@@ -223,10 +221,7 @@ static int launch_l2norm_impl(const float* x, int64_t rows, int32_t dim, __half*
         FFR_LAUNCH_CHECK("l2norm_rows_sub");
         return FFR_OK;
     }
-    const int k1_rows = knobs().k1_rows;                                   // experiments: rows in flight at dim 128
-    if (vec_ok && dim == 128 && k1_rows == 2)      l2norm_rows_vec_kernel<1, 2><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
-    else if (vec_ok && dim == 128 && k1_rows == 4) l2norm_rows_vec_kernel<1, 4><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
-    else if (vec_ok && dim == 128)  l2norm_rows_vec_kernel<1, 8><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
+    if (vec_ok && dim == 128)       l2norm_rows_vec_kernel<1, 8><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
     else if (vec_ok && dim == 256)  l2norm_rows_vec_kernel<2, 4><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
     else if (vec_ok && dim == 384)  l2norm_rows_vec_kernel<3, 2><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);
     else if (vec_ok && dim == 512)  l2norm_rows_vec_kernel<4, 2><<<g, b, 0, s>>>(x, rows, dim, y16, ld16, y32, norms, sec);

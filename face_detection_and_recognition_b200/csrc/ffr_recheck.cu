@@ -594,7 +594,7 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
                int64_t ref_index_base, uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx,
                float* __restrict__ best_val, RecheckLists lists, float band_tol, int32_t* band_count,
                int64_t* band_rows, int64_t band_cap, const int32_t* __restrict__ ref_map,
-               const int32_t* __restrict__ n_unique_dev, int skip, int emode_arg, SelfArgs self) {
+               const int32_t* __restrict__ n_unique_dev, int emode_arg, SelfArgs self) {
     const int emode = kEuclid ? emode_arg : -1;           // K2s distance mode (Euclid), -1 = cosine
     extern __shared__ __align__(16) float s_c[];               // kFullGroup x dim candidate rows | staged reference tile
     __shared__ float s_ccs[kFullGroup];
@@ -602,14 +602,10 @@ recheck_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __rest
     __shared__ int s_last;
     __shared__ int64_t s_g[kSelf ? kFullGroup : 1];           // kSelf: global indices of the parked full-rescan rows
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    pdl_wait();                 // launched as K2's programmatic dependent: everything below reads K2's lists and outputs
-    if (!(skip & 1))
-        recheck_pairs_phase(s_c, ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
-                            band_rows, band_cap, kVec, emode);
-    if (!(skip & 2))
-        recheck_parts_phase<kSelf>(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol,
-                                   band_count, band_rows, band_cap, kVec, ref_map, n_unique_dev, emode, self);
-    if (skip & 4) return;
+    recheck_pairs_phase(s_c, ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol, band_count,
+                        band_rows, band_cap, kVec, emode);
+    recheck_parts_phase<kSelf>(s_c, ref, n_ref, cand, dim, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol,
+                               band_count, band_rows, band_cap, kVec, ref_map, n_unique_dev, emode, self);
     int64_t count = lists.hdr->full_count;
     if (count > lists.full_cap) count = lists.full_cap;
     if (count == 0) return;
@@ -1001,24 +997,13 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
             attr_set[slot] = true;
         }
     }
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = g2;
-    cfg.blockDim = dim3(kThreads);
-    cfg.dynamicSmemBytes = vec ? smem_full : smem;
-    cfg.stream = s;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;      // K2 (the previous launch) triggers at its entry
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = (knobs().pdl & 2) != 0 ? 1 : 0;        // FFR_PDL bit 1 (bit 0: K1 -> K2)
-    const int skip = knobs().k3_skip;                     // timing experiments only (FFR_K3_SKIP: phases left out, WRONG results)
     auto* fn = self.mode >= 0
                    ? (euclid ? (vec ? recheck_kernel<true, true, true> : recheck_kernel<false, true, true>)
                              : (vec ? recheck_kernel<true, false, true> : recheck_kernel<false, false, true>))
                    : (euclid ? (vec ? recheck_kernel<true, true> : recheck_kernel<false, true>)
                              : (vec ? recheck_kernel<true, false> : recheck_kernel<false, false>));
-    FFR_CUDA_TRY(cudaLaunchKernelEx(&cfg, fn, ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val, lists, band_tol,
-                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, skip, euclid_mode, self));
+    fn<<<g2, kThreads, vec ? smem_full : smem, s>>>(ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val, lists, band_tol,
+                                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, euclid_mode, self);
     FFR_LAUNCH_CHECK("recheck");
     return FFR_OK;
 }

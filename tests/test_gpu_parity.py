@@ -632,14 +632,14 @@ def test_graphed_filter_replays_the_eager_result(ops):
         assert torch.equal(got[0], eager.keep) and torch.equal(got[1], eager.best_idx) and torch.equal(got[2], eager.best_val)
 
 
-@pytest.mark.parametrize("n_cand", [9_000, 40_000, 19_201, 80_001])
-@pytest.mark.parametrize("last_inline", ["0", "1"])
-def test_offloaded_tail_last_tile_both_forms(ops, ffr_env, n_cand, last_inline):
-    """stage32 with the offloaded tail (> 256 references, 128-d): the CTA's last candidate tile is merged + emitted by the
-    epilogue warps themselves (default) or by the helper warps like every other tile (FFR_LAST_INLINE=0).  Sizes with at most
-    one tile per CTA pair (the helper warps then merge nothing at all), two to three, a ragged last tile, and the smallest
-    size range the dispatcher picks this schedule for by itself (the smaller ones force it: FFR_FUSE_K1)."""
-    ffr_env.setenv("FFR_LAST_INLINE", last_inline)
+@pytest.mark.parametrize("n_cand", [200, 9_000, 18_944, 19_201, 37_889, 40_000, 75_776, 80_001])
+def test_offloaded_tail_last_tile_both_forms(ops, ffr_env, n_cand):
+    """stage32 with the offloaded tail (> 256 references, 128-d) has two forms of the end-of-tile work: the CTA's last
+    candidate tile is merged + emitted by the epilogue warps themselves, every other tile by the helper warps.  Sizes (148
+    SMs = 74 CTA pairs of 256-row tiles): one ragged tile for the whole grid, at most one tile per CTA pair (the helper warps
+    then merge nothing at all), exactly one full tile per pair, a ragged last tile, two tiles per pair plus one row, two to
+    three tiles, and the smallest size the dispatcher picks this schedule for by itself and one just above it (the smaller
+    ones force it: FFR_FUSE_K1)."""
     if n_cand < 75_776:
         ffr_env.setenv("FFR_FUSE_K1", "1")
     ref, cand = oracle.make_synthetic(1000, n_cand, 128, seed=n_cand, n_adversarial=300, n_dup_refs=8, unit_norm=False)

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """GPU diagnostic: raw tcgen05 score tiles against a torch fp32 matmul of the same fp16 rows, then quick timings.
-Run on the GPU box:  [FFR_CTA_GROUP=2] python tools/diag_mma.py [--raw] [--perf] [--sweep] [--stream]"""
+Run on the GPU box:  [FFR_CTA_GROUP=2] python tools/diag_mma.py [--raw] [--perf] [--stream]"""
 import os
 import sys
 
@@ -76,7 +76,7 @@ def perf(n_ref, n_cand, dim, flags=0, iters=5, metric="cosine", thr=0.5):
     torch.cuda.synchronize()
     ms = min(ev[i].elapsed_time(ev[i + 1]) for i in range(iters))
     pairs = n_ref * n_cand
-    tag = f"cg={os.environ.get('FFR_CTA_GROUP', '1')} A={os.environ.get('FFR_A_STAGES', '-')} B={os.environ.get('FFR_B_STAGES', '-')}"
+    tag = f"cg={os.environ.get('FFR_CTA_GROUP', '1')}"
     print(f"  perf [{n_ref}x{n_cand}x{dim}] {metric} flags={flags} {tag}: {ms:.3f} ms  {pairs / ms / 1e6:.1f} Gpairs/s  "
           f"{2 * pairs * dim / ms / 1e9:.1f} TFLOP/s  {n_cand * dim * 4 / ms / 1e6:.0f} GB/s(cand)  stats={res.stats} "
           f"keep={res.keep.float().mean().item():.3f}", flush=True)
@@ -144,11 +144,6 @@ if __name__ == "__main__":
         perf(10_000, 1_000_000, 512, flags=ops.FLAG_NO_RECHECK)
         perf(100_000, 1_250_000, 128, flags=ops.FLAG_NO_RECHECK, iters=2)
         perf(256, 2_000_000, 128, flags=ops.FLAG_NO_RECHECK)
-    if "--sweep" in sys.argv and ok:
-        for b in (2, 3, 4, 5, 6):
-            setenv("FFR_B_STAGES", str(b))
-            perf(10_000, 500_000, 256, flags=ops.FLAG_NO_RECHECK, iters=3)
-        delenv("FFR_B_STAGES")
     if "--prof" in sys.argv:
         prof(10_000, 1_000_000, 512)
         prof(10_000, 500_000, 256)
@@ -202,11 +197,7 @@ if __name__ == "__main__":
                 perf(*shape, iters=3)
         delenv("FFR_STAGE32")
     if "--st32prof" in sys.argv:
-        for d in ("0", "1", "2", "3"):
-            setenv("FFR_NORM_DIAG", d)
-            print(" FFR_NORM_DIAG", d)
-            prof(256, 2_000_000, 128)
-        delenv("FFR_NORM_DIAG")
+        prof(256, 2_000_000, 128)
         prof(1000, 100_000, 128)
         for shape in [(1000, 100_000, 128), (256, 2_000_000, 128), (64, 4_000_000, 128), (4000, 400_000, 128)]:
             perf(*shape, iters=3)

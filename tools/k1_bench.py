@@ -15,5 +15,5 @@ for i in range(40):
 torch.cuda.synchronize()
 ts = sorted(ev[i].elapsed_time(ev[i + 1]) for i in range(8, 40))
 med = ts[len(ts) // 2]
-print(f"K1 {rows}x{dim} rows_in_flight={os.environ.get('FFR_K1_ROWS', '8')} blocks/SM={os.environ.get('FFR_K1_BLOCKS_PER_SM', '8')}: median {med * 1e3:.1f} us "
+print(f"K1 {rows}x{dim}: median {med * 1e3:.1f} us "
       f"min {ts[0] * 1e3:.1f} us  {rows * dim * 6 / med / 1e6:.0f} GB/s")
