@@ -99,10 +99,16 @@ namespace {
 
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
-struct WsLayout {
-    size_t hdr, ref16, cand16, recs, full_rows, full_keys, full_ctr, dedup, total;
-    size_t e_bias, e_bias_c, e_nsq, e_scal, e_cscale;     // Euclid on the tensor cores (see EuclidWs)
-    bool mma;
+// One call's workspace, carved into 256-byte aligned buffers.  A buffer the layout leaves out has no bytes: its pointer is the
+// next buffer's and is not used.
+struct Ws {
+    WsHeader* hdr;
+    __half* ref16;
+    __half* cand16;
+    RecheckLists lists;                                   // (header included)
+    void* dedup;                                          // scratch of the duplicate-reference fold
+    float *e_bias, *e_bias_c, *e_nsq, *e_scal, *e_cscale;   // Euclid on the tensor cores
+    size_t total;
 };
 
 // The tcgen05 Euclid kernel exists for cta_group::2 only (an SM count that pairs up, FFR_CTA_GROUP=2): elsewhere Euclid keeps the
@@ -124,28 +130,37 @@ bool mma_eligible(int64_t n_ref, int32_t dim, int metric, int flags) {
 // tiles only ever exist in shared memory: 320 MB less at BASELINE configs[4]'s shard)
 // euclid: the tcgen05 Euclid path's extra buffers -- the reference bias (and its deduplicated copy), the references' squared
 // norms, two scalars, and the candidates' 1 / |c| (n_ref == 0: the caller prepared the references)
-WsLayout ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup,
-                   bool euclid = false) {
-    WsLayout L{};
-    L.mma = mma;
+// base: the workspace to carve (nullptr: only the size is wanted)
+Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup, bool euclid = false,
+             void* base = nullptr) {
+    Ws L{};
     size_t off = 0;
-    L.hdr = off; off += align_up(sizeof(WsHeader), 256);
+    const auto take = [&](size_t bytes) {
+        void* p = reinterpret_cast<void*>(reinterpret_cast<uintptr_t>(base) + off);
+        off += align_up(bytes, 256);
+        return p;
+    };
+    L.hdr = static_cast<WsHeader*>(take(sizeof(WsHeader)));
     if (mma) {
-        const size_t ld = static_cast<size_t>(ffr_padded_dim(dim));
-        L.ref16 = off;  if (dtype == FFR_DTYPE_F32) off += align_up(static_cast<size_t>(n_ref) * ld * 2, 256);
-        L.cand16 = off; if (dtype == FFR_DTYPE_F32 && need_c16) off += align_up(static_cast<size_t>(n_cand) * ld * 2, 256);
-        L.recs = off;      off += align_up(static_cast<size_t>(n_cand) * sizeof(RecheckRec), 256);
-        L.full_rows = off; off += align_up(static_cast<size_t>(n_cand) * sizeof(int32_t), 256);
-        L.full_keys = off; off += align_up(static_cast<size_t>(n_cand) * sizeof(unsigned long long), 256);
-        L.full_ctr = off;  off += align_up((static_cast<size_t>(n_cand) / kFullGroup + 1) * sizeof(int32_t), 256);
-        L.dedup = off;     if (dedup && dtype == FFR_DTYPE_F32) off += align_up(dedup_workspace_bytes(n_ref, static_cast<int32_t>(ld)), 256);
+        const size_t ld = static_cast<size_t>(ffr_padded_dim(dim)), nr = static_cast<size_t>(n_ref), nc = static_cast<size_t>(n_cand);
+        const bool f32 = dtype == FFR_DTYPE_F32;
+        L.ref16 = static_cast<__half*>(take(f32 ? nr * ld * 2 : 0));
+        L.cand16 = static_cast<__half*>(take(f32 && need_c16 ? nc * ld * 2 : 0));
+        L.lists.hdr = L.hdr;
+        L.lists.recs = static_cast<RecheckRec*>(take(nc * sizeof(RecheckRec)));
+        L.lists.rec_cap = n_cand;
+        L.lists.full_rows = static_cast<int32_t*>(take(nc * sizeof(int32_t)));
+        L.lists.full_keys = static_cast<unsigned long long*>(take(nc * sizeof(unsigned long long)));
+        L.lists.full_ctr = static_cast<int32_t*>(take((nc / kFullGroup + 1) * sizeof(int32_t)));
+        L.lists.full_cap = n_cand;
+        L.dedup = take(dedup && f32 ? dedup_workspace_bytes(n_ref, static_cast<int32_t>(ld)) : 0);
         if (euclid) {
             const size_t nb = n_ref > 0 ? static_cast<size_t>(euclid_bias_len(n_ref)) * 4 : 0;
-            L.e_bias = off;    off += align_up(nb, 256);
-            L.e_bias_c = off;  if (dedup) off += align_up(nb, 256);
-            L.e_nsq = off;     off += align_up(static_cast<size_t>(n_ref) * 4, 256);
-            L.e_scal = off;    off += 256;
-            L.e_cscale = off;  off += align_up(static_cast<size_t>(n_cand) * 4, 256);
+            L.e_bias = static_cast<float*>(take(nb));
+            L.e_bias_c = static_cast<float*>(take(dedup ? nb : 0));
+            L.e_nsq = static_cast<float*>(take(nr * 4));
+            L.e_scal = static_cast<float*>(take(256));
+            L.e_cscale = static_cast<float*>(take(nc * 4));
         }
     }
     L.total = off;
@@ -166,15 +181,107 @@ int check_common(const void* ref, int64_t n_ref, const void* cand, int64_t n_can
     return FFR_OK;
 }
 
-// core: ref16_pre != nullptr -> references already normalised/converted (ctx pipeline caches them)
-// ref16_pre != nullptr: the caller already holds the prepared references (fp16, normalised; when map_pre / nuniq_pre are given:
-// exact duplicates folded, see ffr_dedup.cu)
-// ref16_pre with metric Euclid: fp16(r * 2^-f) rows, and euclid_pre = {bias, bias_max} (launch_euclid_refs)
-int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre, const int32_t* nuniq_pre, int64_t n_ref,
-                const void* cand, int64_t n_cand, int32_t dim,
-                int dtype, int metric, float thr, int64_t ref_index_base, uint8_t* keep, int32_t* best_idx,
-                float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, int flags,
-                void* workspace, size_t ws_bytes, cudaStream_t s, const float* const* euclid_pre = nullptr) {
+// K2's reference operand: fp16 rows (cosine: normalised; Euclid: fp16(r * 2^-f), with the bias and its maximum), and when
+// bit-identical rows were folded, the map from K2's columns back to the reference rows and the device-side unique-row count
+struct Refs16 {
+    const __half* rows;
+    const int32_t* map;
+    const int32_t* n_unique;
+    const float* bias;
+    const float* bias_max;
+};
+
+// E1/E2 (ffr_l2norm.cu, two launches): the references' Euclid form into L's buffers
+int prepare_euclid_refs(const float* ref, int64_t n_ref, int32_t dim, const Ws& L, Refs16& r, cudaStream_t s) {
+    r.rows = L.ref16; r.bias = L.e_bias; r.bias_max = L.e_scal + 1;
+    return launch_euclid_refs(ref, n_ref, dim, ffr_padded_dim(dim), L.ref16, L.e_bias, L.e_nsq,
+                              reinterpret_cast<uint32_t*>(L.e_scal), L.e_scal + 1, s);
+}
+
+// Fold bit-identical reference rows (ffr_dedup.cu, four launches): K2 scans the unique ones and maps its columns back; a
+// Euclid bias is compacted with the rows
+int fold_refs(const float* ref, int64_t n_ref, int32_t dim, const Ws& L, Refs16& r, cudaStream_t s) {
+    __half* rows = nullptr;
+    int32_t *map = nullptr, *n_unique = nullptr;
+    float* bias_c = r.bias != nullptr ? L.e_bias_c : nullptr;
+    const int rc = launch_dedup_refs(ref, r.rows, n_ref, dim, ffr_padded_dim(dim), L.dedup, &rows, &map, &n_unique, s, r.bias,
+                                     bias_c);
+    if (rc != FFR_OK) return rc;
+    r = {rows, map, n_unique, bias_c, r.bias_max};
+    return FFR_OK;
+}
+
+// What a caller's preparation hands K2 besides the references
+struct K2In {
+    Refs16 ref;
+    __half* cand16;
+    const float* cand32;        // non-null: K2 normalises the candidates itself (K1 fused)
+    float* cand_scale;          // Euclid: the candidates' 1 / |c| (K1 writes it)
+    bool after_k1;              // the launch right before K2 is K1 (PDL edge)
+    int launches;               // kernels the preparation launched
+};
+
+// One filter call from the workspace checks on: the exact kernel K2s, or the caller's preparation of K2's operands (prep: K1
+// and what goes with it), then K2, K3 and for Euclid the value pass.  ref / cand: the rows K2s, K3 and the value pass read
+// (fp16 input: the rows K2 reads); self.mode >= 0: cand is rows [self.row0, ...) of ref.
+template <class Prep>
+int run_filter(const void* ref, int64_t n_ref, const void* cand, int64_t n_cand, int32_t dim, int dtype, int metric, float thr,
+               int64_t ref_index_base, const FilterOut& out, int flags, SelfArgs self, bool mma, const Ws& L, void* workspace,
+               size_t ws_bytes, const char* ws_hint, cudaStream_t s, Prep prep) {
+    if (workspace == nullptr || ws_bytes < L.total) {
+        set_error("workspace too small: need %zu bytes, got %zu%s", L.total, workspace ? ws_bytes : (size_t)0, ws_hint);
+        return FFR_ERR_WORKSPACE;
+    }
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) { set_error("workspace must be 256-byte aligned"); return FFR_ERR_INVALID; }
+    g_last = {workspace, mma ? 1 : 0, 0};
+    if (out.band.count != nullptr) FFR_CUDA_TRY(cudaMemsetAsync(out.band.count, 0, sizeof(int32_t), s));
+    // the re-check header (list counters) must be zero before K2: the K1 launch does it when there is one
+    if (!(mma && dtype == FFR_DTYPE_F32 && n_cand > 0)) FFR_CUDA_TRY(cudaMemsetAsync(L.hdr, 0, sizeof(WsHeader), s));
+    if (n_cand == 0) return FFR_OK;
+    const float* ref32 = static_cast<const float*>(ref);
+    const float* cand32 = static_cast<const float*>(cand);
+    if (!mma) {
+        if (dtype != FFR_DTYPE_F32) {
+            set_error("fp16 inputs are only accepted by the tcgen05 cosine path (n_ref > 8, dim <= 512; not with metric euclid)");
+            return FFR_ERR_UNSUPPORTED;
+        }
+        g_last.launches = 1;
+        return self.mode >= 0 ? launch_filter_fp32_self(ref32, n_ref, n_cand, dim, metric, self, thr, out, s)
+                              : launch_filter_fp32(ref32, n_ref, cand32, n_cand, dim, metric, thr, ref_index_base, out, s);
+    }
+    K2In in{};
+    int rc = prep(in);
+    if (rc != FFR_OK) return rc;
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    const bool recheck = dtype == FFR_DTYPE_F32 && !(flags & FFR_FLAG_NO_RECHECK);
+    g_last.launches = in.launches + 1 + (recheck ? 1 : 0) + (euclid ? 1 : 0);
+    const float delta = recheck_delta();
+    float thr_band = delta;
+    if (out.band.count != nullptr && out.band.tol + delta > thr_band) thr_band = out.band.tol + delta;
+    if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
+    // Euclid: K2 and K3 only choose the index -- a threshold that never flags a row, no band -- and the value pass decides
+    rc = launch_filter_mma(in.ref.rows, n_ref, in.cand16, in.cand32, dim, n_cand, ffr_padded_dim(dim), euclid ? -INFINITY : thr,
+                           delta, euclid ? 0.f : thr_band, ref_index_base, out, L.lists, recheck ? 0 : 1, in.after_k1, in.ref.map,
+                           in.ref.n_unique, s, in.ref.bias, in.cand_scale, in.ref.bias_max, self);
+    if (rc != FFR_OK) return rc;
+    if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
+    const int emode = euclid ? k2s_form(ref32, cand32, n_ref, dim) : -1;
+    if (recheck) {
+        FilterOut k3 = out;
+        if (euclid) k3.band.count = nullptr;
+        rc = launch_recheck(ref32, n_ref, cand32, n_cand, dim, thr, ref_index_base, k3, L.lists, in.ref.map, in.ref.n_unique, s,
+                            emode, self);
+        if (rc != FFR_OK) return rc;
+    }
+    if (euclid) return launch_euclid_values(ref32, cand32, n_cand, dim, thr, ref_index_base, out, emode, s, self.mode >= 0);
+    return FFR_OK;
+}
+
+// Gallery call.  pre != nullptr: the caller already holds the prepared references (the host-buffer pipeline prepares them once
+// for all its chunks).
+int filter_core(const void* ref, int64_t n_ref, const void* cand, int64_t n_cand, int32_t dim, int dtype, int metric, float thr,
+                int64_t ref_index_base, const FilterOut& out, int flags, void* workspace, size_t ws_bytes, cudaStream_t s,
+                const Refs16* pre = nullptr) {
     const bool mma = mma_eligible(n_ref, dim, metric, flags);
     if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
         set_error("FFR_FLAG_FORCE_MMA: tcgen05 path needs dim <= 512, metric cosine, or metric euclid with n_ref > 8, the re-check "
@@ -187,128 +294,56 @@ int filter_core(const void* ref, const __half* ref16_pre, const int32_t* map_pre
         return FFR_ERR_UNSUPPORTED;
     }
     const int32_t ld = ffr_padded_dim(dim);
+    const float* ref32 = static_cast<const float*>(ref);
+    const float* cand32 = static_cast<const float*>(cand);
     // K2 normalises the candidates itself (K1 fused) when the shape pays for it; in its stage32 form no fp16 copy exists.
     // (Euclid always takes the K1 schedule: K1 also writes the candidates' 1 / |c|.)
-    const bool fuse = mma && !euclid && dtype == FFR_DTYPE_F32 && n_cand > 0 &&
-                      filter_mma_can_fuse(static_cast<const float*>(cand), n_ref, n_cand, dim, ld);
+    const bool fuse = mma && !euclid && dtype == FFR_DTYPE_F32 && n_cand > 0 && filter_mma_can_fuse(cand32, n_ref, n_cand, dim, ld);
     const bool need_c16 = !(fuse && filter_mma_skips_cand16(n_ref, n_cand, dim));
-    const bool dedup = mma && dtype == FFR_DTYPE_F32 && ref16_pre == nullptr && dedup_wanted(n_ref, n_cand);
-    const WsLayout L = ws_layout(ref16_pre ? 0 : n_ref, n_cand, dim, dtype, mma, need_c16, dedup, mma && euclid);
-    if (workspace == nullptr || ws_bytes < L.total) {
-        set_error("workspace too small: need %zu bytes, got %zu%s", L.total, workspace ? ws_bytes : (size_t)0,
-                  (mma && dtype == FFR_DTYPE_F32 && need_c16 && (reinterpret_cast<uintptr_t>(cand) & 15) != 0)
-                      ? " (candidate rows are not 16-byte aligned: the fused schedule ffr_filter_workspace_bytes sized for cannot run)" : "");
-        return FFR_ERR_WORKSPACE;
-    }
-    if (reinterpret_cast<uintptr_t>(workspace) & 255) { set_error("workspace must be 256-byte aligned"); return FFR_ERR_INVALID; }
-    uint8_t* ws = static_cast<uint8_t*>(workspace);
-    WsHeader* hdr = reinterpret_cast<WsHeader*>(ws + L.hdr);
-    g_last = {workspace, mma ? 1 : 0, 0};
-    if (band_count != nullptr) FFR_CUDA_TRY(cudaMemsetAsync(band_count, 0, sizeof(int32_t), s));
-    // the re-check header (list counters) must be zero before K2: the K1 launch does it when there is one
-    const bool k1_runs = mma && dtype == FFR_DTYPE_F32 && n_cand > 0;
-    if (!k1_runs) FFR_CUDA_TRY(cudaMemsetAsync(hdr, 0, sizeof(WsHeader), s));
-    if (n_cand == 0) return FFR_OK;
-
-    if (!mma) {
-        if (dtype != FFR_DTYPE_F32) {
-            set_error("fp16 inputs are only accepted by the tcgen05 cosine path (n_ref > 8, dim <= 512; not with metric euclid)");
-            return FFR_ERR_UNSUPPORTED;
+    const bool dedup = mma && dtype == FFR_DTYPE_F32 && pre == nullptr && dedup_wanted(n_ref, n_cand);
+    const Ws L = ws_layout(pre ? 0 : n_ref, n_cand, dim, dtype, mma, need_c16, dedup, mma && euclid, workspace);
+    const bool misaligned = mma && dtype == FFR_DTYPE_F32 && need_c16 && (reinterpret_cast<uintptr_t>(cand) & 15) != 0;
+    return run_filter(ref, n_ref, cand, n_cand, dim, dtype, metric, thr, ref_index_base, out, flags, kNoSelf, mma, L, workspace,
+                      ws_bytes, misaligned ? " (candidate rows are not 16-byte aligned: the fused schedule ffr_filter_workspace_bytes "
+                                             "sized for cannot run)" : "", s,
+                      [&](K2In& in) {
+        int rc;
+        if (pre != nullptr) in.ref = *pre;
+        if (euclid) {
+            in.cand_scale = L.e_cscale;
+            if (pre == nullptr) {
+                rc = prepare_euclid_refs(ref32, n_ref, dim, L, in.ref, s);
+                if (rc != FFR_OK) return rc;
+                in.launches += 2;
+            }
         }
-        g_last.launches = 1;
-        return launch_filter_fp32(static_cast<const float*>(ref), n_ref, static_cast<const float*>(cand), n_cand, dim,
-                                  metric, thr, ref_index_base, keep, best_idx, best_val, band_tol, band_count,
-                                  band_rows, band_cap, s);
-    }
-
-    const __half* ref16 = ref16_pre;
-    __half* cand16 = nullptr;
-    const float* fuse_cand = nullptr;        // non-null: K2 normalises the candidates itself (K1 fused)
-    int launches = 0;
-    int rc;
-    // Euclid: the reference bias, its maximum and the candidates' 1 / |c| (K2's score is acc + bias * scale)
-    const float* e_bias = nullptr;
-    const float* e_bmax = nullptr;
-    float* e_cscale = nullptr;
-    if (mma && euclid) {
-        e_cscale = reinterpret_cast<float*>(ws + L.e_cscale);
-        if (ref16_pre != nullptr) {
-            e_bias = euclid_pre[0]; e_bmax = euclid_pre[1];
-        } else {
-            __half* r16 = reinterpret_cast<__half*>(ws + L.ref16);
-            float* bias = reinterpret_cast<float*>(ws + L.e_bias);
-            float* scal = reinterpret_cast<float*>(ws + L.e_scal);
-            rc = launch_euclid_refs(static_cast<const float*>(ref), n_ref, dim, ld, r16, bias, reinterpret_cast<float*>(ws + L.e_nsq),
-                                    reinterpret_cast<uint32_t*>(scal), scal + 1, s);
-            if (rc != FFR_OK) return rc;
-            launches += 2;
-            ref16 = r16; e_bias = bias; e_bmax = scal + 1;
+        if (dtype != FFR_DTYPE_F32) {          // fp16 input: K2 reads the rows as they are
+            in.ref.rows = static_cast<const __half*>(ref);
+            in.cand16 = const_cast<__half*>(static_cast<const __half*>(cand));
+            return FFR_OK;
         }
-    }
-    if (dtype == FFR_DTYPE_F32) {
-        // K1: references (unless the caller cached them) and candidates in ONE launch, which also zeroes the header
+        // K1: references (unless prepared already) and candidates in ONE launch, which also zeroes the header
         static_assert(sizeof(WsHeader) % 4 == 0 && sizeof(WsHeader) / 4 <= 256, "header is zeroed by one CTA");
-        __half* r16 = ref16 == nullptr ? reinterpret_cast<__half*>(ws + L.ref16) : nullptr;
-        fuse_cand = fuse ? static_cast<const float*>(cand) : nullptr;
-        __half* c16 = need_c16 ? reinterpret_cast<__half*>(ws + L.cand16) : nullptr;
-        const bool k1_cand = fuse_cand == nullptr;          // otherwise K2's normaliser warps produce the fp16 rows themselves
-        const float* r32 = r16 && !euclid ? static_cast<const float*>(ref) : nullptr;   // (Euclid: prepared above)
-        const int64_t r_rows = r32 ? n_ref : 0;
-        if (k1_cand) rc = launch_l2norm_pair(static_cast<const float*>(cand), n_cand, c16, r32, r_rows, r16, dim, ld, hdr,
-                                             static_cast<int32_t>(sizeof(WsHeader) / 4), s, e_cscale);
-        else         rc = launch_l2norm_pair(r32, r_rows, r16, nullptr, 0, nullptr, dim, ld, hdr,
-                                             static_cast<int32_t>(sizeof(WsHeader) / 4), s);
+        const int32_t hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
+        __half* r16 = in.ref.rows == nullptr ? L.ref16 : nullptr;
+        const float* r32 = r16 ? ref32 : nullptr;
+        const int64_t r_rows = r16 ? n_ref : 0;
+        in.cand32 = fuse ? cand32 : nullptr;
+        in.cand16 = need_c16 ? L.cand16 : nullptr;
+        // (fused: K2's normaliser warps produce the candidates' fp16 rows themselves)
+        if (fuse) rc = launch_l2norm_pair(r32, r_rows, r16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s);
+        else      rc = launch_l2norm_pair(cand32, n_cand, in.cand16, r32, r_rows, r16, dim, ld, L.hdr, hdr_words, s, in.cand_scale);
         if (rc != FFR_OK) return rc;
-        ++launches;
-        if (r16 != nullptr) ref16 = r16;
-        cand16 = c16;
-        if (dedup) {                       // fold bit-identical reference rows: K2 scans the unique ones and maps its columns back
-            __half* r16c = nullptr;
-            int32_t *map = nullptr, *nuniq = nullptr;
-            float* bias_c = euclid ? reinterpret_cast<float*>(ws + L.e_bias_c) : nullptr;
-            rc = launch_dedup_refs(static_cast<const float*>(ref), ref16, n_ref, dim, ld, ws + L.dedup, &r16c, &map, &nuniq, s,
-                                   euclid ? e_bias : nullptr, bias_c);
+        ++in.launches;
+        if (r16 != nullptr) in.ref.rows = r16;
+        if (dedup) {
+            rc = fold_refs(ref32, n_ref, dim, L, in.ref, s);
             if (rc != FFR_OK) return rc;
-            launches += 4;
-            ref16 = r16c; map_pre = map; nuniq_pre = nuniq;
-            if (euclid) e_bias = bias_c;
+            in.launches += 4;
         }
-    } else {
-        if (ref16 == nullptr) ref16 = static_cast<const __half*>(ref);
-        cand16 = const_cast<__half*>(static_cast<const __half*>(cand));      // fp16 input: only read
-    }
-    const bool recheck = (dtype == FFR_DTYPE_F32) && !(flags & FFR_FLAG_NO_RECHECK);
-    g_last.launches = launches + 1 + (recheck ? 1 : 0) + (euclid ? 1 : 0);
-    RecheckLists lists;
-    lists.hdr = hdr;
-    lists.recs = reinterpret_cast<RecheckRec*>(ws + L.recs);
-    lists.rec_cap = n_cand;
-    lists.full_rows = reinterpret_cast<int32_t*>(ws + L.full_rows);
-    lists.full_keys = reinterpret_cast<unsigned long long*>(ws + L.full_keys);
-    lists.full_ctr = reinterpret_cast<int32_t*>(ws + L.full_ctr);
-    lists.full_cap = n_cand;
-    const float delta = recheck_delta();
-    float thr_band = delta;
-    if (band_count != nullptr && band_tol + delta > thr_band) thr_band = band_tol + delta;
-    if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
-    // Euclid: K2 and K3 only choose the index -- a threshold that never flags a row, no band -- and the value pass decides
-    rc = launch_filter_mma(ref16, n_ref, cand16, fuse_cand, dim, n_cand, ld, euclid ? -INFINITY : thr, delta, euclid ? 0.f : thr_band,
-                           ref_index_base, keep, best_idx, best_val, lists, recheck ? 0 : 1, band_tol, band_count, band_rows,
-                           band_cap, /*after_k1=*/dtype == FFR_DTYPE_F32 && !dedup, map_pre, nuniq_pre, s,
-                           e_bias, e_cscale, e_bmax);
-    if (rc != FFR_OK) return rc;
-    if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
-    const int emode = euclid ? k2s_dist_mode_gallery(static_cast<const float*>(ref), static_cast<const float*>(cand), dim) : -1;
-    if (recheck) {
-        rc = launch_recheck(static_cast<const float*>(ref), n_ref, static_cast<const float*>(cand), n_cand, dim, nullptr,
-                            nullptr, thr, ref_index_base, keep, best_idx, best_val, lists, band_tol,
-                            euclid ? nullptr : band_count, band_rows, band_cap, map_pre, nuniq_pre, s, emode);
-        if (rc != FFR_OK) return rc;
-    }
-    if (euclid)
-        return launch_euclid_values(static_cast<const float*>(ref), static_cast<const float*>(cand), n_cand, dim, thr,
-                                    ref_index_base, keep, best_idx, best_val, band_tol, band_count, band_rows, band_cap, emode, s);
-    return FFR_OK;
+        in.after_k1 = !dedup;
+        return FFR_OK;
+    });
 }
 
 // Self mode (ffr_filter_self): x is both matrices.  K1 normalises x ONCE and, for cosine, the A operand is the candidates' slice
@@ -319,14 +354,13 @@ bool self_mma_eligible(int64_t n, int32_t dim, int flags) {
     return !(flags & FFR_FLAG_FORCE_FP32) && dim <= 512 && n > 8 && euclid_mma_available();
 }
 
-WsLayout self_ws_layout(int64_t n, int64_t n_rows, int32_t dim, int metric, bool mma) {
+Ws self_ws_layout(int64_t n, int64_t n_rows, int32_t dim, int metric, bool mma, void* base = nullptr) {
     const bool euclid = metric == FFR_METRIC_EUCLID;
-    return ws_layout(n, n_rows, dim, FFR_DTYPE_F32, mma, /*need_c16=*/euclid, /*dedup=*/false, mma && euclid);
+    return ws_layout(n, n_rows, dim, FFR_DTYPE_F32, mma, /*need_c16=*/euclid, /*dedup=*/false, mma && euclid, base);
 }
 
 int self_core(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, int mode, float thr,
-              uint8_t* keep, int32_t* best_idx, float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows,
-              int64_t band_cap, int flags, void* workspace, size_t ws_bytes, cudaStream_t s) {
+              const FilterOut& out, int flags, void* workspace, size_t ws_bytes, cudaStream_t s) {
     const bool mma = self_mma_eligible(n, dim, flags);
     if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
         set_error("FFR_FLAG_FORCE_MMA: the self-mode tcgen05 path needs n > 8, dim <= 512 and cta_group::2 (n=%lld dim=%d)",
@@ -334,76 +368,26 @@ int self_core(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int3
         return FFR_ERR_UNSUPPORTED;
     }
     const bool euclid = metric == FFR_METRIC_EUCLID;
-    const WsLayout L = self_ws_layout(n, n_rows, dim, metric, mma);
-    if (workspace == nullptr || ws_bytes < L.total) {
-        set_error("workspace too small: need %zu bytes, got %zu", L.total, workspace ? ws_bytes : (size_t)0);
-        return FFR_ERR_WORKSPACE;
-    }
-    if (reinterpret_cast<uintptr_t>(workspace) & 255) { set_error("workspace must be 256-byte aligned"); return FFR_ERR_INVALID; }
-    uint8_t* ws = static_cast<uint8_t*>(workspace);
-    WsHeader* hdr = reinterpret_cast<WsHeader*>(ws + L.hdr);
-    g_last = {workspace, mma ? 1 : 0, 0};
-    if (band_count != nullptr) FFR_CUDA_TRY(cudaMemsetAsync(band_count, 0, sizeof(int32_t), s));
-    if (!(mma && n_rows > 0)) FFR_CUDA_TRY(cudaMemsetAsync(hdr, 0, sizeof(WsHeader), s));     // (otherwise K1 zeroes it)
-    if (n_rows == 0) return FFR_OK;
-    const SelfArgs self{row_begin, mode};
-    if (!mma) {
-        g_last.launches = 1;
-        return launch_filter_fp32_self(x, n, n_rows, dim, metric, self, thr, keep, best_idx, best_val, band_tol, band_count,
-                                       band_rows, band_cap, s);
-    }
-    const int32_t ld = ffr_padded_dim(dim);
+    const Ws L = self_ws_layout(n, n_rows, dim, metric, mma, workspace);
     const float* cand = x + row_begin * dim;
-    __half* x16 = reinterpret_cast<__half*>(ws + L.ref16);
-    __half* c16 = nullptr;
-    const float *e_bias = nullptr, *e_bmax = nullptr;
-    float* e_cscale = nullptr;
-    int rc, launches = 0;
-    const int32_t hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
-    if (euclid) {
-        float* bias = reinterpret_cast<float*>(ws + L.e_bias);
-        float* scal = reinterpret_cast<float*>(ws + L.e_scal);
-        rc = launch_euclid_refs(x, n, dim, ld, x16, bias, reinterpret_cast<float*>(ws + L.e_nsq), reinterpret_cast<uint32_t*>(scal),
-                                scal + 1, s);
-        if (rc != FFR_OK) return rc;
-        c16 = reinterpret_cast<__half*>(ws + L.cand16);
-        e_cscale = reinterpret_cast<float*>(ws + L.e_cscale);
-        rc = launch_l2norm_pair(cand, n_rows, c16, nullptr, 0, nullptr, dim, ld, hdr, hdr_words, s, e_cscale);
-        if (rc != FFR_OK) return rc;
-        launches += 3;
-        e_bias = bias; e_bmax = scal + 1;
-    } else {
-        rc = launch_l2norm_pair(x, n, x16, nullptr, 0, nullptr, dim, ld, hdr, hdr_words, s);
-        if (rc != FFR_OK) return rc;
-        ++launches;
-        c16 = x16 + row_begin * ld;
-    }
-    g_last.launches = launches + 2 + (euclid ? 1 : 0);
-    RecheckLists lists;
-    lists.hdr = hdr;
-    lists.recs = reinterpret_cast<RecheckRec*>(ws + L.recs);
-    lists.rec_cap = n_rows;
-    lists.full_rows = reinterpret_cast<int32_t*>(ws + L.full_rows);
-    lists.full_keys = reinterpret_cast<unsigned long long*>(ws + L.full_keys);
-    lists.full_ctr = reinterpret_cast<int32_t*>(ws + L.full_ctr);
-    lists.full_cap = n_rows;
-    const float delta = recheck_delta();
-    float thr_band = delta;
-    if (band_count != nullptr && band_tol + delta > thr_band) thr_band = band_tol + delta;
-    if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
-    rc = launch_filter_mma(x16, n, c16, nullptr, dim, n_rows, ld, euclid ? -INFINITY : thr, delta, euclid ? 0.f : thr_band, 0,
-                           keep, best_idx, best_val, lists, 0, band_tol, nullptr, band_rows, band_cap, /*after_k1=*/true,
-                           nullptr, nullptr, s, e_bias, e_cscale, e_bmax, self);
-    if (rc != FFR_OK) return rc;
-    if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
-    const int emode = euclid ? k2s_dist_mode_gallery(x, cand, dim) : -1;
-    rc = launch_recheck(x, n, cand, n_rows, dim, nullptr, nullptr, thr, 0, keep, best_idx, best_val, lists, band_tol,
-                        euclid ? nullptr : band_count, band_rows, band_cap, nullptr, nullptr, s, emode, self);
-    if (rc != FFR_OK) return rc;
-    if (euclid)
-        return launch_euclid_values(x, cand, n_rows, dim, thr, 0, keep, best_idx, best_val, band_tol, band_count, band_rows,
-                                    band_cap, emode, s, /*self=*/true);
-    return FFR_OK;
+    return run_filter(x, n, cand, n_rows, dim, FFR_DTYPE_F32, metric, thr, 0, out, flags, SelfArgs{row_begin, mode}, mma, L,
+                      workspace, ws_bytes, "", s, [&](K2In& in) {
+        const int32_t ld = ffr_padded_dim(dim), hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
+        int rc;
+        in.after_k1 = true;
+        if (euclid) {
+            rc = prepare_euclid_refs(x, n, dim, L, in.ref, s);
+            if (rc != FFR_OK) return rc;
+            in.cand16 = L.cand16;
+            in.cand_scale = L.e_cscale;
+            in.launches = 3;
+            return launch_l2norm_pair(cand, n_rows, in.cand16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s, in.cand_scale);
+        }
+        in.ref.rows = L.ref16;
+        in.cand16 = L.ref16 + row_begin * ld;
+        in.launches = 1;
+        return launch_l2norm_pair(x, n, L.ref16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s);
+    });
 }
 
 }  // namespace
@@ -474,8 +458,8 @@ int ffr_filter_ex(const void* ref, int64_t n_ref, const void* cand, int64_t n_ca
     int rc = check_common(ref, n_ref, cand, n_cand, dim, dtype, metric, keep, best_idx);
     if (rc != FFR_OK) return rc;
     if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
-    return filter_core(ref, nullptr, nullptr, nullptr, n_ref, cand, n_cand, dim, dtype, metric, thr, ref_index_base, keep, best_idx,
-                       best_val, band_tol, band_count, band_rows, band_cap, flags, workspace, ws_bytes,
+    return filter_core(ref, n_ref, cand, n_cand, dim, dtype, metric, thr, ref_index_base,
+                       FilterOut{keep, best_idx, best_val, {band_tol, band_count, band_rows, band_cap}}, flags, workspace, ws_bytes,
                        static_cast<cudaStream_t>(stream));
 }
 
@@ -510,8 +494,9 @@ int ffr_filter_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows
         return FFR_ERR_UNSUPPORTED;
     }
     if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
-    return self_core(x, n, row_begin, n_rows, dim, metric, mode, thr, keep, best_idx, best_val, band_tol, band_count, band_rows,
-                     band_cap, flags, workspace, ws_bytes, static_cast<cudaStream_t>(stream));
+    return self_core(x, n, row_begin, n_rows, dim, metric, mode, thr,
+                     FilterOut{keep, best_idx, best_val, {band_tol, band_count, band_rows, band_cap}}, flags, workspace, ws_bytes,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int ffr_filter_stats(const void* workspace, int64_t out[8], ffr_stream_t stream) {
@@ -562,23 +547,12 @@ int ffr_first_match_stream(float* gallery_feat, float* gallery_bbox, int32_t* ga
 int ffr_debug_mma_scores(const void* ref16, int64_t n_ref, const void* cand16, int64_t n_cand, int32_t dim_pad,
                          float thr, uint8_t* keep, int32_t* idx, float* val, float* scores, void* workspace,
                          size_t ws_bytes, ffr_stream_t stream) {
-    const size_t n = static_cast<size_t>(n_cand);
-    const size_t need = 256 + align_up(n * sizeof(RecheckRec), 256) + align_up(n * 4, 256) + align_up(n * 8, 256) +
-                        align_up((n / kFullGroup + 1) * 4, 256);
-    if (workspace == nullptr || ws_bytes < need) { set_error("debug_mma_scores: workspace needs %zu bytes", need); return FFR_ERR_WORKSPACE; }
+    const Ws L = ws_layout(0, n_cand, dim_pad, FFR_DTYPE_F16, /*mma=*/true, false, false, false, workspace);
+    if (workspace == nullptr || ws_bytes < L.total) { set_error("debug_mma_scores: workspace needs %zu bytes", L.total); return FFR_ERR_WORKSPACE; }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    FFR_CUDA_TRY(cudaMemsetAsync(workspace, 0, 256, s));
-    uint8_t* ws = static_cast<uint8_t*>(workspace);
-    RecheckLists lists;
-    lists.hdr = reinterpret_cast<WsHeader*>(ws);
-    size_t off = 256;
-    lists.recs = reinterpret_cast<RecheckRec*>(ws + off); off += align_up(n * sizeof(RecheckRec), 256);
-    lists.full_rows = reinterpret_cast<int32_t*>(ws + off); off += align_up(n * 4, 256);
-    lists.full_keys = reinterpret_cast<unsigned long long*>(ws + off); off += align_up(n * 8, 256);
-    lists.full_ctr = reinterpret_cast<int32_t*>(ws + off);
-    lists.rec_cap = lists.full_cap = n_cand;
+    FFR_CUDA_TRY(cudaMemsetAsync(L.hdr, 0, sizeof(WsHeader), s));
     return launch_filter_mma_debug(static_cast<const __half*>(ref16), n_ref, static_cast<const __half*>(cand16), n_cand,
-                                   dim_pad, thr, recheck_delta(), keep, idx, val, lists, scores, s);
+                                   dim_pad, thr, recheck_delta(), FilterOut{keep, idx, val, {}}, L.lists, scores, s);
 }
 
 }  // extern "C"
@@ -592,12 +566,8 @@ struct ffr_ctx {
     cudaStream_t s_copy, s_comp;
     cudaEvent_t ev_h2d[2], ev_done[2];
     float* d_ref;
-    __half* d_ref16;
-    void* d_dedup;             // scratch of the duplicate-reference fold (per call, not per chunk)
-    float* d_ebias;            // Euclid: reference bias [pad(max_ref)], its deduplicated copy, squared norms, two scalars
-    float* d_ebias_c;
-    float* d_ensq;
-    float* d_escal;
+    void* d_prep;              // the prepared references (per call, not per chunk) ...
+    Ws prep;                   // ... carved: fp16 rows, the duplicate fold's scratch, Euclid's bias, its folded copy and scalars
     float* d_cand[2];
     uint8_t* d_keep[2];
     int32_t* d_idx[2];
@@ -614,8 +584,7 @@ void ffr_ctx_destroy(ffr_ctx* c) {
     cudaSetDevice(c->device);
     if (c->s_comp) cudaStreamSynchronize(c->s_comp);
     if (c->s_copy) cudaStreamSynchronize(c->s_copy);
-    cudaFree(c->d_ref); cudaFree(c->d_ref16); cudaFree(c->d_dedup);
-    cudaFree(c->d_ebias); cudaFree(c->d_ebias_c); cudaFree(c->d_ensq); cudaFree(c->d_escal);
+    cudaFree(c->d_ref); cudaFree(c->d_prep);
     for (int i = 0; i < 2; ++i) {
         cudaFree(c->d_cand[i]); cudaFree(c->d_keep[i]); cudaFree(c->d_idx[i]); cudaFree(c->d_val[i]); cudaFree(c->ws[i]);
         if (c->ev_h2d[i]) cudaEventDestroy(c->ev_h2d[i]);
@@ -638,14 +607,10 @@ int ffr_ctx_create(int device, int64_t max_ref, int64_t chunk_cand, int32_t max_
     FFR_CTX_TRY(cudaSetDevice(device));
     FFR_CTX_TRY(cudaStreamCreateWithFlags(&c->s_copy, cudaStreamNonBlocking));
     FFR_CTX_TRY(cudaStreamCreateWithFlags(&c->s_comp, cudaStreamNonBlocking));
-    const size_t ld = static_cast<size_t>(ffr_padded_dim(max_dim));
     FFR_CTX_TRY(cudaMalloc(&c->d_ref, static_cast<size_t>(max_ref) * max_dim * sizeof(float)));
-    FFR_CTX_TRY(cudaMalloc(&c->d_ref16, static_cast<size_t>(max_ref) * ld * 2));
-    FFR_CTX_TRY(cudaMalloc(&c->d_dedup, dedup_workspace_bytes(max_ref, static_cast<int32_t>(ld))));
-    FFR_CTX_TRY(cudaMalloc(&c->d_ebias, static_cast<size_t>(euclid_bias_len(max_ref)) * sizeof(float)));
-    FFR_CTX_TRY(cudaMalloc(&c->d_ebias_c, static_cast<size_t>(euclid_bias_len(max_ref)) * sizeof(float)));
-    FFR_CTX_TRY(cudaMalloc(&c->d_ensq, static_cast<size_t>(max_ref) * sizeof(float)));
-    FFR_CTX_TRY(cudaMalloc(&c->d_escal, 256));
+    // prepared references: any n_ref <= max_ref and dim <= max_dim, either metric, folded or not
+    FFR_CTX_TRY(cudaMalloc(&c->d_prep, ws_layout(max_ref, 0, max_dim, FFR_DTYPE_F32, true, false, true, true).total));
+    c->prep = ws_layout(max_ref, 0, max_dim, FFR_DTYPE_F32, true, false, true, true, c->d_prep);
     // any dim <= max_dim, either metric
     c->ws_bytes = ws_layout(1, chunk_cand, max_dim <= 512 ? max_dim : 512, FFR_DTYPE_F32, true, true, false, true).total;
     if (c->ws_bytes < 4096) c->ws_bytes = 4096;
@@ -674,26 +639,18 @@ int ffr_ctx_filter_host(ffr_ctx* c, const float* ref, int64_t n_ref, const float
     const int64_t l0 = ffr_launch_count();
     const bool mma = mma_eligible(n_ref, dim, metric, flags);
     FFR_CUDA_TRY(cudaMemcpyAsync(c->d_ref, ref, static_cast<size_t>(n_ref) * dim * sizeof(float), cudaMemcpyHostToDevice, c->s_comp));
-    const __half* ref16 = nullptr;
-    const int32_t *ref_map = nullptr, *n_unique = nullptr;
-    const bool euclid = metric == FFR_METRIC_EUCLID;
-    const float* euclid_pre[2] = {c->d_ebias, c->d_escal + 1};
+    Refs16 pre{};
     if (mma) {      // references are normalised / converted (and exact duplicates folded) once, not per chunk
-        if (euclid)
-            rc = launch_euclid_refs(c->d_ref, n_ref, dim, ffr_padded_dim(dim), c->d_ref16, c->d_ebias, c->d_ensq,
-                                    reinterpret_cast<uint32_t*>(c->d_escal), c->d_escal + 1, c->s_comp);
-        else
-            rc = launch_l2norm(c->d_ref, n_ref, dim, c->d_ref16, ffr_padded_dim(dim), nullptr, nullptr, c->s_comp);
+        if (metric == FFR_METRIC_EUCLID) {
+            rc = prepare_euclid_refs(c->d_ref, n_ref, dim, c->prep, pre, c->s_comp);
+        } else {
+            rc = launch_l2norm(c->d_ref, n_ref, dim, c->prep.ref16, ffr_padded_dim(dim), nullptr, nullptr, c->s_comp);
+            pre.rows = c->prep.ref16;
+        }
         if (rc != FFR_OK) return rc;
-        ref16 = c->d_ref16;
         if (dedup_wanted(n_ref, n_cand)) {
-            __half* r16c = nullptr;
-            int32_t *map = nullptr, *nuniq = nullptr;
-            rc = launch_dedup_refs(c->d_ref, c->d_ref16, n_ref, dim, ffr_padded_dim(dim), c->d_dedup, &r16c, &map, &nuniq, c->s_comp,
-                                   euclid ? c->d_ebias : nullptr, c->d_ebias_c);
+            rc = fold_refs(c->d_ref, n_ref, dim, c->prep, pre, c->s_comp);
             if (rc != FFR_OK) return rc;
-            ref16 = r16c; ref_map = map; n_unique = nuniq;
-            if (euclid) euclid_pre[0] = c->d_ebias_c;
         }
     }
     int64_t i = 0;
@@ -705,9 +662,9 @@ int ffr_ctx_filter_host(ffr_ctx* c, const float* ref, int64_t n_ref, const float
                                      cudaMemcpyHostToDevice, c->s_copy));
         FFR_CUDA_TRY(cudaEventRecord(c->ev_h2d[b], c->s_copy));
         FFR_CUDA_TRY(cudaStreamWaitEvent(c->s_comp, c->ev_h2d[b], 0));
-        rc = filter_core(c->d_ref, ref16, ref_map, n_unique, n_ref, c->d_cand[b], m, dim, FFR_DTYPE_F32, metric, thr, ref_index_base,
-                         c->d_keep[b], c->d_idx[b], c->d_val[b], 0.f, nullptr, nullptr, 0, flags, c->ws[b], c->ws_bytes,
-                         c->s_comp, euclid_pre);
+        rc = filter_core(c->d_ref, n_ref, c->d_cand[b], m, dim, FFR_DTYPE_F32, metric, thr, ref_index_base,
+                         FilterOut{c->d_keep[b], c->d_idx[b], c->d_val[b], {}}, flags, c->ws[b], c->ws_bytes, c->s_comp,
+                         mma ? &pre : nullptr);
         if (rc != FFR_OK) return rc;
         FFR_CUDA_TRY(cudaMemcpyAsync(keep + off, c->d_keep[b], static_cast<size_t>(m), cudaMemcpyDeviceToHost, c->s_comp));
         FFR_CUDA_TRY(cudaMemcpyAsync(best_idx + off, c->d_idx[b], static_cast<size_t>(m) * sizeof(int32_t), cudaMemcpyDeviceToHost, c->s_comp));
@@ -901,7 +858,8 @@ int ffr_allreduce_best(ffr_comm* c, const float* ref_local, int64_t n_ref_local,
     if (rc != FFR_OK) return rc;
     const int e = g_nccl.allreduce(keys, keys, static_cast<size_t>(n_cand), /*ncclUint64*/ 5, /*ncclMax*/ 2, c->comm, s);
     if (e != 0) return nccl_fail(e, "ncclAllReduce");
-    return launch_emit_keys(keys, n_cand, metric, thr, keep, best_idx, best_val, band_tol, band_count, band_rows, band_cap, s);
+    return launch_emit_keys(keys, n_cand, metric, thr, FilterOut{keep, best_idx, best_val, {band_tol, band_count, band_rows, band_cap}},
+                            s);
 }
 
 }  // extern "C"

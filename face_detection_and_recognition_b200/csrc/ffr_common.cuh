@@ -86,6 +86,22 @@ struct SelfArgs {
 };
 constexpr SelfArgs kNoSelf = {0, -1};
 
+// ---- a filter call's outputs (host launchers; K2s and the value pass take Band as a kernel parameter) ----------------------
+// Rows with |best - thr| <= tol are appended (unordered) to rows[0..cap) and counted in *count (which may exceed cap);
+// count nullptr: no band.
+struct Band {
+    float tol;
+    int32_t* count;
+    int64_t* rows;
+    int64_t cap;
+};
+struct FilterOut {
+    uint8_t* keep;
+    int32_t* idx;
+    float* val;            // may be nullptr
+    Band band;
+};
+
 // ---- device helpers -------------------------------------------------------------------------------
 #ifdef __CUDACC__
 
@@ -110,7 +126,7 @@ __device__ __forceinline__ float warp_sum(float v) {
 // filter K2s uses for an Euclid score (ffr_filter_fp32.cu), so that K5's threshold -- the largest reference-to-mean distance --
 // is bit-identical to the distance the filter later computes for that same reference as a candidate (the reference gets both
 // from one np.linalg.norm: the farthest reference always passes `<= thres`, filter_faces_using_reference.py:88-99,189).
-// mode (k2s_dist_mode on the host): 0 = scalar lane-strided; 1, 2, 4, 8 = float4 #(lane + 32 j), j < mode; 16 / 32 = sub-warp
+// mode (k2s_form on the host): 0 = scalar lane-strided; 1, 2, 4, 8 = float4 #(lane + 32 j), j < mode; 16 / 32 = sub-warp
 // form, 8 / 16 lanes per row with float4 #(sub + L j), j < 4.  The whole warp calls it; every lane returns the distance.
 __device__ __forceinline__ float k2s_euclid_dist(const float* __restrict__ c, const float* m, int32_t dim, int lane, int mode) {
     float a = 0.f;
@@ -329,12 +345,15 @@ __device__ __host__ constexpr uint32_t umma_idesc_f16(uint32_t m, uint32_t n) {
 int launch_l2norm(const float* x, int64_t rows, int32_t dim, __half* y16, int32_t ld16, float* y32, float* norms,
                   cudaStream_t s);
 int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric,
-                       float thr, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
-                       float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s);
+                       float thr, int64_t ref_index_base, const FilterOut& out, cudaStream_t s);
 // K2s self form: candidates x[self.row0 .. self.row0 + n_cand) against all n rows of x, excluded references skipped
 int launch_filter_fp32_self(const float* x, int64_t n, int64_t n_cand, int32_t dim, int metric, SelfArgs self, float thr,
-                            uint8_t* keep, int32_t* idx, float* val, float band_tol, int32_t* band_count, int64_t* band_rows,
-                            int64_t band_cap, cudaStream_t s);
+                            const FilterOut& out, cudaStream_t s);
+// The form K2s scores (ref, cand) row pairs with when it scans n_ref references (launch_filter_fp32 dispatches on it):
+// 0 = scalar lane-strided; 1, 2, 4, 8 = float4 per lane; 16 / 32 = the sub-warp kernel (n_ref <= 2, dim 128 / 256).  Every
+// kernel whose Euclid distance must be K2s's bit for bit (K5, K3's Euclid form, the value pass, the all-reduce merge) takes
+// k2s_euclid_dist's mode from it.
+int k2s_form(const float* ref, const float* cand, int64_t n_ref, int32_t dim);
 int launch_l2norm_pair(const float* x_a, int64_t rows_a, __half* y16_a, const float* x_b, int64_t rows_b, __half* y16_b,
                        int32_t dim, int32_t ld16, void* zero_ptr, int32_t zero_words, cudaStream_t s,
                        float* scale_a = nullptr);
@@ -346,10 +365,9 @@ int launch_euclid_refs(const float* ref, int64_t n_ref, int32_t dim, int32_t ld1
 inline int64_t euclid_bias_len(int64_t n_ref) { return (n_ref + 255) / 256 * 256; }
 bool filter_mma_can_fuse(const float* cand32, int64_t n_ref, int64_t n_cand, int32_t dim, int32_t dim_pad);
 int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const float* cand32, int32_t dim,
-                      int64_t n_cand, int32_t dim_pad,
-                      float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
-                      RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
-                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
+                      int64_t n_cand, int32_t dim_pad, float thr, float delta, float thr_band, int64_t ref_index_base,
+                      const FilterOut& out, RecheckLists lists, int no_recheck, bool after_k1, const int32_t* ref_map,
+                      const int32_t* n_ref_dev, cudaStream_t s,
                       const float* euclid_bias = nullptr, const float* cand_scale = nullptr, const float* bias_max = nullptr,
                       SelfArgs self = kNoSelf);
 // exact-duplicate reference rows folded before K2 (ffr_dedup.cu)
@@ -360,16 +378,13 @@ int launch_dedup_refs(const float* ref32, const __half* ref16_full, int64_t n_re
                       const float* bias = nullptr, float* bias_c = nullptr);   // Euclid: the bias is compacted with the rows
 bool filter_mma_skips_cand16(int64_t n_ref, int64_t n_cand, int32_t dim);
 void get_last_k2_config(int out[8]);
-int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim,
-                   const float* ref_norm, const float* cand_norm, float thr, int64_t ref_index_base,
-                   uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
-                   float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode = -1,
-                   SelfArgs self = kNoSelf);
-// Euclid after the tensor-core pass: keep / best_val / band from the K2s distance to the chosen reference (ffr_filter_fp32.cu)
+int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, float thr,
+                   int64_t ref_index_base, const FilterOut& out, RecheckLists lists, const int32_t* ref_map,
+                   const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode = -1, SelfArgs self = kNoSelf);
+// Euclid after the tensor-core pass: keep / best_val / band from the K2s distance to the chosen reference out.idx (only read)
+// (ffr_filter_fp32.cu)
 int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
-                         uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
-                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s, bool self = false);
+                         const FilterOut& out, int mode, cudaStream_t s, bool self = false);
 int launch_ref_stats_batched(const float* ref_feat, const int32_t* offsets, int32_t n_classes, int32_t dim, float* mean,
                              float* thres, cudaStream_t s);
 int launch_first_match_stream(float* g_feat, float* g_bbox, int32_t* g_count, int32_t cap, const float* queries,
@@ -377,19 +392,15 @@ int launch_first_match_stream(float* g_feat, float* g_bbox, int32_t* g_count, in
                               float harsh_thres, int32_t* match_idx, cudaStream_t s);
 void set_mma_prof_buffer(unsigned long long* dev_ptr);   // diagnostics: [grid][16] stall-cycle counters of K2
 int launch_ref_stats(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres, cudaStream_t s);
-int k2s_dist_mode(const float* rows, int32_t dim);       // which K2s form scores (n_ref = 1, Euclid) rows of this width / alignment
-int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim);   // ... and which form K2s uses for n_ref > 2
 // gallery over ranks (ffr_recheck.cu): the merge key of each row's winner on this rank, and the outputs from the reduced keys
 int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, const float* cand, int64_t n_cand, int32_t dim,
                      int metric, const int32_t* best_idx, unsigned long long* keys, cudaStream_t s);
-int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, uint8_t* keep, int32_t* best_idx,
-                     float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s);
+int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, const FilterOut& out, cudaStream_t s);
 int launch_pack_results(const uint8_t* keep, const int32_t* idx, int64_t m, int64_t m_pad, uint8_t* packed,
                         cudaStream_t s);
 int launch_unpack_results(const uint8_t* packed, int64_t m, int64_t m_pad, int nranks, uint8_t* keep, int32_t* idx,
                           cudaStream_t s);
 int launch_filter_mma_debug(const __half* ref16, int64_t n_ref, const __half* cand16, int64_t n_cand, int32_t dim_pad,
-                            float thr, float delta, uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
-                            float* scores, cudaStream_t s);
+                            float thr, float delta, const FilterOut& out, RecheckLists lists, float* scores, cudaStream_t s);
 
 }  // namespace ffr

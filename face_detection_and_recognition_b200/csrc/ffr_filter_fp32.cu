@@ -25,13 +25,6 @@ namespace {
 
 constexpr int kThreads = 256;
 
-struct BandOut {
-    float tol;
-    int32_t* count;
-    int64_t* rows;
-    int64_t cap;
-};
-
 template <int NV, bool kCosine>
 __device__ __forceinline__ void score_row(const float4 (&c)[NV], const float4 (&r)[NV], float cc_sqrt, float& score) {
     // returns cosine similarity or euclid distance of the candidate (regs c) and one reference (regs r)
@@ -80,7 +73,7 @@ __global__ void __launch_bounds__(kThreads)
 filter_fp32_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int64_t n_cand,
                    int32_t dim, float thr, int64_t ref_index_base,
                    uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
-                   BandOut band, SelfArgs self) {
+                   Band band, SelfArgs self) {
     static_assert(!kSelf || kRegRefs == 0, "self form: references from global memory");
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
@@ -165,7 +158,7 @@ __global__ void __launch_bounds__(kThreads)
 filter_fp32_sub_kernel(const float* __restrict__ ref, int32_t n_ref, const float* __restrict__ cand, int64_t n_cand,
                        int32_t dim, float thr, int64_t ref_index_base,
                        uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
-                       BandOut band) {
+                       Band band) {
     constexpr int kRowsPerWarp = 32 / L;
     constexpr int kGroups = 2;                                      // row groups in flight per warp (4 KB)
     const int lane = threadIdx.x & 31, sub = lane % L, rsel = lane / L;
@@ -257,7 +250,7 @@ __global__ void __launch_bounds__(kThreads)
 filter_fp32_generic_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand,
                            int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
                            uint8_t* __restrict__ keep, int32_t* __restrict__ best_idx, float* __restrict__ best_val,
-                           BandOut band, SelfArgs self) {
+                           Band band, SelfArgs self) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
@@ -339,7 +332,7 @@ template <int kMode, bool kSelf = false>
 __global__ void __launch_bounds__(kThreads)
 euclid_value_kernel(const float* __restrict__ ref, const float* __restrict__ cand, int64_t n_cand, int32_t dim, float thr,
                     int64_t ref_index_base, uint8_t* __restrict__ keep, const int32_t* __restrict__ best_idx,
-                    float* __restrict__ best_val, BandOut band) {
+                    float* __restrict__ best_val, Band band) {
     const int lane = threadIdx.x & 31;
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
@@ -365,16 +358,16 @@ euclid_value_kernel(const float* __restrict__ ref, const float* __restrict__ can
 
 template <int NV, bool kCosine>
 int launch_vec(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, float thr,
-               int64_t base, uint8_t* keep, int32_t* idx, float* val, BandOut band, dim3 g, cudaStream_t s) {
+               int64_t base, const FilterOut& o, dim3 g, cudaStream_t s) {
     const dim3 b(kThreads);
     const int64_t ref_vecs = n_ref * NV;
     if (ref_vecs <= 8) {
-        if (n_ref == 1)      filter_fp32_kernel<NV, kCosine, 1><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
-        else if (n_ref == 2) filter_fp32_kernel<NV, kCosine, 2><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
-        else if (n_ref <= 4) filter_fp32_kernel<NV, kCosine, (NV <= 2 ? 4 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
-        else                 filter_fp32_kernel<NV, kCosine, (NV == 1 ? 8 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
+        if (n_ref == 1)      filter_fp32_kernel<NV, kCosine, 1><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, o.keep, o.idx, o.val, o.band, kNoSelf);
+        else if (n_ref == 2) filter_fp32_kernel<NV, kCosine, 2><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, o.keep, o.idx, o.val, o.band, kNoSelf);
+        else if (n_ref <= 4) filter_fp32_kernel<NV, kCosine, (NV <= 2 ? 4 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, o.keep, o.idx, o.val, o.band, kNoSelf);
+        else                 filter_fp32_kernel<NV, kCosine, (NV == 1 ? 8 : 1)><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, o.keep, o.idx, o.val, o.band, kNoSelf);
     } else {
-        filter_fp32_kernel<NV, kCosine, 0><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, keep, idx, val, band, kNoSelf);
+        filter_fp32_kernel<NV, kCosine, 0><<<g, b, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, base, o.keep, o.idx, o.val, o.band, kNoSelf);
     }
     FFR_LAUNCH_CHECK("filter_fp32");
     return FFR_OK;
@@ -382,25 +375,31 @@ int launch_vec(const float* ref, int64_t n_ref, const float* cand, int64_t n_can
 
 }  // namespace
 
+int k2s_form(const float* ref, const float* cand, int64_t n_ref, int32_t dim) {
+    const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
+                        ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
+    if (!vec_ok) return 0;                                                     // filter_fp32_generic_kernel
+    if (n_ref <= 2 && (dim == 128 || dim == 256)) return dim == 128 ? 16 : 32;   // filter_fp32_sub_kernel<dim / 16>
+    const int nv = (dim + 127) / 128;                                          // filter_fp32_kernel<NV>
+    return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
+}
+
 int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric,
-                       float thr, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
-                       float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s) {
+                       float thr, int64_t ref_index_base, const FilterOut& o, cudaStream_t s) {
     if (n_cand == 0) return FFR_OK;
     const int sms = num_sms();
     const int64_t blocks_needed = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
     int64_t grid = blocks_needed < static_cast<int64_t>(sms) * 8 ? blocks_needed : static_cast<int64_t>(sms) * 8;
     const dim3 g(static_cast<unsigned>(grid));
-    BandOut band{band_tol, band_count, band_rows, band_cap};
     const bool cosine = metric == FFR_METRIC_COSINE;
-    const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
-                        ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
-    if (!vec_ok) {
-        if (cosine) filter_fp32_generic_kernel<true><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, kNoSelf);
-        else        filter_fp32_generic_kernel<false><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, kNoSelf);
+    const int form = k2s_form(ref, cand, n_ref, dim);
+    if (form == 0) {
+        if (cosine) filter_fp32_generic_kernel<true><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band, kNoSelf);
+        else        filter_fp32_generic_kernel<false><<<g, kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band, kNoSelf);
         FFR_LAUNCH_CHECK("filter_fp32_generic");
         return FFR_OK;
     }
-    if (n_ref <= 2 && (dim == 128 || dim == 256)) {
+    if (form >= 16) {
         const int64_t rows_per_warp = (dim == 128 ? 4 : 2) * 2;
         const int64_t w_needed = (n_cand + rows_per_warp - 1) / rows_per_warp;
         int64_t gsub = (w_needed + (kThreads / 32) - 1) / (kThreads / 32);
@@ -408,98 +407,77 @@ int launch_filter_fp32(const float* ref, int64_t n_ref, const float* cand, int64
         const dim3 gs(static_cast<unsigned>(gsub));
         const int32_t nr = static_cast<int32_t>(n_ref);
         if (dim == 128) {
-            if (cosine) filter_fp32_sub_kernel<8, true><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
-            else        filter_fp32_sub_kernel<8, false><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
+            if (cosine) filter_fp32_sub_kernel<8, true><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band);
+            else        filter_fp32_sub_kernel<8, false><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band);
         } else {
-            if (cosine) filter_fp32_sub_kernel<16, true><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
-            else        filter_fp32_sub_kernel<16, false><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band);
+            if (cosine) filter_fp32_sub_kernel<16, true><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band);
+            else        filter_fp32_sub_kernel<16, false><<<gs, kThreads, 0, s>>>(ref, nr, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band);
         }
         FFR_LAUNCH_CHECK("filter_fp32_sub");
         return FFR_OK;
     }
-    const int nv = (dim + 127) / 128;
 #define FFR_DISPATCH(NV)                                                                                          \
-    return cosine ? launch_vec<NV, true>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, g, s) \
-                  : launch_vec<NV, false>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band, g, s)
-    if (nv <= 1) { FFR_DISPATCH(1); }
-    if (nv <= 2) { FFR_DISPATCH(2); }
-    if (nv <= 4) { FFR_DISPATCH(4); }
-    FFR_DISPATCH(8);
+    return cosine ? launch_vec<NV, true>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, o, g, s)             \
+                  : launch_vec<NV, false>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, o, g, s)
+    switch (form) {
+        case 1: FFR_DISPATCH(1);
+        case 2: FFR_DISPATCH(2);
+        case 4: FFR_DISPATCH(4);
+        default: FFR_DISPATCH(8);
+    }
 #undef FFR_DISPATCH
 }
 
-// mirrors launch_filter_fp32's choice of kernel for (n_ref = 1, metric Euclid)
-int k2s_dist_mode(const float* rows, int32_t dim) {
-    const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(rows) & 15) == 0);
-    if (!vec_ok) return 0;
-    if (dim == 128 || dim == 256) return dim == 128 ? 16 : 32;
-    const int nv = (dim + 127) / 128;
-    return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
-}
-
-// mirrors launch_filter_fp32's choice of kernel for n_ref > 2 (metric Euclid): the warp-per-row kernel with NV float4 per lane,
-// or the scalar catch-all
-int k2s_dist_mode_gallery(const float* ref, const float* cand, int32_t dim) {
-    const bool vec_ok = (dim % 4 == 0) && dim <= 1024 && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
-                        ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
-    if (!vec_ok) return 0;
-    const int nv = (dim + 127) / 128;
-    return nv <= 1 ? 1 : (nv <= 2 ? 2 : (nv <= 4 ? 4 : 8));
-}
-
 int launch_euclid_values(const float* ref, const float* cand, int64_t n_cand, int32_t dim, float thr, int64_t ref_index_base,
-                         uint8_t* keep, const int32_t* idx, float* val, float band_tol, int32_t* band_count,
-                         int64_t* band_rows, int64_t band_cap, int mode, cudaStream_t s, bool self) {
+                         const FilterOut& o, int mode, cudaStream_t s, bool self) {
     if (n_cand == 0) return FFR_OK;
     int64_t grid = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
     if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
     const dim3 g(static_cast<unsigned>(grid));
-    const BandOut band{band_tol, band_count, band_rows, band_cap};
     if (self) {
         switch (mode) {
-            case 1: euclid_value_kernel<1, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-            case 2: euclid_value_kernel<2, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-            case 4: euclid_value_kernel<4, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-            case 8: euclid_value_kernel<8, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-            default: euclid_value_kernel<0, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+            case 1: euclid_value_kernel<1, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+            case 2: euclid_value_kernel<2, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+            case 4: euclid_value_kernel<4, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+            case 8: euclid_value_kernel<8, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+            default: euclid_value_kernel<0, true><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
         }
         FFR_LAUNCH_CHECK("euclid_values");
         return FFR_OK;
     }
     switch (mode) {
-        case 1: euclid_value_kernel<1><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-        case 2: euclid_value_kernel<2><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-        case 4: euclid_value_kernel<4><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-        case 8: euclid_value_kernel<8><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
-        default: euclid_value_kernel<0><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, keep, idx, val, band); break;
+        case 1: euclid_value_kernel<1><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+        case 2: euclid_value_kernel<2><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+        case 4: euclid_value_kernel<4><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+        case 8: euclid_value_kernel<8><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
+        default: euclid_value_kernel<0><<<g, kThreads, 0, s>>>(ref, cand, n_cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, o.band); break;
     }
     FFR_LAUNCH_CHECK("euclid_values");
     return FFR_OK;
 }
 
 int launch_filter_fp32_self(const float* x, int64_t n, int64_t n_cand, int32_t dim, int metric, SelfArgs self, float thr,
-                            uint8_t* keep, int32_t* idx, float* val, float band_tol, int32_t* band_count, int64_t* band_rows,
-                            int64_t band_cap, cudaStream_t s) {
+                            const FilterOut& o, cudaStream_t s) {
     if (n_cand == 0) return FFR_OK;
     const float* cand = x + self.row0 * dim;
     const int sms = num_sms();
     const int64_t blocks_needed = (n_cand + (kThreads / 32) - 1) / (kThreads / 32);
     const dim3 g(static_cast<unsigned>(blocks_needed < static_cast<int64_t>(sms) * 8 ? blocks_needed : static_cast<int64_t>(sms) * 8));
-    const BandOut band{band_tol, band_count, band_rows, band_cap};
     const bool cosine = metric == FFR_METRIC_COSINE;
-    // the form K2s's gallery kernel takes for n_ref > 2 (k2s_dist_mode_gallery): what the tcgen05 Euclid value pass reproduces
-    const int mode = k2s_dist_mode_gallery(x, cand, dim);
+    // the self kernel reads its references from global memory, in the form of K2s's scan of more than two references (the
+    // form the tcgen05 Euclid value pass reproduces), whatever n is
+    const int mode = k2s_form(x, cand, INT64_MAX, dim);
 #define FFR_SELF_LAUNCH(NV)                                                                                                   \
-    if (cosine) filter_fp32_kernel<NV, true, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);  \
-    else        filter_fp32_kernel<NV, false, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self)
+    if (cosine) filter_fp32_kernel<NV, true, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, o.keep, o.idx, o.val, o.band, self);  \
+    else        filter_fp32_kernel<NV, false, 0, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, o.keep, o.idx, o.val, o.band, self)
     switch (mode) {
         case 1: FFR_SELF_LAUNCH(1); break;
         case 2: FFR_SELF_LAUNCH(2); break;
         case 4: FFR_SELF_LAUNCH(4); break;
         case 8: FFR_SELF_LAUNCH(8); break;
         default:
-            if (cosine) filter_fp32_generic_kernel<true, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);
-            else        filter_fp32_generic_kernel<false, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, keep, idx, val, band, self);
+            if (cosine) filter_fp32_generic_kernel<true, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, o.keep, o.idx, o.val, o.band, self);
+            else        filter_fp32_generic_kernel<false, true><<<g, kThreads, 0, s>>>(x, n, cand, n_cand, dim, thr, 0, o.keep, o.idx, o.val, o.band, self);
     }
 #undef FFR_SELF_LAUNCH
     FFR_LAUNCH_CHECK("filter_fp32_self");
@@ -508,7 +486,7 @@ int launch_filter_fp32_self(const float* x, int64_t n, int64_t n_cand, int32_t d
 
 int launch_ref_stats(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres, cudaStream_t s) {
     const size_t smem = (static_cast<size_t>(dim) + 8) * sizeof(float);
-    ref_stats_kernel<<<1, 256, smem, s>>>(ref_feat, n_ref, dim, mean, thres, k2s_dist_mode(ref_feat, dim));
+    ref_stats_kernel<<<1, 256, smem, s>>>(ref_feat, n_ref, dim, mean, thres, k2s_form(ref_feat, ref_feat, 1, dim));
     FFR_LAUNCH_CHECK("ref_stats");
     return FFR_OK;
 }

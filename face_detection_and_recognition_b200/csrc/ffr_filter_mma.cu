@@ -1502,13 +1502,11 @@ int a_stage_count(int32_t dim_pad) {
     return a_stage <= 32768 ? 3 : (a_stage <= 65536 ? 2 : 1);
 }
 
-struct BandArgs { float tol; int32_t* count; int64_t* rows; int64_t cap; };
-
 // cand32 != nullptr: the candidates' normalisation runs inside the kernel, which then WRITES cand16 (workspace) itself
 int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, const float* cand32, int32_t dim,
                            int64_t n_cand, int32_t dim_pad,
-                           float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
-                           RecheckLists lists, int no_recheck, BandArgs band, float* dbg_scores, bool after_k1,
+                           float thr, float delta, float thr_band, int64_t ref_index_base, const FilterOut& out,
+                           RecheckLists lists, int no_recheck, float* dbg_scores, bool after_k1,
                            const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
                            const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
     if (dim_pad % kBlockK != 0 || dim_pad < kBlockK || dim_pad > 512) {
@@ -1579,8 +1577,8 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     KParams p;
     p.n_ref = n_ref; p.n_ref_dev = n_ref_dev; p.ref_map = ref_map; p.n_cand = n_cand; p.kb_count = kb; p.a_stages = a_stages; p.b_stages = b_stages;
     p.thr = thr; p.delta = delta; p.thr_band = thr_band; p.ref_index_base = ref_index_base;
-    p.keep = keep; p.best_idx = idx; p.best_val = val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof;
-    p.band_tol = band.tol; p.band_count = no_recheck ? band.count : nullptr; p.band_rows = band.rows; p.band_cap = band.cap;
+    p.keep = out.keep; p.best_idx = out.idx; p.best_val = out.val; p.lists = lists; p.no_recheck = no_recheck; p.dbg_scores = dbg_scores; p.prof = prof;
+    p.band_tol = out.band.tol; p.band_count = no_recheck ? out.band.count : nullptr; p.band_rows = out.band.rows; p.band_cap = out.band.cap;
     p.ref_bias = euclid_bias; p.cand_scale = cand_scale; p.bias_max = bias_max;
     p.self_row0 = self.row0; p.self_mode = self.mode;
     p.cand32 = cand32; p.cand16 = cand16; p.dim = dim;
@@ -1686,14 +1684,13 @@ bool filter_mma_can_fuse(const float* cand32, int64_t n_ref, int64_t n_cand, int
 }
 
 int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const float* cand32, int32_t dim,
-                      int64_t n_cand, int32_t dim_pad,
-                      float thr, float delta, float thr_band, int64_t ref_index_base, uint8_t* keep, int32_t* idx, float* val,
-                      RecheckLists lists, int no_recheck, float band_tol, int32_t* band_count, int64_t* band_rows,
-                      int64_t band_cap, bool after_k1, const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
+                      int64_t n_cand, int32_t dim_pad, float thr, float delta, float thr_band, int64_t ref_index_base,
+                      const FilterOut& out, RecheckLists lists, int no_recheck, bool after_k1, const int32_t* ref_map,
+                      const int32_t* n_ref_dev, cudaStream_t s,
                       const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
     return launch_filter_mma_impl(ref16, n_ref, cand16, cand32, dim, n_cand, dim_pad, thr, delta, thr_band, ref_index_base,
-                                  keep, idx, val, lists, no_recheck, BandArgs{band_tol, band_count, band_rows, band_cap}, nullptr,
-                                  after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale, bias_max, self);
+                                  out, lists, no_recheck, nullptr, after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale,
+                                  bias_max, self);
 }
 
 // true when the fused schedule needs NO fp16 copy of the candidates in the workspace (stage32: the fp16 A tiles only ever
@@ -1712,11 +1709,9 @@ void get_last_k2_config(int out[8]) { for (int i = 0; i < 8; ++i) out[i] = g_las
 
 // test hook (not part of the ABI in include/ffr.h): additionally dumps the full score matrix
 int launch_filter_mma_debug(const __half* ref16, int64_t n_ref, const __half* cand16, int64_t n_cand, int32_t dim_pad,
-                            float thr, float delta, uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
-                            float* scores, cudaStream_t s) {
-    return launch_filter_mma_impl(ref16, n_ref, const_cast<__half*>(cand16), nullptr, dim_pad, n_cand, dim_pad, thr, delta, delta, 0, keep, idx,
-                                  val, lists, 0, BandArgs{0.f, nullptr, nullptr, 0}, scores, false, nullptr, nullptr, s,
-                                  nullptr, nullptr, nullptr, kNoSelf);
+                            float thr, float delta, const FilterOut& out, RecheckLists lists, float* scores, cudaStream_t s) {
+    return launch_filter_mma_impl(ref16, n_ref, const_cast<__half*>(cand16), nullptr, dim_pad, n_cand, dim_pad, thr, delta, delta, 0, out,
+                                  lists, 0, scores, false, nullptr, nullptr, s, nullptr, nullptr, nullptr, kNoSelf);
 }
 
 }  // namespace ffr

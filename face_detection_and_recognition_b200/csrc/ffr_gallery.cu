@@ -254,7 +254,7 @@ int launch_ref_stats_batched(const float* ref_feat, const int32_t* offsets, int3
     if (n_classes == 0) return FFR_OK;
     const size_t smem = (static_cast<size_t>(dim) + 8) * sizeof(float);
     ref_stats_batched_kernel<<<static_cast<unsigned>(n_classes), 256, smem, s>>>(ref_feat, offsets, dim, mean, thres,
-                                                                                    k2s_dist_mode(ref_feat, dim));
+                                                                                    k2s_form(ref_feat, ref_feat, 1, dim));
     FFR_LAUNCH_CHECK("ref_stats_batched");
     return FFR_OK;
 }

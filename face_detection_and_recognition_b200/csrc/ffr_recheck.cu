@@ -943,7 +943,8 @@ int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, co
     // K3's choice (launch_recheck) wherever K3 runs: its candidates are always 16-byte aligned there, these need not be
     const bool vec = (dim % 4 == 0) && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) &&
                      ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
-    const int emode = metric == FFR_METRIC_EUCLID ? k2s_dist_mode_gallery(ref, cand, dim) : -1;
+    // the whole gallery's form (more than two references over all ranks): the merge reproduces the one-GPU call's values
+    const int emode = metric == FFR_METRIC_EUCLID ? k2s_form(ref, cand, INT64_MAX, dim) : -1;
     int64_t grid = (n_cand + kWarps - 1) / kWarps;
     if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
     best_key_kernel<<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, ref_index_base, cand, n_cand, dim, best_idx,
@@ -952,22 +953,19 @@ int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, co
     return FFR_OK;
 }
 
-int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, uint8_t* keep, int32_t* best_idx,
-                     float* best_val, float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap, cudaStream_t s) {
+int launch_emit_keys(const unsigned long long* keys, int64_t n_cand, int metric, float thr, const FilterOut& o, cudaStream_t s) {
     if (n_cand == 0) return FFR_OK;
     int64_t grid = (n_cand + 255) / 256;
     if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
-    emit_keys_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(keys, n_cand, metric == FFR_METRIC_EUCLID, thr, keep, best_idx,
-                                                                best_val, band_tol, band_count, band_rows, band_cap);
+    emit_keys_kernel<<<static_cast<unsigned>(grid), 256, 0, s>>>(keys, n_cand, metric == FFR_METRIC_EUCLID, thr, o.keep, o.idx,
+                                                                o.val, o.band.tol, o.band.count, o.band.rows, o.band.cap);
     FFR_LAUNCH_CHECK("emit_keys");
     return FFR_OK;
 }
 
-int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim,
-                   const float* /*ref_norm*/, const float* /*cand_norm*/, float thr, int64_t ref_index_base,
-                   uint8_t* keep, int32_t* idx, float* val, RecheckLists lists,
-                   float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
-                   const int32_t* ref_map, const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode, SelfArgs self) {
+int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, float thr,
+                   int64_t ref_index_base, const FilterOut& o, RecheckLists lists, const int32_t* ref_map,
+                   const int32_t* n_unique_dev, cudaStream_t s, int euclid_mode, SelfArgs self) {
     if (n_cand == 0) return FFR_OK;
     const bool euclid = euclid_mode >= 0;
     static_assert(kFullGroup % kWarps == 0, "every warp parks kFullGroup / kWarps candidate rows of a full-rescan group");
@@ -1002,8 +1000,9 @@ int launch_recheck(const float* ref, int64_t n_ref, const float* cand, int64_t n
                              : (vec ? recheck_kernel<true, false, true> : recheck_kernel<false, false, true>))
                    : (euclid ? (vec ? recheck_kernel<true, true> : recheck_kernel<false, true>)
                              : (vec ? recheck_kernel<true, false> : recheck_kernel<false, false>));
-    fn<<<g2, kThreads, vec ? smem_full : smem, s>>>(ref, n_ref, cand, dim, thr, ref_index_base, keep, idx, val, lists, band_tol,
-                                                    band_count, band_rows, band_cap, ref_map, n_unique_dev, euclid_mode, self);
+    fn<<<g2, kThreads, vec ? smem_full : smem, s>>>(ref, n_ref, cand, dim, thr, ref_index_base, o.keep, o.idx, o.val, lists,
+                                                    o.band.tol, o.band.count, o.band.rows, o.band.cap, ref_map, n_unique_dev,
+                                                    euclid_mode, self);
     FFR_LAUNCH_CHECK("recheck");
     return FFR_OK;
 }

@@ -88,6 +88,25 @@ def l2norm_rows(x: torch.Tensor, want_f16: bool = False, want_f32: bool = True, 
     return out
 
 
+def _outputs(out, n: int, dev: torch.device, band_tol: Optional[float]):
+    """(keep, idx, val, band_count, band_rows): the caller's ``out`` or new [n] tensors, and the band's count and row buffers
+    (None without ``band_tol``)."""
+    if out is None:
+        out = (torch.empty((n,), dtype=torch.uint8, device=dev), torch.empty((n,), dtype=torch.int32, device=dev),
+               torch.empty((n,), dtype=torch.float32, device=dev))
+    keep, idx, val = out
+    band_count = band_rows = None
+    if band_tol is not None:
+        band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
+        band_rows = torch.empty((max(n, 1),), dtype=torch.int64, device=dev)
+    return keep, idx, val, band_count, band_rows
+
+
+def _band(band_count: torch.Tensor, band_rows: torch.Tensor, n: int) -> torch.Tensor:
+    """The band's rows, sorted (the kernels append them in any order; a count above n is capped)."""
+    return torch.sort(band_rows[:min(int(band_count.item()), n)]).values
+
+
 @dataclass
 class FilterResult:
     keep: torch.Tensor                       # uint8 [M]   1 = similar ("clean"), 0 = discard ("unclean")
@@ -130,18 +149,8 @@ def face_filter(ref: torch.Tensor, cand: torch.Tensor, thr: float, metric="cosin
         raise ValueError("ref and cand must be on the same device")
     n_ref, n_cand = ref.shape[0], cand.shape[0]
     dev = cand.device
-    if out is None:
-        keep = torch.empty((n_cand,), dtype=torch.uint8, device=dev)
-        idx = torch.empty((n_cand,), dtype=torch.int32, device=dev)
-        val = torch.empty((n_cand,), dtype=torch.float32, device=dev)
-    else:
-        keep, idx, val = out
-    ws_bytes = int(lib.ffr_filter_workspace_bytes(n_ref, n_cand, dim, dtype, m))
-    ws = _workspace(dev, ws_bytes)
-    band_count = band_rows = None
-    if band_tol is not None:
-        band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
-        band_rows = torch.empty((max(n_cand, 1),), dtype=torch.int64, device=dev)
+    keep, idx, val, band_count, band_rows = _outputs(out, n_cand, dev, band_tol)
+    ws = _workspace(dev, int(lib.ffr_filter_workspace_bytes(n_ref, n_cand, dim, dtype, m)))
     with torch.cuda.device(dev):
         check(lib.ffr_filter_ex(ref.data_ptr(), n_ref, cand.data_ptr() if n_cand else None, n_cand, dim, dtype,
                                 None, None, m, float(thr), int(ref_index_base),
@@ -152,8 +161,7 @@ def face_filter(ref: torch.Tensor, cand: torch.Tensor, thr: float, metric="cosin
                                 ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
         res = FilterResult(keep, idx, val)
         if band_tol is not None:
-            n = int(band_count.item())
-            res.band_rows = torch.sort(band_rows[:min(n, n_cand)]).values
+            res.band_rows = _band(band_count, band_rows, n_cand)
         if want_stats:
             res.stats = _stats(lib, ws, dev)
     return res
@@ -197,17 +205,8 @@ def self_filter(x: torch.Tensor, thr: float, metric="cosine", mode="others", row
     begin, end = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
     n_rows = max(end - begin, 0)
     dev = x.device
-    if out is None:
-        keep = torch.empty((n_rows,), dtype=torch.uint8, device=dev)
-        idx = torch.empty((n_rows,), dtype=torch.int32, device=dev)
-        val = torch.empty((n_rows,), dtype=torch.float32, device=dev)
-    else:
-        keep, idx, val = out
+    keep, idx, val, band_count, band_rows = _outputs(out, n_rows, dev, band_tol)
     ws = _workspace(dev, int(lib.ffr_filter_self_workspace_bytes(n, n_rows, dim, m)))
-    band_count = band_rows = None
-    if band_tol is not None:
-        band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
-        band_rows = torch.empty((max(n_rows, 1),), dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
         check(lib.ffr_filter_self(x.data_ptr(), n, begin, end - begin, dim, m, md, float(thr),
                                   keep.data_ptr() if n_rows else None, idx.data_ptr() if n_rows else None,
@@ -217,7 +216,7 @@ def self_filter(x: torch.Tensor, thr: float, metric="cosine", mode="others", row
                                   ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
         res = FilterResult(keep, idx, val)
         if band_tol is not None:
-            res.band_rows = torch.sort(band_rows[:min(int(band_count.item()), n_rows)]).values
+            res.band_rows = _band(band_count, band_rows, n_rows)
         if want_stats:
             res.stats = _stats(lib, ws, dev)
     return res
@@ -478,16 +477,9 @@ class ResultGather:
             raise ValueError(f"best_idx must be an int32 tensor of shape ({n_cand},) on {dev}, got "
                              f"{getattr(best_idx, 'dtype', type(best_idx))} {tuple(getattr(best_idx, 'shape', ()))} "
                              f"on {getattr(best_idx, 'device', None)}")
-        if out is None:
-            out = (torch.empty((n_cand,), dtype=torch.uint8, device=dev), torch.empty((n_cand,), dtype=torch.int32, device=dev),
-                   torch.empty((n_cand,), dtype=torch.float32, device=dev))
-        keep, idx, val = out
+        keep, idx, val, band_count, band_rows = _outputs(out, n_cand, dev, band_tol)
         if idx.data_ptr() != best_idx.data_ptr():
             idx.copy_(best_idx)
-        band_count = band_rows = None
-        if band_tol is not None:
-            band_count = torch.zeros((1,), dtype=torch.int32, device=dev)
-            band_rows = torch.empty((max(n_cand, 1),), dtype=torch.int64, device=dev)
         ws = _workspace(dev, int(self._lib.ffr_allreduce_best_workspace_bytes(n_cand)))
         with torch.cuda.device(dev):
             check(self._lib.ffr_allreduce_best(self._h, ref_local.data_ptr() if n_ref else None, n_ref, int(ref_index_base),
@@ -499,7 +491,7 @@ class ResultGather:
                                                ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
         res = FilterResult(keep, idx, val)
         if band_tol is not None:
-            res.band_rows = torch.sort(band_rows[:min(int(band_count.item()), n_cand)]).values
+            res.band_rows = _band(band_count, band_rows, n_cand)
         return res
 
     def all_gather(self, keep_local: torch.Tensor, idx_local: torch.Tensor):
