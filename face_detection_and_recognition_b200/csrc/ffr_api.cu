@@ -23,8 +23,8 @@ std::atomic<int64_t> g_launches{0};
 std::atomic<float> g_delta{4e-4f};       // recheck window in cosine units, see DESIGN.md §4 (fp16 operand rounding)
 std::atomic<const Knobs*> g_knobs{nullptr};
 std::mutex g_knobs_mu;
-struct LastCall { const void* ws; int path; int launches; };
-thread_local LastCall g_last = {nullptr, 0, 0};
+struct LastCall { const void* ws; int path; int launches; bool pairs; };
+thread_local LastCall g_last = {nullptr, 0, 0, false};
 // profiling hook: CUDA events recorded on the launch stream right before / after the tcgen05 kernel
 thread_local cudaEvent_t g_ev_k2_begin = nullptr, g_ev_k2_end = nullptr;
 }  // namespace
@@ -108,6 +108,8 @@ struct Ws {
     RecheckLists lists;                                   // (header included)
     void* dedup;                                          // scratch of the duplicate-reference fold
     float *e_bias, *e_bias_c, *e_nsq, *e_scal, *e_cscale;   // Euclid on the tensor cores
+    uint2* pair_raw;                                      // match lists: K2's raw pair list ...
+    int32_t* exact_rows;                                  // ... and its exact-row list (Euclid)
     size_t total;
 };
 
@@ -131,8 +133,10 @@ bool mma_eligible(int64_t n_ref, int32_t dim, int metric, int flags) {
 // euclid: the tcgen05 Euclid path's extra buffers -- the reference bias (and its deduplicated copy), the references' squared
 // norms, two scalars, and the candidates' 1 / |c| (n_ref == 0: the caller prepared the references)
 // base: the workspace to carve (nullptr: only the size is wanted)
+// pair_cap >= 0: a match-list call -- no re-check lists and no fold; the raw pair list (pair_cap entries) and, Euclid, the
+// exact-row list follow the Euclid buffers
 Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup, bool euclid = false,
-             void* base = nullptr) {
+             void* base = nullptr, int64_t pair_cap = -1) {
     Ws L{};
     size_t off = 0;
     const auto take = [&](size_t bytes) {
@@ -147,6 +151,7 @@ Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bo
         L.ref16 = static_cast<__half*>(take(f32 ? nr * ld * 2 : 0));
         L.cand16 = static_cast<__half*>(take(f32 && need_c16 ? nc * ld * 2 : 0));
         L.lists.hdr = L.hdr;
+        if (pair_cap < 0) {
         L.lists.recs = static_cast<RecheckRec*>(take(nc * sizeof(RecheckRec)));
         L.lists.rec_cap = n_cand;
         L.lists.full_rows = static_cast<int32_t*>(take(nc * sizeof(int32_t)));
@@ -154,6 +159,7 @@ Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bo
         L.lists.full_ctr = static_cast<int32_t*>(take((nc / kFullGroup + 1) * sizeof(int32_t)));
         L.lists.full_cap = n_cand;
         L.dedup = take(dedup && f32 ? dedup_workspace_bytes(n_ref, static_cast<int32_t>(ld)) : 0);
+        }
         if (euclid) {
             const size_t nb = n_ref > 0 ? static_cast<size_t>(euclid_bias_len(n_ref)) * 4 : 0;
             L.e_bias = static_cast<float*>(take(nb));
@@ -161,6 +167,10 @@ Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bo
             L.e_nsq = static_cast<float*>(take(nr * 4));
             L.e_scal = static_cast<float*>(take(256));
             L.e_cscale = static_cast<float*>(take(nc * 4));
+        }
+        if (pair_cap >= 0) {
+            L.pair_raw = static_cast<uint2*>(take(static_cast<size_t>(pair_cap) * sizeof(uint2)));
+            L.exact_rows = static_cast<int32_t*>(take(euclid ? nc * sizeof(int32_t) : 0));
         }
     }
     L.total = off;
@@ -354,6 +364,32 @@ bool self_mma_eligible(int64_t n, int32_t dim, int flags) {
     return !(flags & FFR_FLAG_FORCE_FP32) && dim <= 512 && n > 8 && euclid_mma_available();
 }
 
+// K1 schedule without a fold (self mode, match lists): Euclid -- E1/E2 turn the references into the B operand and its bias, K1 over
+// the candidates writes the normalised A rows and 1 / |c|; cosine -- K1 over the references and candidates in one launch, or
+// (self_row0 >= 0: the candidates are rows [self_row0, ...) of ref) over ref ONCE, the A operand being the candidates' slice of
+// that fp16 copy.  The K1 launch zeroes the header.
+int prep_k1(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int64_t self_row0, int32_t dim, bool euclid,
+            const Ws& L, K2In& in, cudaStream_t s) {
+    const int32_t ld = ffr_padded_dim(dim), hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
+    in.after_k1 = true;
+    if (euclid) {
+        const int rc = prepare_euclid_refs(ref, n_ref, dim, L, in.ref, s);
+        if (rc != FFR_OK) return rc;
+        in.cand16 = L.cand16;
+        in.cand_scale = L.e_cscale;
+        in.launches = 3;
+        return launch_l2norm_pair(cand, n_cand, in.cand16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s, in.cand_scale);
+    }
+    in.ref.rows = L.ref16;
+    in.launches = 1;
+    if (self_row0 >= 0) {
+        in.cand16 = L.ref16 + self_row0 * ld;
+        return launch_l2norm_pair(ref, n_ref, L.ref16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s);
+    }
+    in.cand16 = L.cand16;
+    return launch_l2norm_pair(cand, n_cand, in.cand16, ref, n_ref, L.ref16, dim, ld, L.hdr, hdr_words, s);
+}
+
 Ws self_ws_layout(int64_t n, int64_t n_rows, int32_t dim, int metric, bool mma, void* base = nullptr) {
     const bool euclid = metric == FFR_METRIC_EUCLID;
     return ws_layout(n, n_rows, dim, FFR_DTYPE_F32, mma, /*need_c16=*/euclid, /*dedup=*/false, mma && euclid, base);
@@ -367,27 +403,68 @@ int self_core(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int3
                   (long long)n, dim);
         return FFR_ERR_UNSUPPORTED;
     }
-    const bool euclid = metric == FFR_METRIC_EUCLID;
     const Ws L = self_ws_layout(n, n_rows, dim, metric, mma, workspace);
     const float* cand = x + row_begin * dim;
     return run_filter(x, n, cand, n_rows, dim, FFR_DTYPE_F32, metric, thr, 0, out, flags, SelfArgs{row_begin, mode}, mma, L,
                       workspace, ws_bytes, "", s, [&](K2In& in) {
-        const int32_t ld = ffr_padded_dim(dim), hdr_words = static_cast<int32_t>(sizeof(WsHeader) / 4);
-        int rc;
-        in.after_k1 = true;
-        if (euclid) {
-            rc = prepare_euclid_refs(x, n, dim, L, in.ref, s);
-            if (rc != FFR_OK) return rc;
-            in.cand16 = L.cand16;
-            in.cand_scale = L.e_cscale;
-            in.launches = 3;
-            return launch_l2norm_pair(cand, n_rows, in.cand16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s, in.cand_scale);
-        }
-        in.ref.rows = L.ref16;
-        in.cand16 = L.ref16 + row_begin * ld;
-        in.launches = 1;
-        return launch_l2norm_pair(x, n, L.ref16, nullptr, 0, nullptr, dim, ld, L.hdr, hdr_words, s);
+        return prep_k1(x, n, cand, n_rows, row_begin, dim, metric == FFR_METRIC_EUCLID, L, in, s);
     });
+}
+
+// ---- match lists (ffr_match_pairs*; DESIGN.md section 4, "Match lists") --------------------------------------------------------
+// The tensor-core path takes self mode's rule (self_mma_eligible: n_ref > 8, dim <= 512, cta_group::2, not FFR_FLAG_FORCE_FP32) for
+// both metrics, gallery and self.
+
+// self: the candidates are rows of the references (cosine reads them from the references' fp16 copy)
+Ws pairs_ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int metric, bool self, bool mma, int64_t pair_cap,
+                   void* base = nullptr) {
+    const bool euclid = metric == FFR_METRIC_EUCLID;
+    return ws_layout(n_ref, n_cand, dim, FFR_DTYPE_F32, mma, /*need_c16=*/!self || euclid, /*dedup=*/false, mma && euclid, base,
+                     pair_cap);
+}
+
+int check_pairs_out(int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap, int64_t* pair_count, int flags) {
+    if (pair_count == nullptr || pair_cap < 0 || (pair_cap > 0 && (pair_cand == nullptr || pair_ref == nullptr || pair_val == nullptr))) {
+        set_error("pairs: need pair_count, pair_cap >= 0 and, for pair_cap > 0, the three output arrays");
+        return FFR_ERR_INVALID;
+    }
+    if (flags & FFR_FLAG_NO_RECHECK) {
+        set_error("FFR_FLAG_NO_RECHECK is not supported by the match lists (the fp32 value decides every pair)");
+        return FFR_ERR_UNSUPPORTED;
+    }
+    return FFR_OK;
+}
+
+// One match-list call from the workspace checks on: the exact kernel, or the K1 preparation (which zeroes the header), K2's pairs
+// form and the finishing pass.  self.mode >= 0: cand is rows [self.row0, ...) of ref.
+int run_pairs(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
+              int64_t ref_index_base, const PairOut& out, SelfArgs self, bool mma, const Ws& L, void* workspace, size_t ws_bytes,
+              cudaStream_t s) {
+    if (workspace == nullptr || ws_bytes < L.total) {
+        set_error("workspace too small: need %zu bytes, got %zu", L.total, workspace ? ws_bytes : (size_t)0);
+        return FFR_ERR_WORKSPACE;
+    }
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) { set_error("workspace must be 256-byte aligned"); return FFR_ERR_INVALID; }
+    g_last = {workspace, mma ? 1 : 0, 0, true};
+    if (!mma || n_cand == 0) {
+        FFR_CUDA_TRY(cudaMemsetAsync(L.hdr, 0, sizeof(WsHeader), s));
+        FFR_CUDA_TRY(cudaMemsetAsync(out.count, 0, sizeof(int64_t), s));
+        if (n_cand == 0) return FFR_OK;
+        g_last.launches = 1;
+        return launch_pairs_exact(ref, n_ref, cand, n_cand, dim, metric, thr, ref_index_base, self, out, s);
+    }
+    K2In in{};
+    int rc = prep_k1(ref, n_ref, cand, n_cand, self.mode >= 0 ? self.row0 : -1, dim, metric == FFR_METRIC_EUCLID, L, in, s);
+    if (rc != FFR_OK) return rc;
+    g_last.launches = in.launches + 2;
+    const PairRaw raw{L.pair_raw, out.cap, L.exact_rows, reinterpret_cast<const uint32_t*>(L.e_scal)};
+    if (g_ev_k2_begin != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_begin, s));
+    rc = launch_filter_mma(in.ref.rows, n_ref, in.cand16, nullptr, dim, n_cand, ffr_padded_dim(dim), thr, recheck_delta(), 0.f,
+                           0, FilterOut{}, L.lists, 0, in.after_k1, nullptr, nullptr, s, in.ref.bias, in.cand_scale, in.ref.bias_max,
+                           self, &raw);
+    if (rc != FFR_OK) return rc;
+    if (g_ev_k2_end != nullptr) FFR_CUDA_TRY(cudaEventRecord(g_ev_k2_end, s));
+    return launch_pairs_finish(ref, n_ref, cand, dim, metric, thr, ref_index_base, self, raw, L.hdr, out, s);
 }
 
 }  // namespace
@@ -510,7 +587,73 @@ int ffr_filter_stats(const void* workspace, int64_t out[8], ffr_stream_t stream)
     out[4] = h.part_count;
     out[5] = h.refs_scanned;
     out[6] = out[7] = 0;
+    if (g_last.ws == workspace && g_last.pairs) {        // a match-list call: the raw pairs K2 listed
+        out[0] = static_cast<int64_t>(h.raw_count);
+        out[1] = out[4] = out[5] = 0;
+    }
     return FFR_OK;
+}
+
+size_t ffr_match_pairs_workspace_bytes(int64_t n_ref, int64_t n_cand, int32_t dim, int metric, int64_t pair_cap) {
+    if (n_ref <= 0 || n_cand < 0 || dim <= 0 || pair_cap < 0) return 0;
+    // sized for the tcgen05 path whenever it could run
+    return pairs_ws_layout(n_ref, n_cand, dim, metric, false, dim <= 512 && n_ref > 8, pair_cap).total;
+}
+
+int ffr_match_pairs(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
+                    int64_t ref_index_base, int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap,
+                    int64_t* pair_count, int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream) {
+    if (n_ref <= 0) { set_error("n_ref must be > 0 (got %lld)", (long long)n_ref); return FFR_ERR_INVALID; }
+    if (n_cand < 0 || n_cand > static_cast<int64_t>(INT32_MAX)) { set_error("n_cand must be in [0, 2^31) (got %lld)", (long long)n_cand); return FFR_ERR_INVALID; }
+    if (dim <= 0) { set_error("dim must be > 0 (got %d)", dim); return FFR_ERR_INVALID; }
+    if (ref == nullptr || (n_cand > 0 && cand == nullptr)) { set_error("null pointer argument"); return FFR_ERR_INVALID; }
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) { set_error("unknown metric %d", metric); return FFR_ERR_INVALID; }
+    if (ref_index_base < 0 || ref_index_base + n_ref > static_cast<int64_t>(INT32_MAX)) {
+        set_error("pairs: reference indices [%lld, %lld) do not fit int32", (long long)ref_index_base, (long long)(ref_index_base + n_ref));
+        return FFR_ERR_INVALID;
+    }
+    int rc = check_pairs_out(pair_cand, pair_ref, pair_val, pair_cap, pair_count, flags);
+    if (rc != FFR_OK) return rc;
+    if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
+    const bool mma = self_mma_eligible(n_ref, dim, flags);
+    if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
+        set_error("FFR_FLAG_FORCE_MMA: the match lists' tcgen05 path needs n_ref > 8, dim <= 512 and cta_group::2 (n_ref=%lld dim=%d)",
+                  (long long)n_ref, dim);
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const Ws L = pairs_ws_layout(n_ref, n_cand, dim, metric, false, mma, pair_cap, workspace);
+    return run_pairs(ref, n_ref, cand, n_cand, dim, metric, thr, ref_index_base, PairOut{pair_cand, pair_ref, pair_val, pair_cap, pair_count},
+                     kNoSelf, mma, L, workspace, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+
+size_t ffr_match_pairs_self_workspace_bytes(int64_t n, int64_t n_rows, int32_t dim, int metric, int64_t pair_cap) {
+    if (n <= 0 || n_rows < 0 || dim <= 0 || pair_cap < 0) return 0;
+    return pairs_ws_layout(n, n_rows, dim, metric, true, dim <= 512 && n > 8, pair_cap).total;
+}
+
+int ffr_match_pairs_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, float thr,
+                         int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap, int64_t* pair_count,
+                         int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream) {
+    if (n <= 0 || n > static_cast<int64_t>(INT32_MAX)) { set_error("n must be in (0, 2^31) (got %lld)", (long long)n); return FFR_ERR_INVALID; }
+    if (dim <= 0) { set_error("dim must be > 0 (got %d)", dim); return FFR_ERR_INVALID; }
+    if (row_begin < 0 || n_rows < 0 || row_begin > n - n_rows) {
+        set_error("row range [%lld, %lld) is not inside [0, %lld)", (long long)row_begin, (long long)(row_begin + n_rows), (long long)n);
+        return FFR_ERR_INVALID;
+    }
+    if (x == nullptr) { set_error("null pointer argument"); return FFR_ERR_INVALID; }
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) { set_error("unknown metric %d", metric); return FFR_ERR_INVALID; }
+    int rc = check_pairs_out(pair_cand, pair_ref, pair_val, pair_cap, pair_count, flags);
+    if (rc != FFR_OK) return rc;
+    if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
+    const bool mma = self_mma_eligible(n, dim, flags);
+    if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
+        set_error("FFR_FLAG_FORCE_MMA: the self-mode tcgen05 path needs n > 8, dim <= 512 and cta_group::2 (n=%lld dim=%d)",
+                  (long long)n, dim);
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const Ws L = pairs_ws_layout(n, n_rows, dim, metric, true, mma, pair_cap, workspace);
+    return run_pairs(x, n, x + row_begin * dim, n_rows, dim, metric, thr, 0, PairOut{pair_cand, pair_ref, pair_val, pair_cap, pair_count},
+                     SelfArgs{row_begin, FFR_SELF_EARLIER}, mma, L, workspace, ws_bytes, static_cast<cudaStream_t>(stream));
 }
 
 int ffr_ref_mean_and_thres(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres,

@@ -75,7 +75,30 @@ struct WsHeader {
     int32_t launches;
     int32_t part_count;      // rows whose hidden columns all lie in one 128-reference part (records at the END of recs, growing down)
     int32_t refs_scanned;    // reference rows K2 actually scanned (< n_ref when exact duplicates were folded)
-    int32_t pad[58];
+    // match lists (ffr_match_pairs*): K2's raw pair list and exact-row list, the finishing pass's counters
+    int32_t exact_count;     // Euclid candidates whose scores are unusable (1 / |c| not finite): scanned in fp32
+    int32_t pairs_blocks;    // finishing-pass blocks done (the last one writes the caller's count)
+    unsigned long long raw_count;      // pairs K2 listed (keeps counting past the raw list's capacity)
+    unsigned long long acc_count;      // pairs the finishing pass accepted (slots of the caller's list)
+    unsigned long long acc_exact;      // ... of which from the exact-row list
+    int32_t pad[50];
+};
+static_assert(sizeof(WsHeader) == 256, "the workspace header is 256 bytes");
+
+// A match-list call's outputs (ffr_match_pairs*): accepted pairs go to [0, cap), *count is written by the last kernel
+struct PairOut {
+    int32_t* cand;
+    int32_t* ref;
+    float* val;
+    int64_t cap;
+    int64_t* count;
+};
+// K2's pairs form: raw (candidate row, reference column) entries, exact rows (Euclid candidates with unusable scores)
+struct PairRaw {
+    uint2* raw;
+    int64_t cap;
+    int32_t* exact_rows;
+    const uint32_t* e_max_bits;   // Euclid: E1's largest squared reference norm (bits), from which K2 derives E2's 2^-f
 };
 
 // Self mode (ffr_filter_self): the candidates are rows [row0, row0 + n_cand) of the reference matrix itself, and candidate row g
@@ -153,6 +176,14 @@ __device__ __forceinline__ float k2s_euclid_dist(const float* __restrict__ c, co
         for (int o = L / 2; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
     }
     return __fsqrt_rn(a);
+}
+
+// E2's power of two (ffr_l2norm.cu): 2^-f with f the smallest integer such that 2^(2f) > mx = the largest squared reference norm
+__device__ __forceinline__ float euclid_ref_scale(float mx) {
+    int e = 0;
+    if (mx > 0.f && mx <= 3.4e38f) frexpf(mx, &e);                     // mx < 2^e
+    const int f = (e + 1) >> 1;                                         // |r| < 2^(e/2) <= 2^f
+    return ldexpf(1.0f, -f);
 }
 
 __device__ __forceinline__ float4 ldg_stream_f4(const float4* p) {
@@ -369,7 +400,15 @@ int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const 
                       const FilterOut& out, RecheckLists lists, int no_recheck, bool after_k1, const int32_t* ref_map,
                       const int32_t* n_ref_dev, cudaStream_t s,
                       const float* euclid_bias = nullptr, const float* cand_scale = nullptr, const float* bias_max = nullptr,
-                      SelfArgs self = kNoSelf);
+                      SelfArgs self = kNoSelf, const PairRaw* pairs = nullptr);
+// Match lists (ffr_recheck.cu).  Finishing pass behind K2's pairs form: the fp32 value of every raw entry (and of every exact row
+// against every reference), accepted pairs appended to out, *out.count written by the last block.  self.mode >= 0: cand is rows
+// [self.row0, ...) of ref (references i < g only).
+int launch_pairs_finish(const float* ref, int64_t n_ref, const float* cand, int32_t dim, int metric, float thr, int64_t ref_index_base,
+                        SelfArgs self, const PairRaw& raw, WsHeader* hdr, const PairOut& out, cudaStream_t s);
+// The exact path: one warp per candidate row over every reference, the same value arithmetic; *out.count must be zero before
+int launch_pairs_exact(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
+                       int64_t ref_index_base, SelfArgs self, const PairOut& out, cudaStream_t s);
 // exact-duplicate reference rows folded before K2 (ffr_dedup.cu)
 bool dedup_wanted(int64_t n_ref, int64_t n_cand);
 size_t dedup_workspace_bytes(int64_t n_ref, int32_t ld);

@@ -462,6 +462,8 @@ struct KParams {
     // kSelf: the candidates are rows [self_row0, self_row0 + n_cand) of the reference matrix (DESIGN.md section 4, "Self mode")
     int64_t self_row0;
     int self_mode;                 // FFR_SELF_OTHERS | FFR_SELF_EARLIER
+    // kPairs: the match lists' raw pair list and exact-row list (DESIGN.md section 4, "Match lists")
+    PairRaw pair;
 };
 
 // End of a candidate tile, once per row (the two column halves merged): classify_row writes keep / index / score and decides
@@ -588,6 +590,39 @@ __device__ __forceinline__ void append_rows(const KParams& p, const RowOut (&o)[
     }
 }
 
+// kPairs: append this thread's columns with score >= lo as (candidate row, reference column) to the raw list, warp-aggregated:
+// one 64-bit atomic per warp (the counter keeps counting past the capacity; entries are written below it only).  A lane's
+// columns go out together, so runs of entries share a candidate row.  The whole warp calls it.
+template <int kC>
+__device__ __forceinline__ void append_pairs(const KParams& p, const float (&v)[kC][32], float lo, int64_t row, int32_t base0,
+                                             int lane) {
+    uint32_t mk[kC];
+    int n = 0;
+#pragma unroll
+    for (int cc = 0; cc < kC; ++cc) {
+        mk[cc] = 0;
+#pragma unroll
+        for (int j = 0; j < 32; ++j) mk[cc] |= (v[cc][j] >= lo) ? (1u << j) : 0u;
+        n += __popc(mk[cc]);
+    }
+    int incl = n;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += t;
+    }
+    unsigned long long base = 0;
+    if (lane == 31 && incl > 0) base = atomicAdd(&p.lists.hdr->raw_count, static_cast<unsigned long long>(incl));
+    base = __shfl_sync(0xffffffffu, base, 31);
+    unsigned long long slot = base + static_cast<unsigned long long>(incl - n);
+    const unsigned long long cap = static_cast<unsigned long long>(p.pair.cap);
+#pragma unroll
+    for (int cc = 0; cc < kC; ++cc) {
+        for (uint32_t b = mk[cc]; b != 0u; b &= b - 1u, ++slot)
+            if (slot < cap) p.pair.raw[slot] = make_uint2(static_cast<uint32_t>(row), static_cast<uint32_t>(base0 + cc * 32 + __ffs(b) - 1));
+    }
+}
+
 // Self mode, FFR_SELF_EARLIER: candidate tile t only needs the reference tiles up to the last one with a column below its last
 // row.  The TMA producer, the MMA thread and the epilogue derive the same range from the tile index.  (Candidate tiles stay
 // dealt round-robin: with per-tile work growing linearly, a reversed order gives the busiest CTA pair the same sum -- the
@@ -614,7 +649,11 @@ __device__ __forceinline__ int32_t self_rt_end(const KParams& p, int64_t ct, int
 // column the row may not match -- its own (FFR_SELF_OTHERS) or any at or after it (FFR_SELF_EARLIER) -- runs the masked copy of
 // the epilogue body; FFR_SELF_EARLIER stops every role at the last reference tile with a column below the candidate tile's last
 // row.
-template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr, bool kEuclid = false, bool kSelf = false>
+// kPairs: the match lists' form (ffr_match_pairs*; K1 schedule, cta_group::2, production build): the same loads, bias, masks
+// and max trees, then ONE branch on the part maximum against the row's floor lo_row; inside it every column at or above the
+// floor goes to the raw pair list.  No running top-4, no end-of-tile merge, no K3 lists: the finishing pass decides in fp32.
+template <int kCG, int kNormMode, int kExact, int kAlways, bool kInstr, bool kEuclid = false, bool kSelf = false,
+          bool kPairs = false>
 __global__ void __launch_bounds__(64 + 32 * 8 + (kNormMode ? 64 : 0), 1)   // 10 warps are allocated as 12: <= 168 registers
 filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_constant__ CUtensorMap tmap_ref,
                   const __grid_constant__ CUtensorMap tmap_cand32, const KParams p) {
@@ -623,6 +662,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
     // kInstr: the instrumented build (in-kernel cycle counters, score dump).  The production
     // instantiation contains none of it: the counters alone were half a dozen spilled 64-bit values per role.
     static_assert(!kSelf || (kCG == 2 && kNormMode == 0 && !kInstr), "self mode runs on the K1 schedule, cta_group::2, production build");
+    static_assert(!kPairs || (kCG == 2 && kNormMode == 0 && !kInstr), "the pairs form runs on the K1 schedule, cta_group::2, production build");
     constexpr bool kNorm = kNormMode != 0;
     constexpr bool st32 = kNormMode >= 2;
     // stage32 comes in two forms: kNormMode 2 hands the end-of-tile work (merge of the column halves, classification, K3's
@@ -1164,6 +1204,25 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 // -- s_row not finite -- gets a NaN window here and goes to the full fp32 rescan in the tail.)
                 delta_row = fmaf(__ldg(p.bias_max) * s_row, 4.76837158e-7f, p.delta);
             }
+            // kPairs: the score floor of this row's pairs (DESIGN.md section 4, "Match lists"); +inf lists nothing
+            float lo_row = INFINITY;
+            if constexpr (kPairs) {
+                if (first_tile) pdl_wait();                     // the counters appended to below are zeroed by K1
+                if constexpr (kEuclid) {
+                    // |c - r| <= thr  <=>  (r.c - |r|^2 / 2) 2^-f / |c| >= (|c| - thr^2 / |c|) 2^-f / 2; below that floor by the score's
+                    // window delta_row, and by 2^-18 of the floor's two terms for the roundings of the floor and of the fp32 distance
+                    const float sc = euclid_ref_scale(__uint_as_float(__ldg(p.pair.e_max_bits)));
+                    const float cn = 1.0f / s_row, t2 = p.thr * p.thr * s_row;
+                    lo_row = 0.5f * sc * (cn - t2) - delta_row - sc * (cn + t2) * 3.81469727e-6f;
+                    if (!(fabsf(s_row) <= 3.4e38f)) {          // zero or non-finite row: unusable scores, scanned in fp32 instead
+                        if (row < p.n_cand && h == 0) p.pair.exact_rows[atomicAdd(&p.lists.hdr->exact_count, 1)] = static_cast<int32_t>(row);
+                        lo_row = INFINITY;
+                    }
+                } else {
+                    lo_row = p.thr - p.delta;
+                }
+                if (row >= p.n_cand) lo_row = INFINITY;
+            }
             // One reference tile.  The loop over FULL tiles and the one partial last tile are separate copies of this body: the
             // masking of columns >= n_ref is 260 instructions that the hot loop would otherwise carry (and jump over) on every
             // tile -- the body is what has to stream through the instruction cache.
@@ -1236,7 +1295,11 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                     // short reference sets: some lane of the warp sets a record on nearly every tile, so the update runs
                     // unconditionally and branch-free; long ones: behind one branch on the part maximum.  (Round-1c's
                     // per-chunk update paths are gone from this loop: dead code in it costs wall clock.)
-                    if (grid_updates || m >= gate) update_grid<kChunksPerPart>(v, sx, cm, m, base0, kEuclid ? delta_row : p.delta, grid_exact, t, gate, hid);
+                    if constexpr (kPairs) {
+                        if (__any_sync(0xffffffffu, m >= lo_row)) append_pairs<kChunksPerPart>(p, v, lo_row, row, base0, lane);
+                    } else {
+                        if (grid_updates || m >= gate) update_grid<kChunksPerPart>(v, sx, cm, m, base0, kEuclid ? delta_row : p.delta, grid_exact, t, gate, hid);
+                    }
                     if (pr) c_hot += static_cast<unsigned long long>(clock64() - tp0);
                 } else {
                     // ---- general loop, one chunk at a time: the score dump only
@@ -1290,6 +1353,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
             // warps of ONE lane quadrant (ids 1+q / 5+q, alternating with the tile parity so that an early arrive for tile
             // n + 2 cannot complete tile n's barrier); with CTA-wide barriers every quadrant waited for the slowest warp.
             const long long t_tail0 = pr ? clock64() : 0;
+            if constexpr (!kPairs) {
             // ... except for the CTA's LAST candidate tile: nothing is left to overlap its tail with, and four merger warps (32 rows
             // each) finish it in half the time the two helper warps (64 rows each) need -- the kernel's drain.
             const bool inline_last = kOffload && tile + tile_stride >= n_tiles;
@@ -1383,6 +1447,7 @@ filter_mma_kernel(const __grid_constant__ CUtensorMap tmap_cand, const __grid_co
                 append_rows<1>(p, ro, lane);
             }
             }   // !st32
+            }   // !kPairs
             first_tile = false;
             ++c_it;
             if (pr) c_tail += static_cast<unsigned long long>(clock64() - t_tail0);
@@ -1508,7 +1573,8 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                            float thr, float delta, float thr_band, int64_t ref_index_base, const FilterOut& out,
                            RecheckLists lists, int no_recheck, float* dbg_scores, bool after_k1,
                            const int32_t* ref_map, const int32_t* n_ref_dev, cudaStream_t s,
-                           const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
+                           const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self,
+                           const PairRaw* pairs) {
     if (dim_pad % kBlockK != 0 || dim_pad < kBlockK || dim_pad > 512) {
         set_error("filter_mma: padded dim %d not in {64..512 step 64}", dim_pad);
         return FFR_ERR_UNSUPPORTED;
@@ -1532,6 +1598,10 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     const bool self_mode = self.mode >= 0;
     if (self_mode && (cg != 2 || fuse || no_recheck || dbg_scores != nullptr || n_ref_dev != nullptr)) {
         set_error("filter_mma: the self-mode kernel exists for cta_group::2, the K1 schedule and the re-checked build only");
+        return FFR_ERR_UNSUPPORTED;
+    }
+    if (pairs != nullptr && (cg != 2 || fuse || dbg_scores != nullptr || n_ref_dev != nullptr || (self_mode && self.mode != FFR_SELF_EARLIER))) {
+        set_error("filter_mma: the pairs form exists for cta_group::2, the K1 schedule, unfolded references and FFR_SELF_EARLIER only");
         return FFR_ERR_UNSUPPORTED;
     }
     const int kb = dim_pad / kBlockK;
@@ -1581,6 +1651,7 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     p.band_tol = out.band.tol; p.band_count = no_recheck ? out.band.count : nullptr; p.band_rows = out.band.rows; p.band_cap = out.band.cap;
     p.ref_bias = euclid_bias; p.cand_scale = cand_scale; p.bias_max = bias_max;
     p.self_row0 = self.row0; p.self_mode = self.mode;
+    p.pair = pairs != nullptr ? *pairs : PairRaw{};
     p.cand32 = cand32; p.cand16 = cand16; p.dim = dim;
     p.stage32 = st32 ? 1 : 0;
     p.s_bufs = s_bufs;
@@ -1610,8 +1681,11 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
     static const KernelFn euclid2[2] = {filter_mma_kernel<2, 0, 0, 0, false, true>, filter_mma_kernel<2, 0, 0, 1, false, true>};
     static const KernelFn self2[2][2] = {{filter_mma_kernel<2, 0, 0, 0, false, false, true>, filter_mma_kernel<2, 0, 0, 1, false, false, true>},
                                          {filter_mma_kernel<2, 0, 0, 0, false, true, true>, filter_mma_kernel<2, 0, 0, 1, false, true, true>}};
+    static const KernelFn pairs2[2][2] = {{filter_mma_kernel<2, 0, 0, 0, false, false, false, true>, filter_mma_kernel<2, 0, 0, 0, false, false, true, true>},
+                                          {filter_mma_kernel<2, 0, 0, 0, false, true, false, true>, filter_mma_kernel<2, 0, 0, 0, false, true, true, true>}};
     KernelFn fn;
-    if (self_mode)    fn = self2[euclid ? 1 : 0][p.grid_updates ? 1 : 0];
+    if (pairs)        fn = pairs2[euclid ? 1 : 0][self_mode ? 1 : 0];
+    else if (self_mode) fn = self2[euclid ? 1 : 0][p.grid_updates ? 1 : 0];
     else if (euclid)  fn = euclid2[p.grid_updates ? 1 : 0];
     else if (cg == 2) fn = instr ? instr2[nm] : prod2[nm][(p.grid_exact ? 2 : 0) + (p.grid_updates ? 1 : 0)];
     else              fn = instr ? instr1[nm] : prod1[nm];
@@ -1633,6 +1707,8 @@ int launch_filter_mma_impl(const __half* ref16, int64_t n_ref, __half* cand16, c
                 FFR_CUDA_TRY(cudaFuncSetAttribute(euclid2[v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
                 FFR_CUDA_TRY(cudaFuncSetAttribute(self2[0][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
                 FFR_CUDA_TRY(cudaFuncSetAttribute(self2[1][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+                FFR_CUDA_TRY(cudaFuncSetAttribute(pairs2[0][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
+                FFR_CUDA_TRY(cudaFuncSetAttribute(pairs2[1][v], cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemLimit));
             }
             attr_set[slot] = true;
         }
@@ -1687,10 +1763,11 @@ int launch_filter_mma(const __half* ref16, int64_t n_ref, __half* cand16, const 
                       int64_t n_cand, int32_t dim_pad, float thr, float delta, float thr_band, int64_t ref_index_base,
                       const FilterOut& out, RecheckLists lists, int no_recheck, bool after_k1, const int32_t* ref_map,
                       const int32_t* n_ref_dev, cudaStream_t s,
-                      const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self) {
+                      const float* euclid_bias, const float* cand_scale, const float* bias_max, SelfArgs self,
+                      const PairRaw* pairs) {
     return launch_filter_mma_impl(ref16, n_ref, cand16, cand32, dim, n_cand, dim_pad, thr, delta, thr_band, ref_index_base,
                                   out, lists, no_recheck, nullptr, after_k1, ref_map, n_ref_dev, s, euclid_bias, cand_scale,
-                                  bias_max, self);
+                                  bias_max, self, pairs);
 }
 
 // true when the fused schedule needs NO fp16 copy of the candidates in the workspace (stage32: the fp16 A tiles only ever
@@ -1711,7 +1788,7 @@ void get_last_k2_config(int out[8]) { for (int i = 0; i < 8; ++i) out[i] = g_las
 int launch_filter_mma_debug(const __half* ref16, int64_t n_ref, const __half* cand16, int64_t n_cand, int32_t dim_pad,
                             float thr, float delta, const FilterOut& out, RecheckLists lists, float* scores, cudaStream_t s) {
     return launch_filter_mma_impl(ref16, n_ref, const_cast<__half*>(cand16), nullptr, dim_pad, n_cand, dim_pad, thr, delta, delta, 0, out,
-                                  lists, 0, scores, false, nullptr, nullptr, s, nullptr, nullptr, nullptr, kNoSelf);
+                                  lists, 0, scores, false, nullptr, nullptr, s, nullptr, nullptr, nullptr, kNoSelf, nullptr);
 }
 
 }  // namespace ffr

@@ -282,10 +282,7 @@ euclid_ref_scale_kernel(const float* __restrict__ ref, int64_t n_ref, int32_t di
     const int64_t warp = (static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x) >> 5;
     const int64_t nwarps = (static_cast<int64_t>(gridDim.x) * kThreads) >> 5;
     const float mx = __uint_as_float(*max_bits);
-    int e = 0;
-    if (mx > 0.f && mx <= 3.4e38f) frexpf(mx, &e);                     // mx < 2^e
-    const int f = (e + 1) >> 1;                                         // |r| < 2^(e/2) <= 2^f
-    const float sc = ldexpf(1.0f, -f);
+    const float sc = euclid_ref_scale(mx);
     if (blockIdx.x == 0 && threadIdx.x == 0) *bmax = 0.5f * (mx * sc);
     for (int64_t r = warp; r < n_pad; r += nwarps) {
         if (r >= n_ref) { if (lane == 0) beta[r] = 0.f; continue; }

@@ -864,6 +864,22 @@ __global__ void unpack_results_kernel(const uint8_t* __restrict__ packed, int64_
     }
 }
 
+// |c| of one candidate row, lane-strided (float4 #(lane + 32 j) when vec), warp_sum, IEEE sqrt: the norm the all-reduce merge
+// and the match lists hand cos_fp32.  The whole warp calls it; every lane returns the norm.
+__device__ __forceinline__ float cand_norm_fp32(const float* __restrict__ c, int32_t dim, int lane, bool vec) {
+    float cc = 0.f;
+    if (vec) {
+        const float4* c4 = reinterpret_cast<const float4*>(c);
+        for (int k = lane; k < (dim >> 2); k += 32) {
+            const float4 t = __ldg(c4 + k);
+            cc = fmaf(t.x, t.x, cc); cc = fmaf(t.y, t.y, cc); cc = fmaf(t.z, t.z, cc); cc = fmaf(t.w, t.w, cc);
+        }
+    } else {
+        for (int d = lane; d < dim; d += 32) { const float t = __ldg(c + d); cc = fmaf(t, t, cc); }
+    }
+    return __fsqrt_rn(warp_sum(cc));
+}
+
 // ---- gallery over ranks (ffr_allreduce_best) --------------------------------------------------------------------------
 // Merge / value pass: the fp32 value of each row's winner on this rank, packed into the merge key with pack_key (above) --
 // (orderable(v) << 32) | ~global_idx, v = cosine score or -distance, so "largest key" = best value, then smallest global index
@@ -891,17 +907,7 @@ best_key_kernel(const float* __restrict__ ref, int64_t n_ref, int64_t ref_index_
         if (emode >= 0) {
             v = -k2s_euclid_dist(c, r, dim, lane, emode);
         } else {
-            float cc = 0.f;
-            if (vec) {
-                const float4* c4 = reinterpret_cast<const float4*>(c);
-                for (int k = lane; k < (dim >> 2); k += 32) {
-                    const float4 t = __ldg(c4 + k);
-                    cc = fmaf(t.x, t.x, cc); cc = fmaf(t.y, t.y, cc); cc = fmaf(t.z, t.z, cc); cc = fmaf(t.w, t.w, cc);
-                }
-            } else {
-                for (int d = lane; d < dim; d += 32) { const float t = __ldg(c + d); cc = fmaf(t, t, cc); }
-            }
-            v = cos_fp32(c, r, dim, __fsqrt_rn(warp_sum(cc)), lane, vec);
+            v = cos_fp32(c, r, dim, cand_norm_fp32(c, dim, lane, vec), lane, vec);
         }
         if (lane == 0) keys[row] = pack_key(v, g);
     }
@@ -935,7 +941,166 @@ __global__ void emit_keys_kernel(const unsigned long long* __restrict__ keys, in
     }
 }
 
+// ---- match lists (ffr_match_pairs*) ---------------------------------------------------------------------------------------
+// A pair's fp32 value, the contract's arithmetic on both paths: cosine = cos_fp32 on the candidate's cand_norm_fp32 (the merge's
+// value), Euclid = k2s_euclid_dist in K2s's form emode.  c may be a parked copy of the candidate row: the arithmetic, not the
+// address, fixes the bits.  The whole warp calls it; every lane returns the value.
+template <bool kEuclid>
+__device__ __forceinline__ float pair_value(const float* c, const float* __restrict__ r, int32_t dim, float c_norm, int lane,
+                                            bool vec, int emode) {
+    if constexpr (kEuclid) return k2s_euclid_dist(c, r, dim, lane, emode);
+    else                   return cos_fp32(c, r, dim, c_norm, lane, vec);
+}
+template <bool kEuclid>
+__device__ __forceinline__ bool pair_accepted(float v, float thr) { return kEuclid ? v <= thr : v >= thr; }
+
+// Appends the warp's accepted pairs (lane k holds the k-th pair of this batch) with one atomic on *ctr; returns the batch's count
+__device__ __forceinline__ uint32_t append_accepted(bool acc, int32_t row, int64_t ref, float v, unsigned long long* ctr,
+                                                    const PairOut& out, int lane) {
+    const uint32_t bal = __ballot_sync(0xffffffffu, acc);
+    if (bal == 0u) return 0u;
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(ctr, static_cast<unsigned long long>(__popc(bal)));
+    base = __shfl_sync(0xffffffffu, base, 0);
+    const unsigned long long slot = base + __popc(bal & ((1u << lane) - 1u));
+    if (acc && slot < static_cast<unsigned long long>(out.cap)) {
+        out.cand[slot] = row;
+        out.ref[slot] = static_cast<int32_t>(ref);
+        out.val[slot] = v;
+    }
+    return static_cast<uint32_t>(__popc(bal));
+}
+
+constexpr int kPairMaxDim = 512;      // the finishing pass runs behind the tensor-core path only (dim <= 512)
+
+// Finishing pass.  Work items: groups of 32 raw entries (min(raw count, capacity) of them), then (exact row, 32 references).
+// A warp takes a group's entries one after the other; K2 appends the columns of one (row, tile half) together, so the candidate
+// row is parked in shared memory (and, cosine, its norm summed) once per run of entries, not once per entry.  Accepted pairs are
+// appended warp-aggregated.  The last block to finish writes the caller's count: the accepted pairs, or when the raw list
+// overflowed the raw count plus the exact rows' pairs (the accepted raw entries are a subset of the raw ones).
+template <bool kEuclid>
+__global__ void __launch_bounds__(kThreads)
+pairs_finish_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int32_t dim, float thr,
+                    int64_t ref_index_base, SelfArgs self, PairRaw raw, WsHeader* hdr, PairOut out, bool vec, int emode) {
+    __shared__ __align__(16) float s_rows[kWarps][kPairMaxDim];
+    const int lane = threadIdx.x & 31;
+    float* c_s = s_rows[threadIdx.x >> 5];
+    const int64_t warp = static_cast<int64_t>(blockIdx.x) * kWarps + (threadIdx.x >> 5);
+    const int64_t nwarps = static_cast<int64_t>(gridDim.x) * kWarps;
+    const unsigned long long raw_all = hdr->raw_count;
+    const int64_t n_raw = raw_all < static_cast<unsigned long long>(raw.cap) ? static_cast<int64_t>(raw_all) : raw.cap;
+    const int64_t n_exact = kEuclid ? hdr->exact_count : 0;
+    const int64_t g_raw = (n_raw + 31) / 32, ref_chunks = (n_ref + 31) / 32;
+    const int64_t n_items = g_raw + n_exact * ref_chunks;
+    int64_t parked = -1;
+    float c_norm = 0.f;
+    const auto park = [&](int32_t row) {
+        if (row == parked) return;
+        const float* c = cand + static_cast<int64_t>(row) * dim;
+        __syncwarp();
+        for (int k = lane; k < dim; k += 32) c_s[k] = __ldg(c + k);
+        __syncwarp();
+        if (!kEuclid) c_norm = cand_norm_fp32(c, dim, lane, vec);
+        parked = row;
+    };
+    for (int64_t it = warp; it < n_items; it += nwarps) {
+        bool acc = false;
+        int32_t my_row = 0;
+        int64_t my_ref = 0;
+        float my_v = 0.f;
+        const bool exact = it >= g_raw;
+        if (!exact) {
+            const int64_t e = it * 32 + lane;
+            const uint2 en = e < n_raw ? raw.raw[e] : make_uint2(0xFFFFFFFFu, 0u);
+            for (int k = 0; k < 32; ++k) {
+                const uint32_t row = __shfl_sync(0xffffffffu, en.x, k), col = __shfl_sync(0xffffffffu, en.y, k);
+                if (row == 0xFFFFFFFFu) break;                                 // (the group's tail: the same for every lane)
+                park(static_cast<int32_t>(row));
+                const float v = pair_value<kEuclid>(c_s, ref + static_cast<int64_t>(col) * dim, dim, c_norm, lane, vec, emode);
+                if (lane == k) { my_v = v; my_row = static_cast<int32_t>(row); my_ref = col; acc = pair_accepted<kEuclid>(v, thr); }
+            }
+        } else {
+            const int64_t x = it - g_raw, i0 = (x % ref_chunks) * 32;
+            const int32_t row = __ldg(raw.exact_rows + x / ref_chunks);
+            park(row);
+            const int64_t i_end = self.mode >= 0 ? (self.row0 + row < n_ref ? self.row0 + row : n_ref) : n_ref;
+            for (int k = 0; k < 32 && i0 + k < i_end; ++k) {
+                const float v = pair_value<kEuclid>(c_s, ref + (i0 + k) * dim, dim, c_norm, lane, vec, emode);
+                if (lane == k) { my_v = v; my_row = row; my_ref = i0 + k; acc = pair_accepted<kEuclid>(v, thr); }
+            }
+        }
+        const uint32_t n_acc = append_accepted(acc, my_row, my_ref + ref_index_base, my_v, &hdr->acc_count, out, lane);
+        if (exact && n_acc != 0u && lane == 0) atomicAdd(&hdr->acc_exact, static_cast<unsigned long long>(n_acc));
+    }
+    __threadfence();
+    __syncthreads();
+    if (threadIdx.x == 0 && atomicAdd(&hdr->pairs_blocks, 1) == static_cast<int32_t>(gridDim.x) - 1) {
+        __threadfence();
+        const unsigned long long acc = atomicAdd(&hdr->acc_count, 0ull), ex = atomicAdd(&hdr->acc_exact, 0ull);
+        *out.count = static_cast<int64_t>(raw_all > static_cast<unsigned long long>(raw.cap) ? raw_all + ex : acc);
+    }
+}
+
+// Exact path: one warp per candidate row against every reference (self: the rows i < g), 32 references per append
+template <bool kEuclid>
+__global__ void __launch_bounds__(kThreads)
+pairs_exact_kernel(const float* __restrict__ ref, int64_t n_ref, const float* __restrict__ cand, int64_t n_cand, int32_t dim,
+                   float thr, int64_t ref_index_base, SelfArgs self, PairOut out, bool vec, int emode) {
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = static_cast<int64_t>(blockIdx.x) * kWarps + (threadIdx.x >> 5);
+    const int64_t nwarps = static_cast<int64_t>(gridDim.x) * kWarps;
+    unsigned long long* ctr = reinterpret_cast<unsigned long long*>(out.count);
+    for (int64_t row = warp; row < n_cand; row += nwarps) {
+        const float* c = cand + row * dim;
+        const float c_norm = kEuclid ? 0.f : cand_norm_fp32(c, dim, lane, vec);
+        const int64_t i_end = self.mode >= 0 ? (self.row0 + row < n_ref ? self.row0 + row : n_ref) : n_ref;
+        for (int64_t i0 = 0; i0 < i_end; i0 += 32) {
+            bool acc = false;
+            float my_v = 0.f;
+            for (int k = 0; k < 32 && i0 + k < i_end; ++k) {
+                const float v = pair_value<kEuclid>(c, ref + (i0 + k) * dim, dim, c_norm, lane, vec, emode);
+                if (lane == k) { my_v = v; acc = pair_accepted<kEuclid>(v, thr); }
+            }
+            append_accepted(acc, static_cast<int32_t>(row), i0 + lane + ref_index_base, my_v, ctr, out, lane);
+        }
+    }
+}
+
+// the candidates' float4 form (cos_fp32 / cand_norm_fp32) and K2s's Euclid form, the same for both paths of a call
+bool pairs_vec(const float* ref, const float* cand, int32_t dim) {
+    return (dim % 4 == 0) && ((reinterpret_cast<uintptr_t>(ref) & 15) == 0) && ((reinterpret_cast<uintptr_t>(cand) & 15) == 0);
+}
+int pairs_emode(const float* ref, const float* cand, int64_t n_ref, int32_t dim, int metric, SelfArgs self) {
+    if (metric != FFR_METRIC_EUCLID) return -1;
+    return k2s_form(ref, cand, self.mode >= 0 ? INT64_MAX : n_ref, dim);
+}
+
 }  // namespace
+
+int launch_pairs_finish(const float* ref, int64_t n_ref, const float* cand, int32_t dim, int metric, float thr, int64_t ref_index_base,
+                        SelfArgs self, const PairRaw& raw, WsHeader* hdr, const PairOut& out, cudaStream_t s) {
+    if (dim > kPairMaxDim) { set_error("pairs: finishing pass needs dim <= %d", kPairMaxDim); return FFR_ERR_UNSUPPORTED; }
+    const bool vec = pairs_vec(ref, cand, dim);
+    const int emode = pairs_emode(ref, cand, n_ref, dim, metric, self);
+    const unsigned grid = static_cast<unsigned>(num_sms()) * 4;
+    if (emode >= 0) pairs_finish_kernel<true><<<grid, kThreads, 0, s>>>(ref, n_ref, cand, dim, thr, ref_index_base, self, raw, hdr, out, vec, emode);
+    else            pairs_finish_kernel<false><<<grid, kThreads, 0, s>>>(ref, n_ref, cand, dim, thr, ref_index_base, self, raw, hdr, out, vec, emode);
+    FFR_LAUNCH_CHECK("pairs_finish");
+    return FFR_OK;
+}
+
+int launch_pairs_exact(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
+                       int64_t ref_index_base, SelfArgs self, const PairOut& out, cudaStream_t s) {
+    if (n_cand == 0) return FFR_OK;
+    const bool vec = pairs_vec(ref, cand, dim);
+    const int emode = pairs_emode(ref, cand, n_ref, dim, metric, self);
+    int64_t grid = (n_cand + kWarps - 1) / kWarps;
+    if (grid > static_cast<int64_t>(num_sms()) * 8) grid = static_cast<int64_t>(num_sms()) * 8;
+    if (emode >= 0) pairs_exact_kernel<true><<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, self, out, vec, emode);
+    else            pairs_exact_kernel<false><<<static_cast<unsigned>(grid), kThreads, 0, s>>>(ref, n_ref, cand, n_cand, dim, thr, ref_index_base, self, out, vec, emode);
+    FFR_LAUNCH_CHECK("pairs_exact");
+    return FFR_OK;
+}
 
 int launch_best_keys(const float* ref, int64_t n_ref, int64_t ref_index_base, const float* cand, int64_t n_cand, int32_t dim,
                      int metric, const int32_t* best_idx, unsigned long long* keys, cudaStream_t s) {

@@ -21,7 +21,8 @@ from . import _lib
 from ._lib import (DTYPE_F16, DTYPE_F32, ERR_UNSUPPORTED, FLAG_FORCE_FP32, FLAG_FORCE_MMA, FLAG_NO_RECHECK, METRIC_COSINE,
                    METRIC_EUCLID, SELF_EARLIER, SELF_OTHERS, FfrError, check)
 
-__all__ = ["l2norm_rows", "face_filter", "self_filter", "cosine_filter", "ref_mean_and_thres", "FilterResult", "HostFilter", "GraphedFilter",
+__all__ = ["l2norm_rows", "face_filter", "self_filter", "match_pairs", "self_pairs", "cosine_filter", "ref_mean_and_thres",
+           "FilterResult", "PairResult", "HostFilter", "GraphedFilter",
            "ResultGather", "launch_count", "METRIC_COSINE", "METRIC_EUCLID", "FLAG_FORCE_FP32", "FLAG_FORCE_MMA",
            "FLAG_NO_RECHECK", "SELF_OTHERS", "SELF_EARLIER"]
 
@@ -220,6 +221,97 @@ def self_filter(x: torch.Tensor, thr: float, metric="cosine", mode="others", row
         if want_stats:
             res.stats = _stats(lib, ws, dev)
     return res
+
+
+@dataclass
+class PairResult:
+    cand: torch.Tensor                       # int64 [P]  candidate row (local to the call / the row range)
+    ref: torch.Tensor                        # int64 [P]  reference row + ref_index_base (self: global row of x, < the candidate's)
+    val: torch.Tensor                        # float32 [P] the pair's fp32 cosine similarity or Euclid distance
+    stats: Optional[dict] = None
+
+
+def _default_pair_cap(n_cand: int) -> int:
+    return max(8 * n_cand, 1 << 16)
+
+
+def _pairs(lib, dev, ws_bytes, launch, cap: int, want_stats: bool) -> PairResult:
+    """Run ``launch(ws, cand, ref, val, cap, count)`` and read the count (the call's one host synchronisation); on overflow run it
+    once more with ``cap = count``, which the C contract guarantees to be complete.  Sorted by (cand, ref)."""
+    for _ in range(2):
+        ws = _workspace(dev, int(ws_bytes(cap)))
+        pc = torch.empty((cap,), dtype=torch.int32, device=dev)
+        pr = torch.empty((cap,), dtype=torch.int32, device=dev)
+        pv = torch.empty((cap,), dtype=torch.float32, device=dev)
+        count = torch.empty((1,), dtype=torch.int64, device=dev)
+        with torch.cuda.device(dev):
+            check(launch(ws, pc.data_ptr() if cap else None, pr.data_ptr() if cap else None, pv.data_ptr() if cap else None, cap,
+                         count.data_ptr()))
+        n = int(count.item())
+        if n <= cap:
+            break
+        cap = n
+    c, r, v = pc[:n].long(), pr[:n].long(), pv[:n]
+    order = torch.argsort((c << 32) | r)
+    res = PairResult(c[order], r[order], v[order])
+    if want_stats:
+        arr = (C.c_int64 * 8)()
+        with torch.cuda.device(dev):
+            check(lib.ffr_filter_stats(ws.data_ptr(), arr, _stream_ptr(dev)))
+        res.stats = {"raw_pairs": arr[0], "path": "tcgen05" if arr[2] == 1 else "fp32", "launches": arr[3]}
+    return res
+
+
+def match_pairs(ref: torch.Tensor, cand: torch.Tensor, thr: float, metric="cosine", ref_index_base: int = 0,
+                cap: Optional[int] = None, flags: int = 0, want_stats: bool = False) -> PairResult:
+    """Every (candidate, reference) pair on the matching side of the threshold -- cosine: ``(r.c)/(|r||c|) >= thr``, euclid:
+    ``|c - r| <= thr`` -- without the [M, N] score matrix.  ``ref`` [N, D], ``cand`` [M, D]: float32 CUDA tensors.
+
+    Each pair's value is its fp32 cosine / distance, and that value decides membership (the tensor cores only pre-select);
+    bit-identical references are not folded.  The list is sorted by (cand, ref).  ``cap`` sizes the device list (default
+    ``max(8 * M, 65536)`` pairs); if more pairs match, the call runs once more with the exact size.  Reading the count is a host
+    synchronisation, so this call cannot be captured into a CUDA graph."""
+    lib = _lib.load()
+    m = _METRICS[metric]
+    for name, t in (("ref", ref), ("cand", cand)):
+        if isinstance(t, torch.Tensor) and t.dtype == torch.float16:
+            raise FfrError(ERR_UNSUPPORTED, f"match_pairs takes float32 embeddings ({name} is float16)")
+    ref = _require_cuda(ref, "ref")
+    cand = _require_cuda(cand, "cand")
+    if ref.dim() != 2 or cand.dim() != 2 or cand.shape[1] != ref.shape[1]:
+        raise ValueError(f"ref {tuple(ref.shape)} and cand {tuple(cand.shape)} must be [N, D] and [M, D]")
+    if ref.device != cand.device:
+        raise ValueError("ref and cand must be on the same device")
+    (n_ref, dim), n_cand, dev = ref.shape, cand.shape[0], cand.device
+    cap = _default_pair_cap(n_cand) if cap is None else int(cap)
+    return _pairs(lib, dev, lambda k: lib.ffr_match_pairs_workspace_bytes(n_ref, n_cand, dim, m, k),
+                  lambda ws, pc, pr, pv, k, cnt: lib.ffr_match_pairs(
+                      ref.data_ptr(), n_ref, cand.data_ptr() if n_cand else None, n_cand, dim, m, float(thr), int(ref_index_base),
+                      pc, pr, pv, k, cnt, int(flags), ws.data_ptr(), ws.numel(), _stream_ptr(dev)), cap, want_stats)
+
+
+def self_pairs(x: torch.Tensor, thr: float, metric="cosine", rows: Optional[Tuple[int, int]] = None, cap: Optional[int] = None,
+               flags: int = 0, want_stats: bool = False) -> PairResult:
+    """Every pair of rows i < j of ``x`` [N, D] (float32 CUDA) on the matching side of the threshold, each unordered pair once:
+    the edges of the duplicate groups ``self_filter(mode="earlier")`` only flags.  ``rows=(begin, end)``: only candidate rows j in
+    that range (results local to it; ``ref`` is a global row of ``x``), so the union over a split of the rows is the whole list.
+    Value, threshold, sorting, ``cap`` (default ``max(8 * rows, 65536)``) and the host synchronisation are ``match_pairs``'s."""
+    lib = _lib.load()
+    m = _METRICS[metric]
+    if isinstance(x, torch.Tensor) and x.dtype == torch.float16:
+        raise FfrError(ERR_UNSUPPORTED, "self_pairs takes float32 embeddings (fp16 rows are not supported)")
+    x = _require_cuda(x, "x")
+    if x.dim() != 2:
+        raise ValueError(f"x {tuple(x.shape)} must be [N, D]")
+    n, dim = x.shape
+    begin, end = (0, n) if rows is None else (int(rows[0]), int(rows[1]))
+    n_rows = max(end - begin, 0)
+    dev = x.device
+    cap = _default_pair_cap(n_rows) if cap is None else int(cap)
+    return _pairs(lib, dev, lambda k: lib.ffr_match_pairs_self_workspace_bytes(n, n_rows, dim, m, k),
+                  lambda ws, pc, pr, pv, k, cnt: lib.ffr_match_pairs_self(
+                      x.data_ptr(), n, begin, end - begin, dim, m, float(thr), pc, pr, pv, k, cnt, int(flags), ws.data_ptr(),
+                      ws.numel(), _stream_ptr(dev)), cap, want_stats)
 
 
 class GraphedFilter:

@@ -135,11 +135,42 @@ int ffr_filter_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows
                     float band_tol, int32_t* band_count, int64_t* band_rows, int64_t band_cap,
                     int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
 
+/* ---- match lists: every (candidate, reference) pair on the matching side of the threshold -------------------------
+ *   cosine: (r.c) / (|r| |c|) >= thr        euclid: |c - r| <= thr
+ * ffr_match_pairs: ref[n_ref, dim] and cand[n_cand, dim] fp32 (device).  ffr_match_pairs_self: x[n, dim] fp32 (device); the
+ * candidates are rows [row_begin, row_begin + n_rows) of x, the references the rows i < j of x (each unordered pair once).
+ *   Indices: pair_cand[k] is the candidate row local to the call (like band_rows); pair_ref[k] is the reference row plus
+ *     ref_index_base (self: the global row of x, always less than the candidate's global row).  The list is unordered.
+ *   Value: pair_val[k] is the pair's fp32 value -- cosine: K3's arithmetic (the candidate norm summed as the all-reduce merge
+ *     sums it); Euclid: the distance the exact kernel K2s computes for that pair in the call of the same shape (self mode: its
+ *     self form).  That fp32 value decides membership on every path; a tensor-core score never does.
+ *   Count (*pair_count, device int64): if *pair_count <= pair_cap, entries [0, *pair_count) are exactly the pairs.  Otherwise
+ *     the list is incomplete and *pair_count is an upper bound: a second call on the same inputs with pair_cap >= *pair_count
+ *     returns the complete list.  pair_cap = 0 is valid: the call counts and writes nothing.
+ *   Bit-identical references are not folded: every copy is a pair.
+ *   Flags: FFR_FLAG_FORCE_FP32 selects the exact CUDA-core kernel; FFR_FLAG_FORCE_MMA fails (FFR_ERR_UNSUPPORTED) where the
+ *     tensor-core path is not eligible; FFR_FLAG_NO_RECHECK is refused (FFR_ERR_UNSUPPORTED): the fp32 decision is the contract.
+ *   Dispatch: tensor cores when n_ref > 8 (self: n > 8), dim <= 512, the GPU runs cta_group::2 and FFR_FLAG_FORCE_FP32 is not
+ *     set; otherwise the exact kernel.  Both paths return the same pairs with bit-identical values.
+ *   Indices must fit int32: ref_index_base >= 0 and ref_index_base + n_ref < 2^31 (self: n < 2^31), else FFR_ERR_INVALID.
+ *   Asynchronous on the stream, no host synchronisation, no allocation.  The workspace (256-byte aligned) holds the raw list of
+ *   pair_cap 8-byte entries besides K1's operands; ffr_filter_stats works on it: out[0] = pairs the tensor-core kernel listed
+ *   for the fp32 decision, out[2] = path, out[3] = kernels launched, the rest 0. */
+size_t ffr_match_pairs_workspace_bytes(int64_t n_ref, int64_t n_cand, int32_t dim, int metric, int64_t pair_cap);
+int ffr_match_pairs(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
+                    int64_t ref_index_base, int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap,
+                    int64_t* pair_count, int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
+size_t ffr_match_pairs_self_workspace_bytes(int64_t n, int64_t n_rows, int32_t dim, int metric, int64_t pair_cap);
+int ffr_match_pairs_self(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int32_t dim, int metric, float thr,
+                         int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap, int64_t* pair_count,
+                         int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
+
 /* statistics of the last ffr_filter* call that used this workspace (device->host copy, synchronises
  * the stream): out[0] = rows re-checked in fp32 against their two or three leading references (near-tie or
  * near-threshold), out[1] = rows that needed the full fp32 rescan, out[2] = path taken (0 fp32 CUDA-core,
  * 1 tcgen05), out[3] = kernels launched, out[4] = rows re-checked against one 128-reference part, out[5] = reference
- * rows the tensor-core kernel scanned (< n_ref when bit-identical reference rows were folded), out[6..7] = 0. */
+ * rows the tensor-core kernel scanned (< n_ref when bit-identical reference rows were folded), out[6..7] = 0.
+ * (After ffr_match_pairs*: see there.) */
 int ffr_filter_stats(const void* workspace, int64_t out[8], ffr_stream_t stream);
 
 /* ---- K5: reference statistics -----------------------------------------------------------------
