@@ -13,7 +13,8 @@ import sys
 PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "libffr_b200.so")
-SOURCES = ["ffr_api.cu", "ffr_l2norm.cu", "ffr_filter_fp32.cu", "ffr_filter_mma.cu", "ffr_recheck.cu", "ffr_gallery.cu", "ffr_dedup.cu"]
+SOURCES = ["ffr_api.cu", "ffr_l2norm.cu", "ffr_filter_fp32.cu", "ffr_filter_mma.cu", "ffr_recheck.cu", "ffr_gallery.cu", "ffr_dedup.cu",
+           "ffr_groups.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC"]
 

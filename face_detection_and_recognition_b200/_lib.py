@@ -52,6 +52,8 @@ SIGNATURES = {
     "ffr_match_pairs_self_workspace_bytes": (_sz, [_i64, _i64, _i32, C.c_int, _i64]),
     "ffr_match_pairs_self": (C.c_int, [_vp, _i64, _i64, _i64, _i32, C.c_int, _f32, _vp, _vp, _vp, _i64, _vp, C.c_int, _vp,
                                        _sz, _vp]),
+    "ffr_self_groups_workspace_bytes": (_sz, [_i64, _i32, C.c_int, _i64]),
+    "ffr_self_groups": (C.c_int, [_vp, _i64, _i32, C.c_int, _f32, _vp, _vp, _i64, _vp, C.c_int, _vp, _sz, _vp]),
     "ffr_ref_mean_and_thres": (C.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "ffr_ref_mean_and_thres_batched": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _vp, _vp]),
     "ffr_first_match_stream": (C.c_int, [_vp, _vp, _vp, _i32, _vp, _vp, _i32, _i32, C.c_int, _f32, _f32, _vp, _vp]),

@@ -110,6 +110,8 @@ struct Ws {
     float *e_bias, *e_bias_c, *e_nsq, *e_scal, *e_cscale;   // Euclid on the tensor cores
     uint2* pair_raw;                                      // match lists: K2's raw pair list ...
     int32_t* exact_rows;                                  // ... and its exact-row list (Euclid)
+    int32_t *edge_cand, *edge_ref;                        // near-duplicate groups: the accepted pairs (the graph's edges) ...
+    float* edge_val;                                      // ... and their values, on both paths
     size_t total;
 };
 
@@ -135,8 +137,9 @@ bool mma_eligible(int64_t n_ref, int32_t dim, int metric, int flags) {
 // base: the workspace to carve (nullptr: only the size is wanted)
 // pair_cap >= 0: a match-list call -- no re-check lists and no fold; the raw pair list (pair_cap entries) and, Euclid, the
 // exact-row list follow the Euclid buffers
+// edge_cap >= 0: a groups call -- the accepted-pair list (edge_cap entries of cand / ref / val) comes last, on either path
 Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bool need_c16, bool dedup, bool euclid = false,
-             void* base = nullptr, int64_t pair_cap = -1) {
+             void* base = nullptr, int64_t pair_cap = -1, int64_t edge_cap = -1) {
     Ws L{};
     size_t off = 0;
     const auto take = [&](size_t bytes) {
@@ -172,6 +175,12 @@ Ws ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int dtype, bool mma, bo
             L.pair_raw = static_cast<uint2*>(take(static_cast<size_t>(pair_cap) * sizeof(uint2)));
             L.exact_rows = static_cast<int32_t*>(take(euclid ? nc * sizeof(int32_t) : 0));
         }
+    }
+    if (edge_cap >= 0) {
+        const size_t ne = static_cast<size_t>(edge_cap);
+        L.edge_cand = static_cast<int32_t*>(take(ne * sizeof(int32_t)));
+        L.edge_ref = static_cast<int32_t*>(take(ne * sizeof(int32_t)));
+        L.edge_val = static_cast<float*>(take(ne * sizeof(float)));
     }
     L.total = off;
     return L;
@@ -415,12 +424,13 @@ int self_core(const float* x, int64_t n, int64_t row_begin, int64_t n_rows, int3
 // The tensor-core path takes self mode's rule (self_mma_eligible: n_ref > 8, dim <= 512, cta_group::2, not FFR_FLAG_FORCE_FP32) for
 // both metrics, gallery and self.
 
-// self: the candidates are rows of the references (cosine reads them from the references' fp16 copy)
+// self: the candidates are rows of the references (cosine reads them from the references' fp16 copy).  edge_cap >= 0: a groups
+// call, whose accepted pairs go to the workspace (pair_cap = edge_cap)
 Ws pairs_ws_layout(int64_t n_ref, int64_t n_cand, int32_t dim, int metric, bool self, bool mma, int64_t pair_cap,
-                   void* base = nullptr) {
+                   void* base = nullptr, int64_t edge_cap = -1) {
     const bool euclid = metric == FFR_METRIC_EUCLID;
     return ws_layout(n_ref, n_cand, dim, FFR_DTYPE_F32, mma, /*need_c16=*/!self || euclid, /*dedup=*/false, mma && euclid, base,
-                     pair_cap);
+                     pair_cap, edge_cap);
 }
 
 int check_pairs_out(int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap, int64_t* pair_count, int flags) {
@@ -654,6 +664,48 @@ int ffr_match_pairs_self(const float* x, int64_t n, int64_t row_begin, int64_t n
     const Ws L = pairs_ws_layout(n, n_rows, dim, metric, true, mma, pair_cap, workspace);
     return run_pairs(x, n, x + row_begin * dim, n_rows, dim, metric, thr, 0, PairOut{pair_cand, pair_ref, pair_val, pair_cap, pair_count},
                      SelfArgs{row_begin, FFR_SELF_EARLIER}, mma, L, workspace, ws_bytes, static_cast<cudaStream_t>(stream));
+}
+
+// Near-duplicate groups: the match list of x against itself goes to the workspace's edge list (run_pairs as ffr_match_pairs_self
+// runs it), then the union-find (ffr_groups.cu) labels each row with its component's smallest row.  *edge_count is the pair count.
+size_t ffr_self_groups_workspace_bytes(int64_t n, int32_t dim, int metric, int64_t edge_cap) {
+    if (n <= 0 || n > static_cast<int64_t>(INT32_MAX) || dim <= 0 || edge_cap < 0) return 0;
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) return 0;
+    return pairs_ws_layout(n, n, dim, metric, true, dim <= 512 && n > 8, edge_cap, nullptr, edge_cap).total;
+}
+
+int ffr_self_groups(const float* x, int64_t n, int32_t dim, int metric, float thr, int32_t* labels, int64_t* group_count,
+                    int64_t edge_cap, int64_t* edge_count, int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream) {
+    if (n <= 0 || n > static_cast<int64_t>(INT32_MAX)) { set_error("n must be in (0, 2^31) (got %lld)", (long long)n); return FFR_ERR_INVALID; }
+    if (dim <= 0) { set_error("dim must be > 0 (got %d)", dim); return FFR_ERR_INVALID; }
+    if (x == nullptr || labels == nullptr || group_count == nullptr) { set_error("null pointer argument"); return FFR_ERR_INVALID; }
+    if (metric != FFR_METRIC_COSINE && metric != FFR_METRIC_EUCLID) { set_error("unknown metric %d", metric); return FFR_ERR_INVALID; }
+    if (edge_count == nullptr || edge_cap < 0) { set_error("groups: need edge_count and edge_cap >= 0"); return FFR_ERR_INVALID; }
+    if (flags & FFR_FLAG_NO_RECHECK) {
+        set_error("FFR_FLAG_NO_RECHECK is not supported by the groups (the fp32 value decides every edge)");
+        return FFR_ERR_UNSUPPORTED;
+    }
+    if (ffr_device_count() == 0) { set_error("no CUDA device"); return FFR_ERR_CUDA; }
+    const bool mma = self_mma_eligible(n, dim, flags);
+    if ((flags & FFR_FLAG_FORCE_MMA) && !mma) {
+        set_error("FFR_FLAG_FORCE_MMA: the self-mode tcgen05 path needs n > 8, dim <= 512 and cta_group::2 (n=%lld dim=%d)",
+                  (long long)n, dim);
+        return FFR_ERR_UNSUPPORTED;
+    }
+    const Ws L = pairs_ws_layout(n, n, dim, metric, true, mma, edge_cap, workspace, edge_cap);
+    cudaStream_t s = static_cast<cudaStream_t>(stream);
+    int rc = run_pairs(x, n, x, n, dim, metric, thr, 0, PairOut{L.edge_cand, L.edge_ref, L.edge_val, edge_cap, edge_count},
+                       SelfArgs{0, FFR_SELF_EARLIER}, mma, L, workspace, ws_bytes, s);
+    if (rc != FFR_OK) return rc;
+    rc = launch_groups_init(labels, n, group_count, s);
+    if (rc != FFR_OK) return rc;
+    // the slots the pairs kernels filled: the finishing pass's accepted count (its *edge_count is an upper bound after an
+    // overflow of the raw list), or the exact kernel's count, which is that same slot counter
+    const unsigned long long* filled = mma ? &L.hdr->acc_count : reinterpret_cast<const unsigned long long*>(edge_count);
+    rc = launch_groups_union(L.edge_ref, L.edge_cand, edge_cap, filled, labels, n, group_count, s);
+    if (rc != FFR_OK) return rc;
+    g_last.launches += edge_cap > 0 ? 3 : 2;
+    return FFR_OK;
 }
 
 int ffr_ref_mean_and_thres(const float* ref_feat, int32_t n_ref, int32_t dim, float* mean, float* thres,

@@ -409,6 +409,12 @@ int launch_pairs_finish(const float* ref, int64_t n_ref, const float* cand, int3
 // The exact path: one warp per candidate row over every reference, the same value arithmetic; *out.count must be zero before
 int launch_pairs_exact(const float* ref, int64_t n_ref, const float* cand, int64_t n_cand, int32_t dim, int metric, float thr,
                        int64_t ref_index_base, SelfArgs self, const PairOut& out, cudaStream_t s);
+// Near-duplicate groups (ffr_groups.cu): labels[i] = i and *group_count = 0; then the union-find over the edges (edge_a[k],
+// edge_b[k]), k < min(*filled, cap) (*filled read on the device), and the final labels (each row's smallest component row) with
+// their count
+int launch_groups_init(int32_t* labels, int64_t n, int64_t* group_count, cudaStream_t s);
+int launch_groups_union(const int32_t* edge_a, const int32_t* edge_b, int64_t cap, const unsigned long long* filled, int32_t* labels,
+                        int64_t n, int64_t* group_count, cudaStream_t s);
 // exact-duplicate reference rows folded before K2 (ffr_dedup.cu)
 bool dedup_wanted(int64_t n_ref, int64_t n_cand);
 size_t dedup_workspace_bytes(int64_t n_ref, int32_t ld);

@@ -104,3 +104,19 @@ def filter_embedding_files(ref_paths: Sequence[str], cand_paths: Sequence[str], 
     finally:
         hf.close()
     return keep, idx, val, cand_prov, ref_prov
+
+
+def group_embedding_files(paths: Sequence[str], thr: float, metric: str = "cosine", feature_size: Optional[int] = None,
+                          device: int = 0):
+    """Near-duplicate groups straight from files (the cleaner's ``.pkl`` / ``data.npy`` / media ``.npy`` output): all embeddings
+    of ``paths`` are loaded into one set and grouped on the GPU (``ops.self_groups``).  Returns (labels int32 [n] NumPy, the
+    number of groups, provenance): ``labels[k]`` is the smallest row of row k's group, and ``prov[k]`` / ``prov[labels[k]]``
+    name the file and the index in it of row k and of its group's first occurrence."""
+    import torch
+
+    from . import ops
+    x, prov = load_embeddings(paths, feature_size)
+    if x.shape[0] == 0:
+        raise ValueError("no embeddings found")
+    res = ops.self_groups(torch.from_numpy(x).to(torch.device("cuda", device)), thr, metric=metric)
+    return res.labels.cpu().numpy(), res.n_groups, prov

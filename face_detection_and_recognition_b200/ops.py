@@ -21,8 +21,8 @@ from . import _lib
 from ._lib import (DTYPE_F16, DTYPE_F32, ERR_UNSUPPORTED, FLAG_FORCE_FP32, FLAG_FORCE_MMA, FLAG_NO_RECHECK, METRIC_COSINE,
                    METRIC_EUCLID, SELF_EARLIER, SELF_OTHERS, FfrError, check)
 
-__all__ = ["l2norm_rows", "face_filter", "self_filter", "match_pairs", "self_pairs", "cosine_filter", "ref_mean_and_thres",
-           "FilterResult", "PairResult", "HostFilter", "GraphedFilter",
+__all__ = ["l2norm_rows", "face_filter", "self_filter", "match_pairs", "self_pairs", "self_groups", "cosine_filter",
+           "ref_mean_and_thres", "FilterResult", "PairResult", "GroupResult", "HostFilter", "GraphedFilter",
            "ResultGather", "launch_count", "METRIC_COSINE", "METRIC_EUCLID", "FLAG_FORCE_FP32", "FLAG_FORCE_MMA",
            "FLAG_NO_RECHECK", "SELF_OTHERS", "SELF_EARLIER"]
 
@@ -312,6 +312,52 @@ def self_pairs(x: torch.Tensor, thr: float, metric="cosine", rows: Optional[Tupl
                   lambda ws, pc, pr, pv, k, cnt: lib.ffr_match_pairs_self(
                       x.data_ptr(), n, begin, end - begin, dim, m, float(thr), pc, pr, pv, k, cnt, int(flags), ws.data_ptr(),
                       ws.numel(), _stream_ptr(dev)), cap, want_stats)
+
+
+@dataclass
+class GroupResult:
+    labels: torch.Tensor                     # int32 [N]  smallest row of each row's group (labels[i] == i: i represents it)
+    n_groups: int                            # number of groups (connected components)
+    n_edges: int                             # matching pairs i < j (the graph's edges)
+    stats: Optional[dict] = None
+
+
+def self_groups(x: torch.Tensor, thr: float, metric="cosine", cap: Optional[int] = None, flags: int = 0,
+                want_stats: bool = False) -> GroupResult:
+    """Near-duplicate groups of ``x`` [N, D] (float32 CUDA): the connected components of the graph whose edges are the pairs
+    ``self_pairs`` lists (cosine ``>= thr``, Euclid ``<= thr``, decided by the fp32 value).  Rows a and c are in one group when
+    a chain of matches joins them, even if a and c do not match each other.  ``labels[i]`` is the smallest row of i's group, so
+    ``x[labels == arange(N)]`` keeps the first occurrence of every group; ``torch.unique(labels, return_counts=True)`` gives the
+    groups and their sizes.  ``cap`` sizes the device edge list (default ``max(8 * N, 65536)``); if more pairs match, the call
+    runs once more with the exact size.  Reading the counts is a host synchronisation."""
+    lib = _lib.load()
+    m = _METRICS[metric]
+    if isinstance(x, torch.Tensor) and x.dtype == torch.float16:
+        raise FfrError(ERR_UNSUPPORTED, "self_groups takes float32 embeddings (fp16 rows are not supported)")
+    x = _require_cuda(x, "x")
+    if x.dim() != 2:
+        raise ValueError(f"x {tuple(x.shape)} must be [N, D]")
+    n, dim = x.shape
+    dev = x.device
+    cap = _default_pair_cap(n) if cap is None else int(cap)
+    labels = torch.empty((n,), dtype=torch.int32, device=dev)
+    counts = torch.empty((2,), dtype=torch.int64, device=dev)            # group count, edge count
+    for _ in range(2):                                                   # _pairs' retry: at most once, with cap = count
+        ws = _workspace(dev, int(lib.ffr_self_groups_workspace_bytes(n, dim, m, cap)))
+        with torch.cuda.device(dev):
+            check(lib.ffr_self_groups(x.data_ptr(), n, dim, m, float(thr), labels.data_ptr(), counts.data_ptr(), cap,
+                                      counts[1:].data_ptr(), int(flags), ws.data_ptr(), ws.numel(), _stream_ptr(dev)))
+        n_groups, n_edges = (int(v) for v in counts.tolist())
+        if n_edges <= cap:
+            break
+        cap = n_edges
+    res = GroupResult(labels, n_groups, n_edges)
+    if want_stats:
+        arr = (C.c_int64 * 8)()
+        with torch.cuda.device(dev):
+            check(lib.ffr_filter_stats(ws.data_ptr(), arr, _stream_ptr(dev)))
+        res.stats = {"raw_pairs": arr[0], "path": "tcgen05" if arr[2] == 1 else "fp32", "launches": arr[3]}
+    return res
 
 
 class GraphedFilter:

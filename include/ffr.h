@@ -165,6 +165,28 @@ int ffr_match_pairs_self(const float* x, int64_t n, int64_t row_begin, int64_t n
                          int32_t* pair_cand, int32_t* pair_ref, float* pair_val, int64_t pair_cap, int64_t* pair_count,
                          int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
 
+/* ---- near-duplicate groups: connected components of the self-mode match graph ----------------------------------------
+ * Which rows of x[n, dim] (fp32, device) belong together.  The graph has the n rows as vertices and as edges exactly the pairs
+ * ffr_match_pairs_self(x, n, 0, n, ...) returns for the same x, metric, thr and flags: cosine >= thr / Euclid <= thr, each
+ * decided by the pair's fp32 value.  Bit-identical rows are not folded: they are edges like any other pair.
+ *   labels (device i32[n]): labels[i] = the smallest row index of i's connected component.  Row i represents its group iff
+ *     labels[i] == i, so dropping every other row keeps exactly one row per group, its first occurrence.  (Unlike
+ *     FFR_SELF_EARLIER, which flags each row that matches some earlier row, this joins rows through chains of matches.)
+ *   *group_count (device int64): the number of components.
+ *   *edge_count (device int64): as *pair_count of the match lists -- if *edge_count <= edge_cap, the labels are complete;
+ *     otherwise they come from a subset of the edges (a finer partition), and a second call with edge_cap >= *edge_count is
+ *     complete.  edge_cap = 0 is valid: the call counts the edges and labels every row as its own group.
+ *   Flags, dispatch and argument checks are ffr_match_pairs_self's (n in (0, 2^31), FFR_FLAG_FORCE_FP32 selects the exact
+ *     kernel, FFR_FLAG_FORCE_MMA fails where the tensor cores are not eligible, FFR_FLAG_NO_RECHECK is refused); labels and
+ *     group_count must be non-null.  Both paths give bit-identical labels: they list the same edges, and a graph has one
+ *     partition into components.
+ *   Asynchronous on the stream, no host synchronisation, no allocation (so it can be captured into a CUDA graph).  The
+ *   workspace (256-byte aligned) holds the match list's buffers plus an edge list of edge_cap 12-byte entries; the union-find
+ *   runs in place in labels.  ffr_filter_stats works on it as after a match-list call. */
+size_t ffr_self_groups_workspace_bytes(int64_t n, int32_t dim, int metric, int64_t edge_cap);
+int ffr_self_groups(const float* x, int64_t n, int32_t dim, int metric, float thr, int32_t* labels, int64_t* group_count,
+                    int64_t edge_cap, int64_t* edge_count, int flags, void* workspace, size_t ws_bytes, ffr_stream_t stream);
+
 /* statistics of the last ffr_filter* call that used this workspace (device->host copy, synchronises
  * the stream): out[0] = rows re-checked in fp32 against their two or three leading references (near-tie or
  * near-threshold), out[1] = rows that needed the full fp32 rescan, out[2] = path taken (0 fp32 CUDA-core,
